@@ -1,13 +1,19 @@
 #!/usr/bin/env python
 """bench.py -- graphs/sec of the BuckGNN 6x512 GraphSAGE forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one `model(x, edge_index, edge_attr, batch)` call on one synthetic batch
 of BASELINE.json configs[1] (256 non-stiffened plate meshes, super node + hub edges,
 random-init weights), CSR build included.  N > 1 (torchrun): every rank runs its own
 256 graphs (graph-sharded inference, no collective on the data path; weak scaling).
-Prints ONE JSON line (rank 0).  See the driver contract in the task notes.
+Prints ONE JSON line (rank 0).
+
+Inputs and weights are generated from fixed seeds, so two runs with the same arguments see
+the same data.  `--dump-outputs DIR` writes what the last timed step returned, `(pred, batch)`
+of rank 0, as DIR/pred.npy and DIR/batch.npy, so that two builds can be compared output
+for output.  With mean pooling `batch` is the input batch vector handed back unchanged, so
+pred.npy carries everything the step computed.
 """
 from __future__ import annotations
 
@@ -66,6 +72,26 @@ def _traffic_from_profile(name_part: str, exclude: str = ""):
             for r in rows[2:] if name_part in r[i_n] and not (exclude and exclude in r[i_n])]
     return {"bytes_per_launch": sum(vals) / len(vals), "launches": len(vals),
             "source": os.path.relpath(files[-1], ROOT)} if vals else None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes every tensor as out_dir/<name>.npy: floating point as float32 (float64 stays float64), integers as
+    float64, which holds them exactly.  The files stay within DUMP_BYTES in all: an array larger than its share is
+    replaced by a sample of its rows, drawn with a fixed seed so that every run keeps the same rows."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        a = (t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()).numpy()
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -158,21 +184,21 @@ def cpu_oracle_throughput(steps: int, warmup: int):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            ref(b.x, b.edge_index, b.edge_attr, b.batch)
+            outs = ref(b.x, b.edge_index, b.edge_attr, b.batch)
             if i >= warmup:
                 times.append(time.perf_counter() - t0)
     t = sum(times) / len(times)
     return dict(value=CPU_SAMPLE_GRAPHS / t, unit="graphs/s", cores=cores, kind="port",
                 sample=f"first {CPU_SAMPLE_GRAPHS} graphs of the workload ({b.num_nodes} nodes, {b.num_edges} edges), "
-                       f"{steps} timed forwards after {warmup} warm-up, torch fp32 oracle"), t
+                       f"{steps} timed forwards after {warmup} warm-up, torch fp32 oracle"), t, outs
 
 
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
-    cpu, t = cpu_oracle_throughput(steps, warmup)
+    steps, warmup = args.steps, args.warmup
+    cpu, t, outs = cpu_oracle_throughput(steps, warmup)
     line = {"metric": "graphs/sec", "value": cpu["value"], "unit": "graphs/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
@@ -182,6 +208,8 @@ def run_reference(args):
             "gpu_launches": 0,
             "note": "PyG/torch_scatter are not installable here; this is the CPU oracle port of the reference forward"}
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("pred", "batch"), outs)))
 
 
 def modes_section(args, dev, resident, world, G, barrier):
@@ -339,9 +367,12 @@ def run_b200(args):
     host = config_batch(1, rank=rank, num_graphs=args.graphs).pin_memory()
     G, N, E = host.num_graphs, host.num_nodes, host.num_edges
     resident = host.to(dev)
-    def fwd(b):
+    def forward(b):
         with torch.no_grad():
-            return model(b.x, b.edge_index, b.edge_attr, b.batch)[0]
+            return model(b.x, b.edge_index, b.edge_attr, b.batch)
+
+    def fwd(b):
+        return forward(b)[0]
 
     def barrier():
         if world > 1:
@@ -366,11 +397,13 @@ def run_b200(args):
         clk.begin()
         ev0.record()
         for _ in range(args.steps):
-            pred = fwd(resident)
+            outs = forward(resident)
         ev1.record()
         barrier()
         clk.end()
     step_ms = ev0.elapsed_time(ev1) / args.steps
+    # (pred, batch) of the last timed step, on the host before any later forward runs
+    last_outs = dict(zip(("pred", "batch"), (t.cpu() for t in outs))) if args.dump_outputs else None
     kernel_ms = engine.TIMERS.summary()          # per kernel class: total ms, calls
     engine.TIMERS.disable()
 
@@ -521,7 +554,7 @@ def run_b200(args):
                          "note": "sum_k max(B_k / measured HBM peak, F_k / measured sustained tensor peak) / step time"}
         cpu = None
         if world == 1 and not args.no_cpu_baseline:
-            cpu, _ = cpu_oracle_throughput(3, 1)
+            cpu, _, _ = cpu_oracle_throughput(3, 1)
         line = {
             "metric": "graphs/sec", "value": value, "unit": "graphs/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": step_ms, "higher_is_better": True, "scaling": "weak",
@@ -565,6 +598,8 @@ def run_b200(args):
             "clocks": clk.summary(),
         }
         print(json.dumps(line))
+        if last_outs is not None:
+            dump_outputs(args.dump_outputs, last_outs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -581,7 +616,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the tf32 / fp32 modes and the training-step section")
     ap.add_argument("--train-precision", default="tf32")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write (pred, batch) of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

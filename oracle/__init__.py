@@ -6,7 +6,7 @@ reported CPU baseline.  Nothing under `buckgnn_b200/` or `Models/` imports it; t
 product path raises if the CUDA library is missing instead of falling back here.
 
 PARITY PINNED TO THE REFERENCE'S OWN SOURCE FILE (round 2).  `reference_source.py` executes
-`/root/reference/Models/BuckGNN.py` unmodified (read where it lies, nothing copied) and
+the reference's `Models/BuckGNN.py` unmodified (read where it lies, nothing copied) and
 `tests/test_reference_source.py` asserts reference == oracle to 1e-6 on the CPU for every
 `model_name` x `pooling_layer` x `prediction_type` that works in the reference (forward,
 autograd gradients, BatchNorm buffers, the dropout RNG stream), plus the reference's broken
@@ -15,7 +15,7 @@ its sha256), so the GPU golden tests compare the CUDA path with the reference, n
 restatement.
 
 What remains restated: the arithmetic INSIDE two third-party packages the reference imports, which
-are neither vendored in `/root/reference` nor installable here (no network): `torch_geometric`
+are neither vendored in the reference project nor dependencies of this one: `torch_geometric`
 (`SAGEConv`, `SAGPooling`, `global_mean_pool`) and `torch_scatter` (`scatter_mean`,
 `scatter_add`), both unpinned by the reference (`README.md:64-70` names them without versions;
 the `lin_l` / `lin_r` parameter names imply PyG >= 1.6 / 2.x).  Their published semantics are

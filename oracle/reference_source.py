@@ -6,13 +6,14 @@ minimal stand-ins for exactly the names that file imports -- `SAGEConv`, `SAGPoo
 `global_{mean,max,add}_pool`, `scatter_add`, `scatter_mean` -- with the constructor / call
 signatures PyG and torch_scatter publish, backed by the operator functions of
 `oracle/buckgnn_oracle.py`.  `load_reference()` then executes the reference source file where it
-lies (`/root/reference/Models/BuckGNN.py`; nothing is copied), so the reference's real
+lies (`Models/BuckGNN.py` of a checkout of the reference project; nothing is copied), so the reference's real
 constructor, layer loops, skip rules, pooling selection, `.squeeze()` and error branches run as
 written.  What stays restated is only the arithmetic inside the two third-party packages.
 
-Used by `tests/test_reference_source.py` (reference == oracle on CPU) and
-`tests/golden/make_golden.py` (the committed fixtures are outputs of the reference file).
-`/root/reference` does not exist on the GPU box: callers must check `reference_available()`.
+Used by `tests/test_reference_source.py` (the reference re-run against its stored outputs) and by
+`tests/golden/make_golden.py` / `make_reference_cases.py` (the committed fixtures are outputs of the reference file).
+The reference project is not part of this repository: set BUCKGNN_REFERENCE_DIR to a checkout of it.
+Without one, callers must check `reference_available()`.
 """
 from __future__ import annotations
 
@@ -28,11 +29,13 @@ import torch.nn.functional as F
 
 from . import buckgnn_oracle as O
 
-REFERENCE_FILE = "/root/reference/Models/BuckGNN.py"
+REFERENCE_DIR = os.environ.get("BUCKGNN_REFERENCE_DIR", "")
+REFERENCE_FILE = os.path.join(REFERENCE_DIR, "Models", "BuckGNN.py") if REFERENCE_DIR else ""
+SKIP_REASON = "needs a checkout of the reference project (github.com/omerkurt-okt/buck-gnn): set BUCKGNN_REFERENCE_DIR"
 
 
 def reference_available(path: str = REFERENCE_FILE) -> bool:
-    return os.path.isfile(path)
+    return bool(path) and os.path.isfile(path)
 
 
 def reference_sha256(path: str = REFERENCE_FILE) -> str:

@@ -1,13 +1,13 @@
 """Generates tests/golden/oracle_golden.json by RUNNING THE REFERENCE'S OWN FILE.
 
-    python tests/golden/make_golden.py          (in the build container, where /root/reference exists)
+    BUCKGNN_REFERENCE_DIR=<checkout of the reference project> python tests/golden/make_golden.py
 
-The model that produces every stored number is `BuckGNN` from `/root/reference/Models/BuckGNN.py`,
+The model that produces every stored number is `BuckGNN` from the reference's `Models/BuckGNN.py`,
 executed unmodified through `oracle/reference_source.py` (its two third-party imports, torch_geometric
 and torch_scatter -- not installable here -- are shimmed with stand-ins of the same signatures, backed by
 the restated operators of oracle/buckgnn_oracle.py).  The file records the sha256 of the reference source
 it ran.  Inputs are regenerated from seeds (buckgnn_b200.synth, torch.manual_seed); outputs are stored.
-On the GPU box /root/reference is absent: tests read the committed JSON; `seeded_model` there builds the
+Without a reference checkout, tests read the committed JSON; `seeded_model` there builds the
 oracle twin with the same seed as a WEIGHT CONTAINER (its state_dict checksum is checked against the file).
 """
 import json
@@ -118,8 +118,8 @@ def topk_gaps(m, b):
 
 def main():
     if not RS.reference_available():
-        raise SystemExit("make_golden.py needs /root/reference (it runs the reference's own Models/BuckGNN.py)")
-    out = {"generated_from": RS.REFERENCE_FILE, "reference_sha256": RS.reference_sha256(),
+        raise SystemExit("make_golden.py runs the reference's own Models/BuckGNN.py: " + RS.SKIP_REASON)
+    out = {"generated_from": os.path.relpath(RS.REFERENCE_FILE, RS.REFERENCE_DIR), "reference_sha256": RS.reference_sha256(),
            "generator": "tests/golden/make_golden.py via oracle/reference_source.py (torch_geometric / torch_scatter shimmed)",
            "forward": {}, "operators": {}, "training": {}}
     for name, over, bkw in FORWARD_CASES:

@@ -1,6 +1,6 @@
 """Stand-ins for the packages the reference's driver scripts import but this image lacks, so that
-`/root/reference/{TRAIN_FINAL,INFERENCE,INFERENCE_TIMER}.py` can be EXECUTED UNMODIFIED against this repo's
-`Models` package (tests/test_reference_scripts.py).  Test infrastructure only.
+`{TRAIN_FINAL,INFERENCE,INFERENCE_TIMER}.py` of a reference checkout (BUCKGNN_REFERENCE_DIR) can be
+EXECUTED UNMODIFIED against this repo's `Models` package (tests/test_reference_scripts.py).  Test infrastructure only.
 
 Stubbed: torch_geometric.loader.DataLoader / torch_geometric.data.Data (a collating loader over the synthetic
 plates of buckgnn_b200.synth), torch_geometric.nn + torch_scatter (oracle/reference_source.py shims; Utils/Losses.py
@@ -19,7 +19,7 @@ import torch
 from buckgnn_b200.synth import collate, make_plate_graph
 from oracle import reference_source as RS
 
-REF = "/root/reference"
+REF = RS.REFERENCE_DIR
 
 
 class StubDataLoader:
@@ -146,7 +146,7 @@ def script_environment():
 
 
 def load_script(name):
-    """Executes /root/reference/<name>.py as a module (not as __main__), unmodified."""
+    """Executes <reference checkout>/<name>.py as a module (not as __main__), unmodified."""
     spec = importlib.util.spec_from_file_location(f"_reference_{name}", f"{REF}/{name}.py")
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)

@@ -7,7 +7,8 @@ load that checkpoint (pickled `DatasetNormalizer` included) and run the test loo
 tests/ref_script_stubs.py (PyG loader, ray, matplotlib, the BDF/OP2 graph builder).  This box has no GPU and the product
 has no CPU path, so `BuckGNN.forward` is replaced -- in this test only -- by a contract-checking wrapper that evaluates
 the oracle on the module's own parameters; constructor, state_dict, `.to()`, `.train()/.eval()`, `parameters()` for Adam,
-the 4-argument call and the `(pred, batch)` return are this repo's.  /root/reference is absent on the GPU box: skipped there.
+the 4-argument call and the `(pred, batch)` return are this repo's.  The scripts are read from a checkout of the
+reference project (BUCKGNN_REFERENCE_DIR), which is not part of this repository: skipped without one.
 """
 import os
 
@@ -18,7 +19,7 @@ import torch
 from oracle import reference_source as RS
 from tests import ref_script_stubs as S
 
-pytestmark = pytest.mark.skipif(not RS.reference_available(), reason="/root/reference not present (GPU box)")
+pytestmark = pytest.mark.skipif(not RS.reference_available(), reason=RS.SKIP_REASON)
 
 
 @pytest.fixture()
