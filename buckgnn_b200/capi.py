@@ -30,7 +30,7 @@ EXPORTED_SYMBOLS = (
     "bg_csr_max_big_rows", "bg_csr_workspace_bytes", "bg_csr_build",
     "bg_batch_info", "bg_graph_ptr_build", "bg_publish_words", "bg_encoder_front",
     "bg_aggregate_workspace_bytes", "bg_hubfold_workspace_bytes", "bg_sage_aggregate", "bg_gemm512",
-    "bg_sage_fused512", "bg_sage_aggregate_hubs",
+    "bg_sage_fused512", "bg_sage_aggregate_hubs", "bg_gemm128", "bg_pool_head128", "bg_pool_head_blocks128",
     "bg_wgrad512", "bg_pool_workspace_bytes", "bg_pool_head", "bg_pool_block_flags", "bg_pool_head_blocks", "bg_cast_f32", "bg_split_tf32",
     "bg_expand_rowptr", "bg_add",
     "bg_train_workspace_bytes", "bg_bn_batch_stats", "bg_bn_act_forward", "bg_sage_backward_rows",
@@ -94,6 +94,12 @@ _SIGNATURES = {
     "bg_sage_fused512": (C.c_int, [C.POINTER(GemmSegment), _I32, _I64, C.c_int, C.c_int, C.POINTER(Epilogue),
                                    C.POINTER(FusedAggregate), _P, C.c_int, _I64, _P]),
     "bg_sage_aggregate_hubs": (C.c_int, [_P, C.c_int, _P, _P, _P, _I32, C.c_int, _P, _P, C.c_size_t, _P]),
+    "bg_gemm128": (C.c_int, [C.POINTER(GemmSegment), _I32, _I64, C.c_int, C.c_int, C.POINTER(Epilogue), _P,
+                             C.c_int, _I64, C.c_int, _P]),
+    "bg_pool_head128": (C.c_int, [_P, C.c_int, _I64, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _P, _P,
+                                  _P, C.c_size_t, _P, _P]),
+    "bg_pool_head_blocks128": (C.c_int, [_P, C.c_int, _I64, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _P,
+                                         _P, _P, _P, _P, C.c_size_t, _P, _P]),
     "bg_wgrad512": (C.c_int, [_P, _I64, _P, _I32, _I64, C.c_int, _I64, _I32, _I64, _P, _P]),
     "bg_pool_workspace_bytes": (C.c_int, [_I64, _SZP]),
     "bg_pool_head": (C.c_int, [_P, C.c_int, _I64, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _P, _P,
@@ -262,6 +268,21 @@ def gemm512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=
            "bg_gemm512")
 
 
+def gemm128(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
+            bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
+            gather=(), gather_ld=128, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+    """bg_gemm128: gemm512 with 128-wide output rows (B [128, k], epilogue vectors [128]).  `gather` and `b_groups`
+    are accepted only so that the library can reject them (BG_ERR_UNSUPPORTED)."""
+    n = len(segments)
+    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
+    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
+    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
+    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
+                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
+    _check(load().bg_gemm128(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group, stream),
+           "bg_gemm128")
+
+
 def sage_fused512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, x, ldx, rowptr, col, aggr, hub_agg=None,
                   big_rows=None, n_big=0, bias=None, bn_scale=None, bn_shift=None, residual=None, ldr=0, relu=False,
                   pool_block_sums=None, pool_block_keep=None):
@@ -292,6 +313,12 @@ def pool_head(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w
                                w3, b3, out_dim, pred, pooled_out, ws, ws_bytes, nonfinite, stream), "bg_pool_head")
 
 
+def pool_head128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim,
+                 pred, pooled_out, ws, ws_bytes, stream, nonfinite=None):
+    _check(load().bg_pool_head128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2, b2,
+                                  w3, b3, out_dim, pred, pooled_out, ws, ws_bytes, nonfinite, stream), "bg_pool_head128")
+
+
 def pool_block_flags(graph_ptr, n_graphs, n_nodes, keep, stream):
     _check(load().bg_pool_block_flags(graph_ptr, n_graphs, n_nodes, keep, stream), "bg_pool_block_flags")
 
@@ -301,6 +328,13 @@ def pool_head_blocks(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, p
     _check(load().bg_pool_head_blocks(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2, b2,
                                       w3, b3, out_dim, pred, pooled_out, block_sums, keep, ws, ws_bytes, nonfinite,
                                       stream), "bg_pool_head_blocks")
+
+
+def pool_head_blocks128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim,
+                        pred, pooled_out, block_sums, keep, ws, ws_bytes, stream, nonfinite=None):
+    _check(load().bg_pool_head_blocks128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2,
+                                         b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, ws, ws_bytes,
+                                         nonfinite, stream), "bg_pool_head_blocks128")
 
 
 def cast_f32(src, dst, dst_dtype, n, stream):

@@ -9,6 +9,7 @@
 #include "aggregate_window.cuh"
 #include "encoder.cuh"
 #include "gemm_tc.cuh"
+#include "gemm128.cuh"
 #include "pool_head.cuh"
 #include "train.cuh"
 #include "sag_pool.cuh"
@@ -24,6 +25,11 @@ void set_last_cuda_error(cudaError_t e, const char* what, const char* file, int 
 }
 static int fail(int code, const char* msg) {
   snprintf(g_last_error, sizeof(g_last_error), "%s", msg);
+  return code;
+}
+// "<entry point>: <message>" for implementations shared by the 512- and 128-wide entry points
+static int fail_in(int code, const char* fn, const char* msg) {
+  snprintf(g_last_error, sizeof(g_last_error), "%s: %s", fn, msg);
   return code;
 }
 
@@ -261,7 +267,7 @@ static int aggregate_dispatch(const T* x, T* out, int64_t N, const int32_t* rowp
 }
 
 
-template <typename T>
+template <typename T, int kW>
 static void pool_launch(const T* x, const int32_t* graph_ptr, int64_t G, int mode, const float* pre_w, const float* pre_b,
                         const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
                         const float* b3, int out_dim, float* pred, float* pooled_out, float* partial, const int32_t* nonfinite,
@@ -269,10 +275,24 @@ static void pool_launch(const T* x, const int32_t* graph_ptr, int64_t G, int mod
   if (mode != BG_POOL_SUPERNODE_ONLY) {
     dim3 grid((unsigned)G, kPoolSlices);
     const int exclude_last = (mode == BG_POOL_MEAN_NO_SUPER || mode == BG_POOL_SUPERNODE_WITH_POOLING) ? 1 : 0;
-    k_pool_partial<T><<<grid, kPoolWarps * 32, 0, stream>>>(x, graph_ptr, partial, exclude_last);
+    k_pool_partial<T, kW><<<grid, kPoolWarps * 32, 0, stream>>>(x, graph_ptr, partial, exclude_last);
   }
-  k_pool_head<T><<<(unsigned)G, 128, 0, stream>>>(x, partial, graph_ptr, mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3,
-                                                   out_dim, pred, pooled_out, nonfinite);
+  k_pool_head<T, kW><<<(unsigned)G, 128, 0, stream>>>(x, partial, graph_ptr, mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3,
+                                                       out_dim, pred, pooled_out, nonfinite);
+}
+
+template <typename T, int kW>
+static void pool_blocks_launch(const T* x, const int32_t* graph_ptr, int64_t G, int mode, const float* pre_w,
+                               const float* pre_b, const float* w1, const float* b1, const float* w2, const float* b2,
+                               const float* w3, const float* b3, int out_dim, float* pred, float* pooled_out,
+                               const float* block_sums, const uint8_t* keep, float* partial, const int32_t* nonfinite,
+                               cudaStream_t stream) {
+  const int exclude_last = (mode == BG_POOL_MEAN_NO_SUPER || mode == BG_POOL_SUPERNODE_WITH_POOLING) ? 1 : 0;
+  dim3 grid((unsigned)G, kPoolSlices);
+  if (mode != BG_POOL_SUPERNODE_ONLY)
+    k_pool_partial_blocks<T, kW><<<grid, kW / 2, 0, stream>>>(x, block_sums, keep, graph_ptr, partial, exclude_last);
+  k_pool_head<T, kW><<<(unsigned)G, 128, 0, stream>>>(x, partial, graph_ptr, mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3,
+                                                       out_dim, pred, pooled_out, nonfinite);
 }
 
 }  // namespace bg
@@ -645,6 +665,79 @@ int bg_sage_fused512(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int 
   return gemm512_impl(segs, n_seg, m, a_dtype, b_dtype, epi, fuse, out, out_dtype, ldo, 2, stream_);
 }
 
+int bg_gemm128(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtype, int b_dtype,
+               const bg_epilogue* epi, void* out, int out_dtype, int64_t ldo, int cta_group, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  // every argument is checked before the first CUDA call
+  if (!segs || n_seg < 1 || n_seg > BG_MAX_GEMM_SEGMENTS) return fail(BG_ERR_INVALID, "bg_gemm128: bad segment count");
+  if (m < 0 || m >= 0x7fffffffLL) return fail(BG_ERR_INVALID, "bg_gemm128: bad m");
+  const int a_fmt = umma_format_of(a_dtype), b_fmt = umma_format_of(b_dtype);
+  if (a_fmt < 0 || b_fmt < 0 || a_fmt != b_fmt)
+    return fail(BG_ERR_INVALID, "bg_gemm128: a_dtype and b_dtype must be the same (bf16, f16 or f32)");
+  if (umma_format_of(out_dtype) < 0) return fail(BG_ERR_INVALID, "bg_gemm128: bad out_dtype");
+  if (cta_group != 2) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: only cta_group = 2 is built");
+  const bool tf32 = a_fmt == 2;
+  const int esz = tf32 ? 4 : 2, osz = out_dtype == BG_F32 ? 4 : 2;
+  const int kblk = kStageKBytes / esz;
+  if (!out || !aligned16(out) || (ldo * osz) % 16 != 0 || ldo < kW128) return fail(BG_ERR_INVALID, "bg_gemm128: bad out/ldo");
+  for (int s = 0; s < n_seg; ++s) {
+    const bg_gemm_segment& g = segs[s];
+    if (!g.a || !g.b) return fail(BG_ERR_INVALID, "bg_gemm128: null operand");
+    if (g.k <= 0 || g.k % kblk != 0) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: k must be a positive multiple of 64 (16-bit) / 32 (tf32)");
+    if (g.b_groups > 1) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: b_groups is not built at width 128");
+    if (!aligned16(g.a) || (g.lda * esz) % 16 != 0 || g.lda < g.k || !aligned16(g.b) || (g.ldb * esz) % 16 != 0 || g.ldb < g.k)
+      return fail(BG_ERR_INVALID, "bg_gemm128: operand alignment / leading dimension");
+  }
+  if (epi) {
+    if (epi->gather[0] || epi->gather[1]) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: gathered addends are not built at width 128");
+    if (epi->residual && (!aligned16(epi->residual) || (epi->ldr * osz) % 16 != 0 || epi->ldr < kW128))
+      return fail(BG_ERR_INVALID, "bg_gemm128: bad residual/ldr");
+    if (epi->bn_scale_host && !epi->bn_shift_host) return fail(BG_ERR_INVALID, "bg_gemm128: bn_scale without bn_shift");
+    if (epi->inv_norm_out && !epi->normalize) return fail(BG_ERR_INVALID, "bg_gemm128: inv_norm_out needs normalize");
+    if ((epi->pool_block_sums != nullptr) != (epi->pool_block_keep != nullptr))
+      return fail(BG_ERR_INVALID, "bg_gemm128: pool_block_sums and pool_block_keep go together");
+    if (epi->pool_block_sums && (!epi->normalize || out_dtype == BG_F32 || epi->residual || !aligned16(epi->pool_block_sums)))
+      return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: the pool-fused epilogue needs normalize, a 16-bit output and no residual");
+  }
+  if (m == 0) return BG_OK;
+  Gemm128Params p;
+  memset(&p, 0, sizeof(p));
+  for (int s = 0; s < n_seg; ++s) {
+    const bg_gemm_segment& g = segs[s];
+    int rc = make_operand_map(&p.seg[s].a, g.a, m, g.k, g.lda, (uint32_t)a_fmt);
+    if (rc == BG_OK) rc = make_operand_map_rows(&p.seg[s].b, g.b, kW128, g.k, g.ldb, (uint32_t)b_fmt, kG128BRows);
+    if (rc != BG_OK) return fail(rc, "bg_gemm128: cuTensorMapEncodeTiled failed");
+    p.kblocks[s] = g.k / kblk;
+  }
+  p.n_seg = n_seg;
+  p.k_elems_per_block = kblk;
+  p.a_fmt = (uint32_t)a_fmt; p.b_fmt = (uint32_t)b_fmt;
+  p.n_tiles = (int32_t)ceil_div64(m, 2 * kTileM);
+  p.m = m;
+  for (int i = 0; i < kW128; ++i) { p.bias[i] = 0.f; p.scale[i] = 1.f; p.shift[i] = 0.f; }
+  if (epi) {
+    if (epi->bias_host) memcpy(p.bias, epi->bias_host, sizeof(float) * kW128);
+    if (epi->bn_scale_host) {
+      memcpy(p.scale, epi->bn_scale_host, sizeof(float) * kW128);
+      memcpy(p.shift, epi->bn_shift_host, sizeof(float) * kW128);
+    }
+    p.normalize = epi->normalize; p.relu = epi->relu;
+    p.residual = epi->residual; p.ldr = epi->ldr;
+    p.inv_norm_out = epi->inv_norm_out;
+    p.pool_sums = epi->pool_block_sums; p.pool_keep = epi->pool_block_keep;
+  }
+  p.out = out; p.ldo = ldo;
+  if (p.pool_sums)
+    return out_dtype == BG_BF16 ? launch_gemm128<__nv_bfloat16, false, true>(p, stream)
+                                : launch_gemm128<__half, false, true>(p, stream);
+#define BG_GEMM128_OUT(RES)                                                              \
+  (out_dtype == BG_BF16 ? launch_gemm128<__nv_bfloat16, RES, false>(p, stream)           \
+   : out_dtype == BG_F16 ? launch_gemm128<__half, RES, false>(p, stream)                 \
+                         : launch_gemm128<float, RES, false>(p, stream))
+  return p.residual ? BG_GEMM128_OUT(true) : BG_GEMM128_OUT(false);
+#undef BG_GEMM128_OUT
+}
+
 int bg_sage_aggregate_hubs(const void* x, int dtype, const int32_t* rowptr, const int32_t* col, const int32_t* big_rows,
                            int32_t n_big, int aggr, void* hub_out, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -707,34 +800,55 @@ int bg_pool_workspace_bytes(int64_t G, size_t* bytes_host) {
   return BG_OK;
 }
 
-int bg_pool_head(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+static int pool_head_impl(const char* fn, int width, const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
                  const float* pre_w, const float* pre_b,
                  const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
                  int32_t out_dim, float* pred, float* pooled_out, void* workspace, size_t workspace_bytes,
                  const int32_t* nonfinite_flag, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (G < 0 || N < 0 || G > 65535LL * 1024) return fail(BG_ERR_INVALID, "bg_pool_head: bad size");
+  if (G < 0 || N < 0 || G > 65535LL * 1024) return fail_in(BG_ERR_INVALID, fn, "bad size");
   if (G == 0) return BG_OK;
-  if (out_dim < 1 || out_dim > 64) return fail(BG_ERR_UNSUPPORTED, "bg_pool_head: out_dim must be in [1,64]");
-  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail(BG_ERR_INVALID, "bg_pool_head: bad pool_mode");
+  if (out_dim < 1 || out_dim > 64) return fail_in(BG_ERR_UNSUPPORTED, fn, "out_dim must be in [1,64]");
+  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail_in(BG_ERR_INVALID, fn, "bad pool_mode");
   if ((pre_w != nullptr) != (pre_b != nullptr) || (pre_w && pool_mode > BG_POOL_MEAN_NO_SUPER) || (pre_w && !aligned16(pre_w)))
-    return fail(BG_ERR_INVALID, "bg_pool_head: pooling MLP needs both pre_w and pre_b and a mean pooling mode");
+    return fail_in(BG_ERR_INVALID, fn, "pooling MLP needs both pre_w and pre_b and a mean pooling mode");
   if (!graph_ptr || !w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !pred || (N > 0 && (!x || !aligned16(x))) || !aligned16(w1))
-    return fail(BG_ERR_INVALID, "bg_pool_head: bad pointer");
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
   size_t need = 0;
   bg_pool_workspace_bytes(G, &need);
-  if (!workspace || workspace_bytes < need) return fail(BG_ERR_WORKSPACE, "bg_pool_head: workspace too small");
+  if (!workspace || workspace_bytes < need) return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
   float* partial = static_cast<float*>(workspace);
   if (dtype == BG_BF16)
-    pool_launch(static_cast<const __nv_bfloat16*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
+    (width == kHidden ? pool_launch<__nv_bfloat16, kHidden> : pool_launch<__nv_bfloat16, kW128>)(
+        static_cast<const __nv_bfloat16*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
   else if (dtype == BG_F16)
-    pool_launch(static_cast<const __half*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
+    (width == kHidden ? pool_launch<__half, kHidden> : pool_launch<__half, kW128>)(
+        static_cast<const __half*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
   else if (dtype == BG_F32)
-    pool_launch(static_cast<const float*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
+    (width == kHidden ? pool_launch<float, kHidden> : pool_launch<float, kW128>)(
+        static_cast<const float*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, partial, nonfinite_flag, stream);
   else
-    return fail(BG_ERR_INVALID, "bg_pool_head: bad dtype");
+    return fail_in(BG_ERR_INVALID, fn, "bad dtype");
   BG_LAUNCH_OK();
   return BG_OK;
+}
+
+int bg_pool_head(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+                 const float* pre_w, const float* pre_b,
+                 const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                 int32_t out_dim, float* pred, float* pooled_out, void* workspace, size_t workspace_bytes,
+                 const int32_t* nonfinite_flag, void* stream_) {
+  return pool_head_impl("bg_pool_head", kHidden, x, dtype, N, graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3,
+                        out_dim, pred, pooled_out, workspace, workspace_bytes, nonfinite_flag, stream_);
+}
+
+int bg_pool_head128(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+                    const float* pre_w, const float* pre_b,
+                    const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                    int32_t out_dim, float* pred, float* pooled_out, void* workspace, size_t workspace_bytes,
+                    const int32_t* nonfinite_flag, void* stream_) {
+  return pool_head_impl("bg_pool_head128", kW128, x, dtype, N, graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3,
+                        b3, out_dim, pred, pooled_out, workspace, workspace_bytes, nonfinite_flag, stream_);
 }
 
 int bg_pool_block_flags(const int32_t* graph_ptr, int64_t G, int64_t N, uint8_t* keep, void* stream_) {
@@ -747,39 +861,54 @@ int bg_pool_block_flags(const int32_t* graph_ptr, int64_t G, int64_t N, uint8_t*
   return BG_OK;
 }
 
-int bg_pool_head_blocks(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+static int pool_head_blocks_impl(const char* fn, int width, const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
                         const float* pre_w, const float* pre_b,
                         const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
                         int32_t out_dim, float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
                         void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (G < 0 || N < 0 || G > 65535LL * 1024) return fail(BG_ERR_INVALID, "bg_pool_head_blocks: bad size");
+  if (G < 0 || N < 0 || G > 65535LL * 1024) return fail_in(BG_ERR_INVALID, fn, "bad size");
   if (G == 0) return BG_OK;
-  if (out_dim < 1 || out_dim > 64) return fail(BG_ERR_UNSUPPORTED, "bg_pool_head_blocks: out_dim must be in [1,64]");
-  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail(BG_ERR_INVALID, "bg_pool_head_blocks: bad pool_mode");
+  if (out_dim < 1 || out_dim > 64) return fail_in(BG_ERR_UNSUPPORTED, fn, "out_dim must be in [1,64]");
+  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail_in(BG_ERR_INVALID, fn, "bad pool_mode");
   if ((pre_w != nullptr) != (pre_b != nullptr) || (pre_w && pool_mode > BG_POOL_MEAN_NO_SUPER) || (pre_w && !aligned16(pre_w)))
-    return fail(BG_ERR_INVALID, "bg_pool_head_blocks: pooling MLP needs both pre_w and pre_b and a mean pooling mode");
+    return fail_in(BG_ERR_INVALID, fn, "pooling MLP needs both pre_w and pre_b and a mean pooling mode");
   if (!graph_ptr || !w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !pred || !aligned16(w1) ||
       (N > 0 && (!x || !aligned16(x) || !block_sums || !aligned16(block_sums) || !keep)))
-    return fail(BG_ERR_INVALID, "bg_pool_head_blocks: bad pointer");
-  if (dtype != BG_BF16 && dtype != BG_F16) return fail(BG_ERR_UNSUPPORTED, "bg_pool_head_blocks: 16-bit rows only");
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  if (dtype != BG_BF16 && dtype != BG_F16) return fail_in(BG_ERR_UNSUPPORTED, fn, "16-bit rows only");
   size_t need = 0;
   bg_pool_workspace_bytes(G, &need);
-  if (!workspace || workspace_bytes < need) return fail(BG_ERR_WORKSPACE, "bg_pool_head_blocks: workspace too small");
+  if (!workspace || workspace_bytes < need) return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
   float* partial = static_cast<float*>(workspace);
-  const int exclude_last = (pool_mode == BG_POOL_MEAN_NO_SUPER || pool_mode == BG_POOL_SUPERNODE_WITH_POOLING) ? 1 : 0;
-  dim3 grid((unsigned)G, kPoolSlices);
-  if (dtype == BG_BF16) {
-    const __nv_bfloat16* xp = static_cast<const __nv_bfloat16*>(x);
-    if (pool_mode != BG_POOL_SUPERNODE_ONLY) k_pool_partial_blocks<__nv_bfloat16><<<grid, 256, 0, stream>>>(xp, block_sums, keep, graph_ptr, partial, exclude_last);
-    k_pool_head<__nv_bfloat16><<<(unsigned)G, 128, 0, stream>>>(xp, partial, graph_ptr, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, nonfinite_flag);
-  } else {
-    const __half* xp = static_cast<const __half*>(x);
-    if (pool_mode != BG_POOL_SUPERNODE_ONLY) k_pool_partial_blocks<__half><<<grid, 256, 0, stream>>>(xp, block_sums, keep, graph_ptr, partial, exclude_last);
-    k_pool_head<__half><<<(unsigned)G, 128, 0, stream>>>(xp, partial, graph_ptr, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, nonfinite_flag);
-  }
+  if (dtype == BG_BF16)
+    (width == kHidden ? pool_blocks_launch<__nv_bfloat16, kHidden> : pool_blocks_launch<__nv_bfloat16, kW128>)(
+        static_cast<const __nv_bfloat16*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, partial, nonfinite_flag, stream);
+  else
+    (width == kHidden ? pool_blocks_launch<__half, kHidden> : pool_blocks_launch<__half, kW128>)(
+        static_cast<const __half*>(x), graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1, w2, b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, partial, nonfinite_flag, stream);
   BG_LAUNCH_OK();
   return BG_OK;
+}
+
+int bg_pool_head_blocks(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+                        const float* pre_w, const float* pre_b,
+                        const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                        int32_t out_dim, float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
+                        void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream_) {
+  return pool_head_blocks_impl("bg_pool_head_blocks", kHidden, x, dtype, N, graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1,
+                               w2, b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, workspace, workspace_bytes,
+                               nonfinite_flag, stream_);
+}
+
+int bg_pool_head_blocks128(const void* x, int dtype, int64_t N, const int32_t* graph_ptr, int64_t G, int pool_mode,
+                           const float* pre_w, const float* pre_b,
+                           const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                           int32_t out_dim, float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
+                           void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream_) {
+  return pool_head_blocks_impl("bg_pool_head_blocks128", kW128, x, dtype, N, graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1,
+                               w2, b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, workspace, workspace_bytes,
+                               nonfinite_flag, stream_);
 }
 
 // ------------------------------------------------------------------ EA-GNN helpers

@@ -23,37 +23,55 @@ constexpr int kPoolWarps = 8;
 enum : int { kPoolMean = BG_POOL_MEAN, kPoolMeanNoSuper = BG_POOL_MEAN_NO_SUPER,
              kPoolSuperOnly = BG_POOL_SUPERNODE_ONLY, kPoolSuperWithPooling = BG_POOL_SUPERNODE_WITH_POOLING };
 
-template <typename T>
+template <typename T, int kW>
 __global__ void __launch_bounds__(kPoolWarps * 32)
 k_pool_partial(const T* __restrict__ x, const int32_t* __restrict__ graph_ptr, float* __restrict__ partial,
                int exclude_last) {
-  __shared__ float red[kPoolWarps][kHidden];
+  __shared__ float red[kPoolWarps][kW];
   const int g = blockIdx.x, slice = blockIdx.y;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int32_t beg = graph_ptr[g], cnt = max(graph_ptr[g + 1] - beg - (exclude_last ? 1 : 0), 0);
   const int32_t s_beg = beg + (int32_t)((int64_t)cnt * slice / kPoolSlices);
   const int32_t s_end = beg + (int32_t)((int64_t)cnt * (slice + 1) / kPoolSlices);
-  float acc[16];
+  constexpr int kCols = kW / 32;                             // columns per lane
+  float acc[kCols];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  for (int i = 0; i < kCols; ++i) acc[i] = 0.f;
   int32_t r = s_beg + warp;
-  for (; r + kPoolWarps < s_end; r += 2 * kPoolWarps) {      // two rows in flight per warp
-    RowFrag<T> f0, f1;
-    f0.load(x + (size_t)r * kHidden, lane);
-    f1.load(x + (size_t)(r + kPoolWarps) * kHidden, lane);
-    f0.template accumulate<BG_AGGR_SUM>(acc);
-    f1.template accumulate<BG_AGGR_SUM>(acc);
-  }
-  for (; r < s_end; r += kPoolWarps) {
-    RowFrag<T> f;
-    f.load(x + (size_t)r * kHidden, lane);
-    f.template accumulate<BG_AGGR_SUM>(acc);
-  }
+  if constexpr (kW == kHidden) {
+    for (; r + kPoolWarps < s_end; r += 2 * kPoolWarps) {      // two rows in flight per warp
+      RowFrag<T> f0, f1;
+      f0.load(x + (size_t)r * kHidden, lane);
+      f1.load(x + (size_t)(r + kPoolWarps) * kHidden, lane);
+      f0.template accumulate<BG_AGGR_SUM>(acc);
+      f1.template accumulate<BG_AGGR_SUM>(acc);
+    }
+    for (; r < s_end; r += kPoolWarps) {
+      RowFrag<T> f;
+      f.load(x + (size_t)r * kHidden, lane);
+      f.template accumulate<BG_AGGR_SUM>(acc);
+    }
 #pragma unroll
-  for (int i = 0; i < 16; ++i) red[warp][RowFrag<T>::col_of(lane, i)] = acc[i];
+    for (int i = 0; i < kCols; ++i) red[warp][RowFrag<T>::col_of(lane, i)] = acc[i];
+  } else {                                                   // narrow rows: lane owns kCols consecutive columns
+    static_assert(kCols == 4, "width 128: 4 columns per lane");
+    for (; r < s_end; r += kPoolWarps) {
+      const T* row = x + (size_t)r * kW + lane * kCols;
+      if constexpr (sizeof(T) == 4) {
+        const float4 v = *reinterpret_cast<const float4*>(row);
+        acc[0] += v.x; acc[1] += v.y; acc[2] += v.z; acc[3] += v.w;
+      } else {
+        const uint2 u = *reinterpret_cast<const uint2*>(row);
+        Pack16<T>::add2(acc[0], acc[1], u.x);
+        Pack16<T>::add2(acc[2], acc[3], u.y);
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < kCols; ++i) red[warp][lane * kCols + i] = acc[i];
+  }
   __syncthreads();
-  float* out = partial + ((size_t)g * kPoolSlices + slice) * kHidden;
-  for (int c = threadIdx.x; c < kHidden; c += blockDim.x) {
+  float* out = partial + ((size_t)g * kPoolSlices + slice) * kW;
+  for (int c = threadIdx.x; c < kW; c += blockDim.x) {
     float v = red[0][c];
 #pragma unroll
     for (int w = 1; w < kPoolWarps; ++w) v += red[w][c];
@@ -72,8 +90,8 @@ __global__ void k_pool_block_flags(const int32_t* __restrict__ graph_ptr, int64_
   if (p > 0) keep[(p - 1) >> 5] = 1;
 }
 
-// grid (G, kPoolSlices), 256 threads = 2 columns each; same partial[g][slice][512] layout as k_pool_partial
-template <typename T>
+// grid (G, kPoolSlices), kW / 2 threads = 2 columns each; same partial[g][slice][kW] layout as k_pool_partial
+template <typename T, int kW>
 __global__ void __launch_bounds__(256)
 k_pool_partial_blocks(const T* __restrict__ x, const float* __restrict__ block_sums, const uint8_t* __restrict__ keep,
                       const int32_t* __restrict__ graph_ptr, float* __restrict__ partial, int exclude_last) {
@@ -88,27 +106,29 @@ k_pool_partial_blocks(const T* __restrict__ x, const float* __restrict__ block_s
     const int32_t e_b = b0 + (int32_t)((int64_t)nb * (slice + 1) / kPoolSlices);
     for (int32_t b = s_b; b < e_b; ++b) {
       if (!keep[b]) {                                 // no graph starts or ends in this block: all 32 rows are ours
-        const float2 v = __ldg(reinterpret_cast<const float2*>(block_sums + (size_t)b * kHidden) + t);
+        const float2 v = __ldg(reinterpret_cast<const float2*>(block_sums + (size_t)b * kW) + t);
         a0 += v.x; a1 += v.y;
       } else {
         const int32_t r0 = max(beg, b << 5), r1 = min(end, (b << 5) + 32);
         for (int32_t r = r0; r < r1; ++r) {
-          const uint32_t u = *(reinterpret_cast<const uint32_t*>(x + (size_t)r * kHidden) + t);
+          const uint32_t u = *(reinterpret_cast<const uint32_t*>(x + (size_t)r * kW) + t);
           a0 = Pack16<T>::add_lo(u, a0); a1 = Pack16<T>::add_hi(u, a1);
         }
       }
     }
   }
-  reinterpret_cast<float2*>(partial + ((size_t)g * kPoolSlices + slice) * kHidden)[t] = make_float2(a0, a1);
+  reinterpret_cast<float2*>(partial + ((size_t)g * kPoolSlices + slice) * kW)[t] = make_float2(a0, a1);
 }
 
 template <typename T> BG_DEVINL float load_as_float(const T* p) {
   if constexpr (sizeof(T) == 4) return *p; else return (float)*p;
 }
 
-// one CTA per graph: pooled feature (512 or 1024 wide) -> optional MLPPooling Linear+ReLU
+// one CTA per graph: pooled feature (kW or 2 kW wide) -> optional MLPPooling Linear+ReLU
 // (Models/BuckGNN.py:568-581) -> decoder Linear(in,128) ReLU Linear(128,64) ReLU Linear(64,out)
-template <typename T>
+// (kW = 128: a model of hidden_channels 128, whose 2-layer decoder Linear(128,64) ReLU Linear(64,out) the caller
+// passes embedded in the 3-layer one: w1 = [W1; 0], w2 = [I64 | 0], b2 = 0)
+template <typename T, int kW>
 __global__ void __launch_bounds__(128)
 k_pool_head(const T* __restrict__ x, const float* __restrict__ partial, const int32_t* __restrict__ graph_ptr,
             int mode, const float* __restrict__ pre_w, const float* __restrict__ pre_b,
@@ -116,35 +136,35 @@ k_pool_head(const T* __restrict__ x, const float* __restrict__ partial, const in
             const float* __restrict__ w2, const float* __restrict__ b2,
             const float* __restrict__ w3, const float* __restrict__ b3, int out_dim,
             float* __restrict__ pred, float* __restrict__ pooled_out, const int32_t* __restrict__ nonfinite) {
-  __shared__ float feat[2 * kHidden];
-  __shared__ float tmp[kHidden];
+  __shared__ float feat[2 * kW];
+  __shared__ float tmp[kW];
   __shared__ float h1[128];
   __shared__ float h2[64];
   const int g = blockIdx.x, t = threadIdx.x;
   const int32_t n_g = graph_ptr[g + 1] - graph_ptr[g];
   const bool no_super = (mode == kPoolMeanNoSuper || mode == kPoolSuperWithPooling);
-  const int in_dim = (mode == kPoolSuperWithPooling) ? 2 * kHidden : kHidden;
+  const int in_dim = (mode == kPoolSuperWithPooling) ? 2 * kW : kW;
   if (mode != kPoolSuperOnly) {
     const float cnt = (float)max(n_g - (no_super ? 1 : 0), 1);
-    for (int c = t; c < kHidden; c += 128) {
-      const float* pp = partial + (size_t)g * kPoolSlices * kHidden + c;
+    for (int c = t; c < kW; c += 128) {
+      const float* pp = partial + (size_t)g * kPoolSlices * kW + c;
       float v = pp[0];
 #pragma unroll
-      for (int s = 1; s < kPoolSlices; ++s) v += pp[(size_t)s * kHidden];
+      for (int s = 1; s < kPoolSlices; ++s) v += pp[(size_t)s * kW];
       feat[c] = v / cnt;
     }
   }
   if (mode == kPoolSuperOnly || mode == kPoolSuperWithPooling) {
-    const int off = (mode == kPoolSuperOnly) ? 0 : kHidden;
-    const T* srow = x + (size_t)(graph_ptr[g + 1] - 1) * kHidden;
-    for (int c = t; c < kHidden; c += 128) feat[off + c] = (n_g > 0) ? load_as_float(srow + c) : 0.f;
+    const int off = (mode == kPoolSuperOnly) ? 0 : kW;
+    const T* srow = x + (size_t)(graph_ptr[g + 1] - 1) * kW;
+    for (int c = t; c < kW; c += 128) feat[off + c] = (n_g > 0) ? load_as_float(srow + c) : 0.f;
   }
   __syncthreads();
   if (pre_w) {                                   // pooling_mpl: relu(Linear(512,512)(mean))
-    for (int o = t; o < kHidden; o += 128) {
-      const float4* wr = reinterpret_cast<const float4*>(pre_w + (size_t)o * kHidden);
+    for (int o = t; o < kW; o += 128) {
+      const float4* wr = reinterpret_cast<const float4*>(pre_w + (size_t)o * kW);
       float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-      for (int k = 0; k < kHidden / 4; ++k) {
+      for (int k = 0; k < kW / 4; ++k) {
         const float4 w = __ldg(wr + k);
         a0 = fmaf(w.x, feat[4 * k], a0); a1 = fmaf(w.y, feat[4 * k + 1], a1);
         a2 = fmaf(w.z, feat[4 * k + 2], a2); a3 = fmaf(w.w, feat[4 * k + 3], a3);
@@ -152,7 +172,7 @@ k_pool_head(const T* __restrict__ x, const float* __restrict__ partial, const in
       tmp[o] = fmaxf((a0 + a1) + (a2 + a3) + pre_b[o], 0.f);
     }
     __syncthreads();
-    for (int c = t; c < kHidden; c += 128) feat[c] = tmp[c];
+    for (int c = t; c < kW; c += 128) feat[c] = tmp[c];
     __syncthreads();
   }
   if (pooled_out)

@@ -312,6 +312,17 @@ def gemm512(segs, m: int, precision: str, out: Activation, *, cta_group: int = 2
     out.refresh_split()
 
 
+def gemm(segs, m: int, precision: str, out: Activation, *, cta_group: int = 2, **epi) -> None:
+    """The update GEMM for the width of `out`: bg_gemm128 for 128-wide rows (a hidden_channels = 128 model on its own
+    kernels), else bg_gemm512."""
+    if out.data.shape[1] != 128:
+        return gemm512(segs, m, precision, out, cta_group=cta_group, **epi)
+    a_code, b_code = PRECISION_FORMATS[precision]
+    capi.gemm128(segs, m, a_code, b_code, out.data.data_ptr(), out.code, out.data.shape[1], _stream(),
+                 cta_group=cta_group, **epi)
+    out.refresh_split()
+
+
 def aggregate(x: Activation, out: Activation, idx: GraphIndex, aggr: str, fold_hubs: bool = True) -> None:
     """K2 over [N,512] rows, or [N,128] rows (the encoder hidden layer of the folded first layer)."""
     width = x.data.shape[1]
@@ -366,13 +377,16 @@ class FoldedLayer0Pack:
     bias_all_gated: Optional[torch.Tensor] = None   # HOST f32 [512]: bias + W_l b3, valid when every row's gate is 1
 
 
-def pack_folded_layer0(enc_last: torch.nn.Linear, conv, bn, aggr: str, precision: str) -> FoldedLayer0Pack:
+def pack_folded_layer0(enc_last: torch.nn.Linear, conv, bn, aggr: str, precision: str, width: int = 512) -> FoldedLayer0Pack:
+    """`width`: the layer's output width (512, or 128 for a hidden_channels = 128 model, whose encoder's last Linear
+    reads the 64-wide hidden layer stored 128 wide: W3 is zero-padded to 128 columns)."""
     dev = conv.lin_l.weight.device
     d64 = lambda t: t.detach().to(torch.float64).cpu()
     W3, b3 = d64(enc_last.weight), d64(enc_last.bias)
+    W3 = torch.nn.functional.pad(W3, (0, 128 - W3.shape[1]))
     Wl, bl, Wr = d64(conv.lin_l.weight), d64(conv.lin_l.bias), d64(conv.lin_r.weight)
     lp = lambda w: pack_linear(w.to(torch.float32).to(dev), precision)
-    gate = torch.cat([(Wl @ b3)[:, None], torch.zeros(512, 63, dtype=torch.float64)], 1)
+    gate = torch.cat([(Wl @ b3)[:, None], torch.zeros(width, 63, dtype=torch.float64)], 1)
     if aggr in ("sum", "add"):
         # the A operand carries deg_i as three base-256 digits (bg_expand_rowptr as_count): a super node's degree
         # (thousands) is not exact in 8 / 11 significant bits, its digits are
@@ -401,8 +415,8 @@ def sage_layer0_folded(h: "Activation", out: "Activation", idx: GraphIndex, w: F
         # indicator / degree digits are exact in tf32 (lo part 0): of the 3xTF32 products only hi*w_hi + hi*w_lo remain
         segs = segs + _segments(ind, w.wgate)[:2]
     with TIMERS.span("sage_update0"):
-        gemm512(segs, n, h.precision, out, cta_group=cta_group, bias=bias.data_ptr(), bn_scale=_p(w.bn_scale),
-                bn_shift=_p(w.bn_shift), normalize=normalize, relu=relu)
+        gemm(segs, n, h.precision, out, cta_group=cta_group, bias=bias.data_ptr(), bn_scale=_p(w.bn_scale),
+             bn_shift=_p(w.bn_shift), normalize=normalize, relu=relu)
 
 
 def encoder_forward(x: torch.Tensor, enc_w: Dict[str, torch.Tensor], w3: LinearPack, precision: str,
@@ -413,22 +427,22 @@ def encoder_forward(x: torch.Tensor, enc_w: Dict[str, torch.Tensor], w3: LinearP
     h = encoder_hidden(x, enc_w, precision, row_gather, nonfinite)
     n = h.data.shape[0]
     with TIMERS.span("encoder_gemm"):
-        gemm512(_segments(h, w3), n, precision, out, cta_group=cta_group, bias=enc_w["b3_host"].data_ptr())
+        gemm(_segments(h, w3), n, precision, out, cta_group=cta_group, bias=enc_w["b3_host"].data_ptr())
 
 
 @dataclass
 class PoolBlocks:
     """What a pool-fused last layer hands to `pool_head`: fp32 column sums of every 32-row block of the layer's
     output, and the flags of the blocks whose rows were stored as well (first / last row of a graph)."""
-    sums: torch.Tensor       # [ceil(N/32), 512] f32
+    sums: torch.Tensor       # [ceil(N/32), width] f32
     keep: torch.Tensor       # [ceil(N/32)] uint8
 
 
-def new_pool_blocks(idx: GraphIndex, device) -> PoolBlocks:
+def new_pool_blocks(idx: GraphIndex, device, width: int = 512) -> PoolBlocks:
     nb = (idx.n_nodes + 31) // 32
     keep = torch.empty(max(nb, 1), dtype=torch.uint8, device=device)
     capi.pool_block_flags(idx.graph_ptr.data_ptr(), idx.n_graphs, idx.n_nodes, keep.data_ptr(), _stream())
-    return PoolBlocks(torch.empty((max(nb, 1), 512), dtype=torch.float32, device=device), keep)
+    return PoolBlocks(torch.empty((max(nb, 1), width), dtype=torch.float32, device=device), keep)
 
 
 def can_fuse_pool(precision: str, normalize: bool, residual: bool) -> bool:
@@ -486,7 +500,7 @@ def sage_layer(x: Activation, agg: Activation, out: Activation, idx: GraphIndex,
     pool = {} if pool_blocks is None else dict(pool_block_sums=pool_blocks.sums.data_ptr(),
                                                pool_block_keep=pool_blocks.keep.data_ptr())
     with TIMERS.span("sage_update" if pool_blocks is None else "sage_update_pool"):
-        gemm512(segs, idx.n_nodes, x.precision, out, cta_group=cta_group,
+        gemm(segs, idx.n_nodes, x.precision, out, cta_group=cta_group,
                 bias=layer.bias.data_ptr(), bn_scale=_p(layer.bn_scale), bn_shift=_p(layer.bn_shift),
                 residual=x.data.data_ptr() if residual else None, ldr=x.data.shape[1],
                 normalize=normalize, relu=relu, **pool)
@@ -500,25 +514,27 @@ def pool_head(x: Activation, idx: GraphIndex, dec: Dict[str, torch.Tensor], out_
     dev = x.data.device
     g = idx.n_graphs
     mode = capi.POOL_MODES[pooling]
-    in_dim = 1024 if pooling == "supernode_with_pooling" else 512
+    width = x.data.shape[1]                  # 512, or 128: bg_pool_head128 / bg_pool_head_blocks128
+    in_dim = 2 * width if pooling == "supernode_with_pooling" else width
     pred = torch.empty((g, out_dim), dtype=torch.float32, device=dev)
     pooled = torch.empty((g, in_dim), dtype=torch.float32, device=dev) if want_pooled else None
     ws_bytes = capi.pool_workspace_bytes(g)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    head, head_blocks = (capi.pool_head128, capi.pool_head_blocks128) if width == 128 else (capi.pool_head, capi.pool_head_blocks)
     with TIMERS.span("pool_head"):
         if blocks is not None:
-            capi.pool_head_blocks(x.data.data_ptr(), x.code, idx.n_nodes, idx.graph_ptr.data_ptr(), g, mode,
-                                  _p(pre["w"]) if pre else None, _p(pre["b"]) if pre else None,
-                                  dec["w1"].data_ptr(), dec["b1"].data_ptr(), dec["w2"].data_ptr(), dec["b2"].data_ptr(),
-                                  dec["w3"].data_ptr(), dec["b3"].data_ptr(), out_dim, pred.data_ptr(), _p(pooled),
-                                  blocks.sums.data_ptr(), blocks.keep.data_ptr(), ws.data_ptr(), ws_bytes, _stream(),
-                                  nonfinite=_p(nonfinite))
+            head_blocks(x.data.data_ptr(), x.code, idx.n_nodes, idx.graph_ptr.data_ptr(), g, mode,
+                        _p(pre["w"]) if pre else None, _p(pre["b"]) if pre else None,
+                        dec["w1"].data_ptr(), dec["b1"].data_ptr(), dec["w2"].data_ptr(), dec["b2"].data_ptr(),
+                        dec["w3"].data_ptr(), dec["b3"].data_ptr(), out_dim, pred.data_ptr(), _p(pooled),
+                        blocks.sums.data_ptr(), blocks.keep.data_ptr(), ws.data_ptr(), ws_bytes, _stream(),
+                        nonfinite=_p(nonfinite))
         else:
-            capi.pool_head(x.data.data_ptr(), x.code, idx.n_nodes, idx.graph_ptr.data_ptr(), g, mode,
-                           _p(pre["w"]) if pre else None, _p(pre["b"]) if pre else None,
-                           dec["w1"].data_ptr(), dec["b1"].data_ptr(), dec["w2"].data_ptr(), dec["b2"].data_ptr(),
-                           dec["w3"].data_ptr(), dec["b3"].data_ptr(), out_dim, pred.data_ptr(), _p(pooled),
-                           ws.data_ptr(), ws_bytes, _stream(), nonfinite=_p(nonfinite))
+            head(x.data.data_ptr(), x.code, idx.n_nodes, idx.graph_ptr.data_ptr(), g, mode,
+                 _p(pre["w"]) if pre else None, _p(pre["b"]) if pre else None,
+                 dec["w1"].data_ptr(), dec["b1"].data_ptr(), dec["w2"].data_ptr(), dec["b2"].data_ptr(),
+                 dec["w3"].data_ptr(), dec["b3"].data_ptr(), out_dim, pred.data_ptr(), _p(pooled),
+                 ws.data_ptr(), ws_bytes, _stream(), nonfinite=_p(nonfinite))
     return pred, pooled
 
 

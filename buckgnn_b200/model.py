@@ -39,6 +39,9 @@ _SAGE_LISTS = {  # model_name -> (ModuleList attribute, aggr)      reference :12
     "GraphSage_meanAggr": ("sage_blocks_mean", "mean"),
     "GraphSage_maxAggr": ("sage_blocks_max", "max"),
 }
+_POOLINGS = ("mean", "mean_no_super", "supernode_only", "supernode_with_pooling", "mlp", "mlp_no_super")
+# models whose eval forward at hidden_channels == 128 runs on the 128-wide kernels (the rest use narrow.WideTwin)
+_NATIVE128_MODELS = tuple(_SAGE_LISTS) + ("GraphSage_addAggr_Shared", "GraphSAGE_MLP")
 
 
 class SAGEConv(nn.Module):
@@ -198,6 +201,7 @@ class BuckGNN(nn.Module):
         self._pack_sig = None
         self._index_cache = None
         self._wide = None                     # hidden_channels != 512: the zero-padded 512-wide twin (narrow.py), built lazily
+        self._ran_native128 = False           # the last forward ran on the 128-wide kernels (check_finite reads self)
         self._param_inputs = None             # set by narrow.WideTwin around a train-mode forward of the twin
 
     # ------------------------------------------------------------------ weight packing
@@ -277,6 +281,54 @@ class BuckGNN(nn.Module):
         self._packs, self._pack_sig = packs, sig
         return packs
 
+    def _packed128(self):
+        """Operand-format copies for the 128-wide kernels (hidden_channels == 128, eval), rebuilt when any parameter /
+        buffer changes.  The 2-layer encoder / decoder of h <= 128 (Models/BuckGNN.py:41-65) run on the 3-layer
+        kernels by exact embedding: encoder Linear(F,64) ReLU [I; 0] ReLU (the 64-wide hidden layer stored 128 wide),
+        then its Linear(64,128) padded to [128,128]; decoder [W1; 0] ReLU [I64 | 0] ReLU W2."""
+        sig = self._signature()
+        if self._pack_sig == sig:
+            return self._packs
+        prec = self.precision
+        f32 = lambda t: t.detach().float().contiguous()
+        enc, dec = self.node_encoder, self.decoder
+        dev = enc[0].weight.device
+        eye = torch.eye(64, device=dev)
+        zeros = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=dev)
+        w2 = zeros(128, 64)
+        w2[:64] = eye
+        packs = {"enc": {"w1": f32(enc[0].weight), "b1": f32(enc[0].bias), "w2": w2, "b2": zeros(128),
+                         "b3_host": engine.host_vector(enc[2].bias)},
+                 "enc_w3": engine.pack_linear(torch.nn.functional.pad(f32(enc[2].weight), (0, 64)), prec)}
+        w1, b1 = zeros(128, dec[0].in_features), zeros(128)
+        w1[:64], b1[:64] = f32(dec[0].weight), f32(dec[0].bias)
+        i64 = zeros(64, 128)
+        i64[:, :64] = eye
+        packs["dec"] = {"w1": w1, "b1": b1, "w2": i64, "b2": zeros(64), "w3": f32(dec[2].weight), "b3": f32(dec[2].bias)}
+        mpl = self.pooling_mpl.mlp[0]
+        packs["pool_mlp"] = {"w": f32(mpl.weight), "b": f32(mpl.bias)}
+        layers, seen = [], {}
+        for conv, bn in self._sage_layers():
+            if id(conv) not in seen:
+                scale, shift = engine.fold_batchnorm(bn) if bn is not None else (None, None)
+                seen[id(conv)] = SageLayerPack(engine.pack_linear(conv.lin_l.weight, prec),
+                                               engine.pack_linear(conv.lin_r.weight, prec),
+                                               engine.host_vector(conv.lin_l.bias), scale, shift)
+            layers.append(seen[id(conv)])
+        packs["layers"] = layers
+        folded = None
+        sl = self._sage_layers()
+        if self.fold_encoder and sl and sl[0][0].aggr != "max":
+            conv0, bn0 = sl[0]
+            folded = engine.pack_folded_layer0(enc[2], conv0, bn0, conv0.aggr, prec, width=128)
+            # a folded weight its storage format cannot hold (fp16, sum / add: the degree digits' gate columns carry
+            # W_l b3 x 65536) would turn every prediction into NaN: run layer 0 unfolded instead
+            if not all(bool(torch.isfinite(t).all()) for pk in (folded.wl3, folded.wr3, folded.wgate) for t in pk.parts):
+                folded = None
+        packs["layer0_folded"] = folded
+        self._packs, self._pack_sig = packs, sig
+        return packs
+
     # ------------------------------------------------------------------ forward
     def _check_model_name(self):
         if self.model_name in ("GraphSage_MLP", "GraphSage_addAggr_woBatchNorm", "GraphSage_sumAggr_woBatchNorm"):
@@ -292,8 +344,21 @@ class BuckGNN(nn.Module):
             raise NotImplementedError("buckgnn_b200: the tcgen05 path holds one 512-column row per TMEM lane; "
                                       "hidden_channels > 512 is not built")
 
+    def _runs_native128(self) -> bool:
+        """hidden_channels == 128 eval forwards of the GraphSAGE models with a graph-level head run on the 128-wide
+        kernels; everything else at a width other than 512 runs on the zero-padded twin (narrow.py)."""
+        return (self.hidden_channels == 128 and not self.training and not self.fuse_aggregate
+                and self.model_name in _NATIVE128_MODELS and self.prediction_type == "buckling"
+                and self.pooling_layer in _POOLINGS)
+
     def forward(self, x, edge_index, edge_attr, batch=None, mask=None):
         self._check_supported(x)
+        self._ran_native128 = False
+        if self._runs_native128():
+            with torch.no_grad():
+                pred = self._forward_cuda(x, edge_index, batch, width=128)
+            self._ran_native128 = True
+            return pred.squeeze(), batch
         if self.hidden_channels != 512:
             # TRAIN_FINAL.py:55,71 / the constructor default use 128: runs as the exact zero-padded 512-wide twin.
             # 129..255 build no encoder in the reference (Models/BuckGNN.py:41,67): the same AttributeError surfaces here.
@@ -301,14 +366,16 @@ class BuckGNN(nn.Module):
                 self.node_encoder                                    # AttributeError for 129 <= hidden <= 255, as the reference
                 from .narrow import WideTwin
                 self._wide = WideTwin(self, self._ctor_kwargs)
-            return self._wide.forward(x, edge_index, edge_attr, batch)
+            out = self._wide.forward(x, edge_index, edge_attr, batch)
+            if self.training:
+                self._pack_sig = None            # BatchNorm statistics changed: the next native eval forward repacks
+            return out
         node_level = "static" in self.prediction_type or "mode_shape" in self.prediction_type
         if self.prediction_type != "buckling" and not node_level:
             raise ValueError(f"Unknown prediction type: {self.prediction_type}")
         if node_level and self.hidden_channels < 256:
             raise NotImplementedError("buckgnn_b200: node-level heads need the 3-layer decoder (hidden_channels >= 256)")
-        if not node_level and self.pooling_layer not in ("mean", "mean_no_super", "supernode_only",
-                                                          "supernode_with_pooling", "mlp", "mlp_no_super"):
+        if not node_level and self.pooling_layer not in _POOLINGS:
             if self.pooling_layer == "hybrid":
                 raise AttributeError("'BuckGNN' object has no attribute 'hybrid_pooling'")   # reference :188,276
             raise ValueError(f"Unknown pooling layer: {self.pooling_layer}")
@@ -367,7 +434,7 @@ class BuckGNN(nn.Module):
     def check_finite(self) -> None:
         """Raises FloatingPointError if the last eval-mode forward met activations its 16-bit storage format cannot
         hold (synchronises; the forward itself reports the condition as NaN predictions without a sync)."""
-        target = self._wide.twin if self._wide is not None else self
+        target = self._wide.twin if self._wide is not None and not self._ran_native128 else self
         flag = getattr(target, "_nonfinite", None)
         if flag is not None and int(flag.item()) != 0:
             raise FloatingPointError(f"buckgnn_b200: activations left the range of precision={target.precision!r} storage "
@@ -436,13 +503,14 @@ class BuckGNN(nn.Module):
                                    nonfinite=flag)
         return pred
 
-    def _forward_cuda(self, x, edge_index, batch, node_level=False):
-        packs = self._packed()
+    def _forward_cuda(self, x, edge_index, batch, node_level=False, width=512):
+        """`width` 128: a hidden_channels = 128 model on the 128-wide kernels (bg_gemm128, bg_pool_head128)."""
+        packs = self._packed() if width == 512 else self._packed128()
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         n = x.shape[0]
         pending = self._begin_graph_index(edge_index, batch, n)       # K1 enqueued, result read-back in flight
-        cur = Activation(n, 512, prec, x.device)
+        cur = Activation(n, width, prec, x.device)
         layers = packs["layers"]
         folded = packs["layer0_folded"]
         flag = self._new_nonfinite_flag(x.device)
@@ -453,8 +521,8 @@ class BuckGNN(nn.Module):
         idx = pending.finish()                                        # host sync hidden behind the encoder
         blocks = None
         if layers:
-            nxt = Activation(n, 512, prec, x.device)
-            agg = Activation(n, 512, prec, x.device)
+            nxt = Activation(n, width, prec, x.device)
+            agg = Activation(n, width, prec, x.device)
             aggr = self._sage_layers()[0][0].aggr
             L = len(layers)
             for i, layer in enumerate(layers):                                            # reference :445-458
@@ -467,7 +535,7 @@ class BuckGNN(nn.Module):
                     # its epilogue sums them per 32-row block instead of storing them (16-bit modes)
                     if (i == L - 1 and not node_level and self.fuse_pool
                             and engine.can_fuse_pool(prec, True, residual)):
-                        blocks = engine.new_pool_blocks(idx, x.device)
+                        blocks = engine.new_pool_blocks(idx, x.device, width)
                     engine.sage_layer(cur, agg, nxt, idx, layer, aggr=aggr, normalize=True, relu=True,
                                       residual=residual, cta_group=cg, pool_blocks=blocks,
                                       fuse_aggregate=self.fuse_aggregate)

@@ -219,6 +219,15 @@ int bg_sage_fused512(const bg_gemm_segment* segments_host, int32_t n_segments, i
                      int a_dtype, int b_dtype, const bg_epilogue* epilogue_host, const bg_fused_aggregate* fused_host,
                      void* out, int out_dtype, int64_t ldo, void* stream);
 
+/* The update GEMM at width 128 (a model with hidden_channels = 128, the reference's default):
+ *    out[m, 0:128] = epilogue( sum_s A_s[m, :] . B_s[:, :]^T ),   B_s [128, k_s] (nn.Linear weight layout)
+ * Same arguments, operand formats, K rules and epilogue order as bg_gemm512, with 128 for 512 throughout: the
+ * epilogue's host vectors are [128], residual / out rows are [M,128] (ld >= 128), pool_block_sums is [ceil(M/32), 128].
+ * Not built at this width (BG_ERR_UNSUPPORTED): gathered addends and b_groups > 1. */
+int bg_gemm128(const bg_gemm_segment* segments_host, int32_t n_segments, int64_t m,
+               int a_dtype, int b_dtype, const bg_epilogue* epilogue_host,
+               void* out, int out_dtype, int64_t ldo, int cta_group, void* stream);
+
 /* Aggregates of the hub rows only, compact: hub_out[b, :] = reduce over the neighbours of node big_rows[b] (mean / sum,
  * 16-bit rows).  workspace: bg_aggregate_workspace_bytes(n_big). */
 int bg_sage_aggregate_hubs(const void* x, int dtype, const int32_t* rowptr, const int32_t* col, const int32_t* big_rows,
@@ -270,6 +279,24 @@ int bg_pool_head_blocks(const void* x, int dtype, int64_t n_nodes, const int32_t
                         const float* w3, const float* b3, int32_t out_dim,
                         float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
                         void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream);
+
+/* bg_pool_head / bg_pool_head_blocks for x [N,128] (hidden_channels = 128): same arguments and pooling modes;
+ * the pooled feature is 128 wide (256 for BG_POOL_SUPERNODE_WITH_POOLING), pre_w / pre_b are [128,128] / [128],
+ * w1 is [128, in], block_sums [ceil(N/32), 128].  The decoder is the same 3-layer head: a 2-layer
+ * Linear(in,64) ReLU Linear(64,out) runs exactly as w1 = [W1; 0] (rows padded to 128), b1 = [b1; 0], w2 = [I64 | 0],
+ * b2 = 0, w3 = W2, b3 = b2. */
+int bg_pool_head128(const void* x, int dtype, int64_t n_nodes, const int32_t* graph_ptr, int64_t n_graphs,
+                    int pool_mode, const float* pre_w, const float* pre_b,
+                    const float* w1, const float* b1, const float* w2, const float* b2,
+                    const float* w3, const float* b3, int32_t out_dim,
+                    float* pred, float* pooled_out,
+                    void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream);
+int bg_pool_head_blocks128(const void* x, int dtype, int64_t n_nodes, const int32_t* graph_ptr, int64_t n_graphs,
+                           int pool_mode, const float* pre_w, const float* pre_b,
+                           const float* w1, const float* b1, const float* w2, const float* b2,
+                           const float* w3, const float* b3, int32_t out_dim,
+                           float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
+                           void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream);
 
 /* ------------------------------------------------------------------ EA-GNN helpers
  * bg_expand_rowptr: row_of[i] = r with rowptr[r] <= i < rowptr[r+1], iota[i] = i   (i < E)
