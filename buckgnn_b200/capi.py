@@ -39,6 +39,8 @@ EXPORTED_SYMBOLS = (
     "bg_dropout_residual", "bg_grad_mask", "bg_segment_expand",
     "bg_sag_workspace_bytes", "bg_sag_select", "bg_sag_connect", "bg_gather_rows", "bg_index_invert", "bg_index_gather",
     "bg_sag_pool_backward", "bg_max_aggregate_backward", "bg_max_bwd_workspace_bytes",
+    "bg_bn_batch_stats128", "bg_bn_act_forward128", "bg_sage_backward_rows128", "bg_pool_backward128",
+    "bg_max_aggregate_backward128", "bg_wgrad128",
 )
 
 
@@ -142,6 +144,15 @@ _SIGNATURES = {
     "bg_max_bwd_workspace_bytes": (C.c_int, [_I32, _I32, _SZP]),
     "bg_max_aggregate_backward": (C.c_int, [_P, _P, _P, C.c_int, _I64, _P, _P, _P, _I32, _P, _P, _P, _I32, _P, _P, _P, C.c_size_t, _P]),
     "bg_sag_pool_backward": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _P, _P, _P, C.c_float, _P, _P, _P, _I32, _P, _P, _P, _P, _P, _P]),
+    "bg_bn_batch_stats128": (C.c_int, [_P, C.c_int, _I64, _P, _P, C.c_float, C.c_float, _P, _P, _P, _P, _P, _P, _P,
+                                       _P, C.c_size_t, _P]),
+    "bg_bn_act_forward128": (C.c_int, [_P, _P, _P, C.c_int, _I64, _P, _P, C.c_float, C.c_uint64, _P]),
+    "bg_sage_backward_rows128": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, _I64, _P, _P, _P, _P, C.c_float, C.c_uint64,
+                                           _P, _P, C.c_int, _P, _P, _P, _P, C.c_size_t, _P]),
+    "bg_pool_backward128": (C.c_int, [_P, _I64, _P, _I64, C.c_int, _I64, _P, C.c_int, _P]),
+    "bg_max_aggregate_backward128": (C.c_int, [_P, _P, _P, C.c_int, _I64, _P, _P, _P, _I32, _P, _P, _P, _I32, _P, _P, _P,
+                                               C.c_size_t, _P]),
+    "bg_wgrad128": (C.c_int, [_P, _P, _P, C.c_int, _I64, _I32, _I64, _P, _P, _P, C.c_int, _P]),
 }
 
 
@@ -350,23 +361,30 @@ def train_workspace_bytes(n_rows: int) -> int:
     return _query("bg_train_workspace_bytes", n_rows)
 
 
+def _w(name: str, width: int) -> str:
+    """Entry point of a training-step kernel for the row width: `name` (512) or `name`128."""
+    if width not in (512, 128):
+        raise ValueError(f"{name}: width must be 512 or 128, got {width}")
+    return name if width == 512 else name + "128"
+
+
 def bn_batch_stats(u, dtype, n_rows, gamma, beta, eps, momentum, running_mean, running_var, num_batches_tracked,
-                   a_out, shift_out, mean_out, invstd_out, ws, ws_bytes, stream):
-    _check(load().bg_bn_batch_stats(u, dtype, n_rows, gamma, beta, eps, momentum, running_mean, running_var,
-                                    num_batches_tracked, a_out, shift_out, mean_out, invstd_out, ws, ws_bytes,
-                                    stream), "bg_bn_batch_stats")
+                   a_out, shift_out, mean_out, invstd_out, ws, ws_bytes, stream, width=512):
+    fn = _w("bg_bn_batch_stats", width)
+    _check(getattr(load(), fn)(u, dtype, n_rows, gamma, beta, eps, momentum, running_mean, running_var,
+                               num_batches_tracked, a_out, shift_out, mean_out, invstd_out, ws, ws_bytes, stream), fn)
 
 
-def bn_act_forward(u, x_prev, y, dtype, n_rows, a, shift, dropout_p, seed, stream):
-    _check(load().bg_bn_act_forward(u, x_prev, y, dtype, n_rows, a, shift, dropout_p, seed, stream),
-           "bg_bn_act_forward")
+def bn_act_forward(u, x_prev, y, dtype, n_rows, a, shift, dropout_p, seed, stream, width=512):
+    fn = _w("bg_bn_act_forward", width)
+    _check(getattr(load(), fn)(u, x_prev, y, dtype, n_rows, a, shift, dropout_p, seed, stream), fn)
 
 
 def sage_backward_rows(u, dy, dy2, inv_norm, rowptr, dtype, n_rows, a, shift, mean, invstd, dropout_p, seed,
-                       dgamma, dbeta, accumulate, dz, dz_scaled, g_out, ws, ws_bytes, stream):
-    _check(load().bg_sage_backward_rows(u, dy, dy2, inv_norm, rowptr, dtype, n_rows, a, shift, mean, invstd,
-                                        dropout_p, seed, dgamma, dbeta, int(bool(accumulate)), dz, dz_scaled, g_out,
-                                        ws, ws_bytes, stream), "bg_sage_backward_rows")
+                       dgamma, dbeta, accumulate, dz, dz_scaled, g_out, ws, ws_bytes, stream, width=512):
+    fn = _w("bg_sage_backward_rows", width)
+    _check(getattr(load(), fn)(u, dy, dy2, inv_norm, rowptr, dtype, n_rows, a, shift, mean, invstd, dropout_p, seed,
+                               dgamma, dbeta, int(bool(accumulate)), dz, dz_scaled, g_out, ws, ws_bytes, stream), fn)
 
 
 def transpose_chunks(src, dtype, n_rows, n_cols, ld, n_chunks, chunk_k, out, stream, out_rows_per_chunk=0):
@@ -390,9 +408,9 @@ def colsum(src, dtype, rows, cols, ld, out, accumulate, ws, ws_bytes, stream):
     _check(load().bg_colsum(src, dtype, rows, cols, ld, out, int(bool(accumulate)), ws, ws_bytes, stream), "bg_colsum")
 
 
-def pool_backward(dpooled, ldp, graph_ptr, n_graphs, pool_mode, n_nodes, dx, dtype, stream):
-    _check(load().bg_pool_backward(dpooled, ldp, graph_ptr, n_graphs, pool_mode, n_nodes, dx, dtype, stream),
-           "bg_pool_backward")
+def pool_backward(dpooled, ldp, graph_ptr, n_graphs, pool_mode, n_nodes, dx, dtype, stream, width=512):
+    fn = _w("bg_pool_backward", width)
+    _check(getattr(load(), fn)(dpooled, ldp, graph_ptr, n_graphs, pool_mode, n_nodes, dx, dtype, stream), fn)
 
 
 def sgemm_workspace_bytes(m: int, n: int, k: int) -> int:
@@ -433,6 +451,12 @@ def expand_wire(wire_edges, e_wire, node_ptr, wire_ptr, full_ptr, n_graphs, e_fu
 def wgrad512(dz, ld_dz, act, act_cols, ld_act, dtype, n_rows, n_chunks, chunk_k, partial, stream):
     _check(load().bg_wgrad512(dz, ld_dz, act, act_cols, ld_act, dtype, n_rows, n_chunks, chunk_k, partial, stream),
            "bg_wgrad512")
+
+
+def wgrad128(dz, agg, x, dtype, n_rows, n_chunks, chunk_k, partial, dwl, dwr, accumulate, stream):
+    """bg_wgrad128: dwl (+)= dz^T agg, dwr (+)= dz^T x for [n_rows, 128] rows; partial [n_chunks * 256, 128] f32."""
+    _check(load().bg_wgrad128(dz, agg, x, dtype, n_rows, n_chunks, chunk_k, partial, dwl, dwr, int(bool(accumulate)),
+                              stream), "bg_wgrad128")
 
 
 def dropout_residual(x, x_prev, y, dtype, n_rows, dropout_p, seed, stream):
@@ -488,7 +512,7 @@ def max_bwd_workspace_bytes(n_big_tgt: int, n_big_src: int) -> int:
 
 
 def max_aggregate_backward(x, agg, dagg, dtype, n_nodes, rowptr_tgt, col_tgt, big_tgt, n_big_tgt, rowptr_src, col_src,
-                           big_src, n_big_src, w_scratch, dx, ws, ws_bytes, stream):
-    _check(load().bg_max_aggregate_backward(x, agg, dagg, dtype, n_nodes, rowptr_tgt, col_tgt, big_tgt, n_big_tgt,
-                                            rowptr_src, col_src, big_src, n_big_src, w_scratch, dx, ws, ws_bytes, stream),
-           "bg_max_aggregate_backward")
+                           big_src, n_big_src, w_scratch, dx, ws, ws_bytes, stream, width=512):
+    fn = _w("bg_max_aggregate_backward", width)
+    _check(getattr(load(), fn)(x, agg, dagg, dtype, n_nodes, rowptr_tgt, col_tgt, big_tgt, n_big_tgt, rowptr_src, col_src,
+                               big_src, n_big_src, w_scratch, dx, ws, ws_bytes, stream), fn)

@@ -299,7 +299,7 @@ static void pool_blocks_launch(const T* x, const int32_t* graph_ptr, int64_t G, 
 
 using namespace bg;
 
-template <typename T>
+template <typename T, int kW>
 static void launch_max_bwd(const void* x, const void* agg, const void* dagg, int64_t N, const int32_t* rowptr_tgt,
                            const int32_t* col_tgt, const int32_t* big_tgt, int32_t n_big_tgt, const int32_t* rowptr_src,
                            const int32_t* col_src, const int32_t* big_src, int32_t n_big_src, void* w_scratch, void* dx,
@@ -307,16 +307,16 @@ static void launch_max_bwd(const void* x, const void* agg, const void* dagg, int
   const T* xp = static_cast<const T*>(x); const T* ap = static_cast<const T*>(agg); const T* dp = static_cast<const T*>(dagg);
   T* wp = static_cast<T*>(w_scratch); T* op = static_cast<T*>(dx);
   // pass 1 (by target): w_i = dagg_i / n_i
-  k_max_bwd_rows<T, 0><<<grid, kMaxBwdWarps * 32, 0, stream>>>(ap, xp, nullptr, dp, rowptr_tgt, col_tgt, N, wp);
+  k_max_bwd_rows<T, 0, kW><<<grid, kMaxBwdWarps * 32, 0, stream>>>(ap, xp, nullptr, dp, rowptr_tgt, col_tgt, N, wp);
   if (n_big_tgt > 0) {
-    k_max_bwd_big<T, 0><<<dim3((unsigned)n_big_tgt, kMaxBwdSlices), kMaxBwdBigWarps * 32, 0, stream>>>(ap, xp, nullptr, rowptr_tgt, col_tgt, big_tgt, partial);
-    k_max_bwd_big_finish<T, 0><<<(unsigned)n_big_tgt, 32, 0, stream>>>(ap, dp, big_tgt, partial, wp);
+    k_max_bwd_big<T, 0, kW><<<dim3((unsigned)n_big_tgt, kMaxBwdSlices), kMaxBwdBigWarps * 32, 0, stream>>>(ap, xp, nullptr, rowptr_tgt, col_tgt, big_tgt, partial);
+    k_max_bwd_big_finish<T, 0, kW><<<(unsigned)n_big_tgt, 32, 0, stream>>>(ap, dp, big_tgt, partial, wp);
   }
   // pass 2 (by source): dx_j = sum_i [agg_i == x_j] w_i
-  k_max_bwd_rows<T, 1><<<grid, kMaxBwdWarps * 32, 0, stream>>>(xp, ap, wp, nullptr, rowptr_src, col_src, N, op);
+  k_max_bwd_rows<T, 1, kW><<<grid, kMaxBwdWarps * 32, 0, stream>>>(xp, ap, wp, nullptr, rowptr_src, col_src, N, op);
   if (n_big_src > 0) {
-    k_max_bwd_big<T, 1><<<dim3((unsigned)n_big_src, kMaxBwdSlices), kMaxBwdBigWarps * 32, 0, stream>>>(xp, ap, wp, rowptr_src, col_src, big_src, partial);
-    k_max_bwd_big_finish<T, 1><<<(unsigned)n_big_src, 32, 0, stream>>>(xp, nullptr, big_src, partial, op);
+    k_max_bwd_big<T, 1, kW><<<dim3((unsigned)n_big_src, kMaxBwdSlices), kMaxBwdBigWarps * 32, 0, stream>>>(xp, ap, wp, rowptr_src, col_src, big_src, partial);
+    k_max_bwd_big_finish<T, 1, kW><<<(unsigned)n_big_src, 32, 0, stream>>>(xp, nullptr, big_src, partial, op);
   }
 }
 
@@ -793,6 +793,41 @@ int bg_wgrad512(const void* dz, int64_t ld_dz, const void* act, int32_t act_cols
   return launch_gemm512<2, float, kAddNone, false>(p, stream);
 }
 
+int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64_t n_rows, int32_t n_chunks, int64_t chunk_k,
+                float* partial, float* dwl, float* dwr, int accumulate, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  // every argument is checked before the first CUDA call
+  const int fmt = umma_format_of(dtype);
+  if (fmt < 0) return fail(BG_ERR_INVALID, "bg_wgrad128: bad dtype");
+  const int esz = fmt == 2 ? 4 : 2;
+  const int kblk = kStageKBytes / esz;                     // nodes per pipeline stage: 64 (16-bit) / 32 (tf32)
+  if (n_rows <= 0 || n_chunks <= 0 || chunk_k <= 0 || chunk_k % kblk != 0 || (int64_t)n_chunks * chunk_k < n_rows ||
+      (int64_t)n_chunks * chunk_k >= 0x7fffffffLL)
+    return fail(BG_ERR_INVALID, "bg_wgrad128: chunk_k must be a multiple of 64 (16-bit) / 32 (tf32) and n_chunks*chunk_k >= n_rows");
+  if (!dz || !agg || !x || !partial || !dwl || !dwr || !aligned16(dz) || !aligned16(agg) || !aligned16(x) || !aligned16(partial))
+    return fail(BG_ERR_INVALID, "bg_wgrad128: null or misaligned pointer");
+  Gemm128Params p;
+  memset(&p, 0, sizeof(p));
+  int rc = make_mn_operand_map(&p.seg[0].a, agg, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
+  if (rc == BG_OK) rc = make_mn_operand_map(&p.seg[1].a, x, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
+  if (rc == BG_OK) rc = make_mn_operand_map(&p.seg[0].b, dz, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
+  if (rc != BG_OK) return fail(rc, "bg_wgrad128: cuTensorMapEncodeTiled failed");
+  p.n_seg = 1;                                             // the MMA warp walks segment 0's K blocks; rank 1 reads seg[1].a
+  p.kblocks[0] = (int32_t)(chunk_k / kblk);
+  p.k_elems_per_block = kblk;
+  p.a_fmt = p.b_fmt = (uint32_t)fmt;
+  p.chunk_k = chunk_k;
+  p.n_tiles = n_chunks;
+  p.m = (int64_t)n_chunks * 2 * kW128;
+  for (int i = 0; i < kW128; ++i) { p.bias[i] = 0.f; p.scale[i] = 1.f; p.shift[i] = 0.f; }
+  p.out = partial; p.ldo = kW128;
+  rc = launch_gemm128<float, false, false, true>(p, stream);
+  if (rc != BG_OK) return rc;
+  k_reduce_wgrad128<<<grid_for(2 * kW128 * kW128, 256, sm_count() * 4), 256, 0, stream>>>(partial, n_chunks, dwl, dwr, accumulate);
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+
 // ------------------------------------------------------------------ K4
 int bg_pool_workspace_bytes(int64_t G, size_t* bytes_host) {
   if (!bytes_host || G < 0) return fail(BG_ERR_INVALID, "bg_pool_workspace_bytes: bad argument");
@@ -1068,25 +1103,50 @@ int bg_max_bwd_workspace_bytes(int32_t n_big_tgt, int32_t n_big_src, size_t* byt
   return BG_OK;
 }
 
+static int max_aggregate_backward_impl(const char* fn, int width, const void* x, const void* agg, const void* dagg, int dtype,
+                                       int64_t N, const int32_t* rowptr_tgt, const int32_t* col_tgt, const int32_t* big_tgt,
+                                       int32_t n_big_tgt, const int32_t* rowptr_src, const int32_t* col_src,
+                                       const int32_t* big_src, int32_t n_big_src, void* w_scratch, void* dx, void* workspace,
+                                       size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (N < 0 || n_big_tgt < 0 || n_big_src < 0) return fail_in(BG_ERR_INVALID, fn, "bad size");
+  if (N == 0) return BG_OK;
+  if (!x || !agg || !dagg || !rowptr_tgt || !rowptr_src || !w_scratch || !dx || !aligned16(x) || !aligned16(agg) ||
+      !aligned16(dagg) || !aligned16(w_scratch) || !aligned16(dx) || (n_big_tgt > 0 && !big_tgt) || (n_big_src > 0 && !big_src))
+    return fail_in(BG_ERR_INVALID, fn, "null or misaligned pointer");
+  size_t need = 0;
+  bg_max_bwd_workspace_bytes(n_big_tgt, n_big_src, &need);
+  if ((n_big_tgt > 0 || n_big_src > 0) && (!workspace || workspace_bytes < need))
+    return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
+  if (width != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  const unsigned grid = grid_for(N * 32, kMaxBwdWarps * 32, sm_count() * 8);
+  if (width == kHidden) {
+    BG_BY_DTYPE(dtype, (launch_max_bwd<T, kHidden>(x, agg, dagg, N, rowptr_tgt, col_tgt, big_tgt, n_big_tgt, rowptr_src, col_src,
+                                                   big_src, n_big_src, w_scratch, dx, static_cast<float*>(workspace), grid, stream)));
+  } else {
+    BG_BY_DTYPE(dtype, (launch_max_bwd<T, kW128>(x, agg, dagg, N, rowptr_tgt, col_tgt, big_tgt, n_big_tgt, rowptr_src, col_src,
+                                                 big_src, n_big_src, w_scratch, dx, static_cast<float*>(workspace), grid, stream)));
+  }
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+
 int bg_max_aggregate_backward(const void* x, const void* agg, const void* dagg, int dtype, int64_t N,
                               const int32_t* rowptr_tgt, const int32_t* col_tgt, const int32_t* big_tgt, int32_t n_big_tgt,
                               const int32_t* rowptr_src, const int32_t* col_src, const int32_t* big_src, int32_t n_big_src,
                               void* w_scratch, void* dx, void* workspace, size_t workspace_bytes, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || n_big_tgt < 0 || n_big_src < 0) return fail(BG_ERR_INVALID, "bg_max_aggregate_backward: bad size");
-  if (N == 0) return BG_OK;
-  if (!x || !agg || !dagg || !rowptr_tgt || !rowptr_src || !w_scratch || !dx || !aligned16(x) || !aligned16(agg) ||
-      !aligned16(dagg) || !aligned16(w_scratch) || !aligned16(dx) || (n_big_tgt > 0 && !big_tgt) || (n_big_src > 0 && !big_src))
-    return fail(BG_ERR_INVALID, "bg_max_aggregate_backward: null or misaligned pointer");
-  size_t need = 0;
-  bg_max_bwd_workspace_bytes(n_big_tgt, n_big_src, &need);
-  if ((n_big_tgt > 0 || n_big_src > 0) && (!workspace || workspace_bytes < need))
-    return fail(BG_ERR_WORKSPACE, "bg_max_aggregate_backward: workspace too small");
-  const unsigned grid = grid_for(N * 32, kMaxBwdWarps * 32, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (launch_max_bwd<T>(x, agg, dagg, N, rowptr_tgt, col_tgt, big_tgt, n_big_tgt, rowptr_src, col_src, big_src,
-                                        n_big_src, w_scratch, dx, static_cast<float*>(workspace), grid, stream)));
-  BG_LAUNCH_OK();
-  return BG_OK;
+  return max_aggregate_backward_impl("bg_max_aggregate_backward", kHidden, x, agg, dagg, dtype, N, rowptr_tgt, col_tgt, big_tgt,
+                                     n_big_tgt, rowptr_src, col_src, big_src, n_big_src, w_scratch, dx, workspace,
+                                     workspace_bytes, stream_);
+}
+
+int bg_max_aggregate_backward128(const void* x, const void* agg, const void* dagg, int dtype, int64_t N,
+                                 const int32_t* rowptr_tgt, const int32_t* col_tgt, const int32_t* big_tgt, int32_t n_big_tgt,
+                                 const int32_t* rowptr_src, const int32_t* col_src, const int32_t* big_src, int32_t n_big_src,
+                                 void* w_scratch, void* dx, void* workspace, size_t workspace_bytes, void* stream_) {
+  return max_aggregate_backward_impl("bg_max_aggregate_backward128", kW128, x, agg, dagg, dtype, N, rowptr_tgt, col_tgt,
+                                     big_tgt, n_big_tgt, rowptr_src, col_src, big_src, n_big_src, w_scratch, dx, workspace,
+                                     workspace_bytes, stream_);
 }
 
 int bg_gather_rows(const void* x, int dtype, int64_t ldx, const int32_t* row_index, const float* row_scale,
@@ -1128,83 +1188,141 @@ int bg_train_workspace_bytes(int64_t N, size_t* bytes_host) {
   return BG_OK;
 }
 
+extern "C++" {
+template <int kW>
+static int bn_batch_stats_impl(const char* fn, const void* u, int dtype, int64_t N, const float* gamma, const float* beta,
+                               float eps, float momentum, float* running_mean, float* running_var, int64_t* num_batches_tracked,
+                               float* a_out, float* shift_out, float* mean_out, float* invstd_out,
+                               void* workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (N <= 0) return fail_in(BG_ERR_INVALID, fn, "needs at least one row");
+  if (!u || !aligned16(u) || !gamma || !beta || !a_out || !shift_out || !mean_out || !invstd_out)
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  if ((running_mean != nullptr) != (running_var != nullptr)) return fail_in(BG_ERR_INVALID, fn, "running_mean and running_var go together");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  size_t need = 0;
+  bg_train_workspace_bytes(N, &need);
+  if (!workspace || workspace_bytes < need) return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
+  float* partial = static_cast<float*>(workspace);
+  const int grid = stat_grid(N);
+  const DropArgs nodrop = drop_args(0.f, 0);
+  BG_BY_DTYPE(dtype, (k_col_stats<T, 0, kW><<<grid, kStatWarps * 32, 0, stream>>>(static_cast<const T*>(u), nullptr, nullptr, N,
+                                                                              nullptr, nullptr, nodrop, partial)))
+  BG_LAUNCH_OK();
+  BnVectors out{a_out, shift_out, mean_out, invstd_out};
+  k_bn_fwd_finalize<kW><<<kW / 64, kHidden, 0, stream>>>(partial, grid, N, gamma, beta, eps, momentum, running_mean, running_var,
+                                                        reinterpret_cast<long long*>(num_batches_tracked), out);
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+}  // extern "C++"
+
 int bg_bn_batch_stats(const void* u, int dtype, int64_t N, const float* gamma, const float* beta, float eps,
                       float momentum, float* running_mean, float* running_var, int64_t* num_batches_tracked,
                       float* a_out, float* shift_out, float* mean_out, float* invstd_out,
                       void* workspace, size_t workspace_bytes, void* stream_) {
+  return bn_batch_stats_impl<kHidden>("bg_bn_batch_stats", u, dtype, N, gamma, beta, eps, momentum, running_mean, running_var,
+                                      num_batches_tracked, a_out, shift_out, mean_out, invstd_out, workspace, workspace_bytes, stream_);
+}
+
+int bg_bn_batch_stats128(const void* u, int dtype, int64_t N, const float* gamma, const float* beta, float eps,
+                         float momentum, float* running_mean, float* running_var, int64_t* num_batches_tracked,
+                         float* a_out, float* shift_out, float* mean_out, float* invstd_out,
+                         void* workspace, size_t workspace_bytes, void* stream_) {
+  return bn_batch_stats_impl<kW128>("bg_bn_batch_stats128", u, dtype, N, gamma, beta, eps, momentum, running_mean, running_var,
+                                    num_batches_tracked, a_out, shift_out, mean_out, invstd_out, workspace, workspace_bytes, stream_);
+}
+
+extern "C++" {
+template <int kW>
+static int bn_act_forward_impl(const char* fn, const void* u, const void* x_prev, void* y, int dtype, int64_t N, const float* a,
+                               const float* shift, float dropout_p, uint64_t seed, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N <= 0) return fail(BG_ERR_INVALID, "bg_bn_batch_stats: needs at least one row");
-  if (!u || !aligned16(u) || !gamma || !beta || !a_out || !shift_out || !mean_out || !invstd_out)
-    return fail(BG_ERR_INVALID, "bg_bn_batch_stats: bad pointer");
-  if ((running_mean != nullptr) != (running_var != nullptr)) return fail(BG_ERR_INVALID, "bg_bn_batch_stats: running_mean and running_var go together");
-  size_t need = 0;
-  bg_train_workspace_bytes(N, &need);
-  if (!workspace || workspace_bytes < need) return fail(BG_ERR_WORKSPACE, "bg_bn_batch_stats: workspace too small");
-  float* partial = static_cast<float*>(workspace);
-  const int grid = stat_grid(N);
-  const DropArgs nodrop = drop_args(0.f, 0);
-  BG_BY_DTYPE(dtype, (k_col_stats<T, 0><<<grid, kStatWarps * 32, 0, stream>>>(static_cast<const T*>(u), nullptr, nullptr, N,
-                                                                          nullptr, nullptr, nodrop, partial)))
-  BG_LAUNCH_OK();
-  BnVectors out{a_out, shift_out, mean_out, invstd_out};
-  k_bn_fwd_finalize<<<kFinalizeCtas, kHidden, 0, stream>>>(partial, grid, N, gamma, beta, eps, momentum, running_mean, running_var,
-                                               reinterpret_cast<long long*>(num_batches_tracked), out);
+  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail_in(BG_ERR_INVALID, fn, "bad size / dropout_p");
+  if (N == 0) return BG_OK;
+  if (!u || !y || !a || !shift || !aligned16(u) || !aligned16(y) || (x_prev && !aligned16(x_prev)))
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
+  const DropArgs d = drop_args(dropout_p, seed);
+  BG_BY_DTYPE(dtype, (k_bn_act_fwd<T, kW><<<grid, 256, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(x_prev),
+                                                                    static_cast<T*>(y), N, a, shift, d)))
   BG_LAUNCH_OK();
   return BG_OK;
 }
+}  // extern "C++"
 
 int bg_bn_act_forward(const void* u, const void* x_prev, void* y, int dtype, int64_t N, const float* a,
                       const float* shift, float dropout_p, uint64_t seed, void* stream_) {
+  return bn_act_forward_impl<kHidden>("bg_bn_act_forward", u, x_prev, y, dtype, N, a, shift, dropout_p, seed, stream_);
+}
+
+int bg_bn_act_forward128(const void* u, const void* x_prev, void* y, int dtype, int64_t N, const float* a,
+                         const float* shift, float dropout_p, uint64_t seed, void* stream_) {
+  return bn_act_forward_impl<kW128>("bg_bn_act_forward128", u, x_prev, y, dtype, N, a, shift, dropout_p, seed, stream_);
+}
+
+extern "C++" {
+template <int kW>
+static int sage_backward_rows_impl(const char* fn, const void* u, const void* dy, const void* dy2, const float* inv_norm,
+                                   const int32_t* rowptr, int dtype, int64_t N, const float* a, const float* shift,
+                                   const float* mean, const float* invstd, float dropout_p, uint64_t seed, float* dgamma,
+                                   float* dbeta, int accumulate, void* dz, void* dz_scaled, void* g_out,
+                                   void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail(BG_ERR_INVALID, "bg_bn_act_forward: bad size / dropout_p");
-  if (N == 0) return BG_OK;
-  if (!u || !y || !a || !shift || !aligned16(u) || !aligned16(y) || (x_prev && !aligned16(x_prev)))
-    return fail(BG_ERR_INVALID, "bg_bn_act_forward: bad pointer");
-  const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
+  if (N <= 0) return fail_in(BG_ERR_INVALID, fn, "needs at least one row");
+  if (!(dropout_p >= 0.f && dropout_p < 1.f)) return fail_in(BG_ERR_INVALID, fn, "bad dropout_p");
+  if (!u || !dy || !dz || !a || !shift || !aligned16(u) || !aligned16(dy) || !aligned16(dz) || (dy2 && !aligned16(dy2)) ||
+      (dz_scaled && (!aligned16(dz_scaled) || !rowptr)) || (g_out && !aligned16(g_out)))
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  const bool bn = mean != nullptr;
+  if (bn && (!invstd || !dgamma || !dbeta)) return fail_in(BG_ERR_INVALID, fn, "BatchNorm needs mean, invstd, dgamma, dbeta");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  size_t need = 0;
+  bg_train_workspace_bytes(N, &need);
+  if (!workspace || workspace_bytes < need) return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
+  float* partial = static_cast<float*>(workspace);
+  const int grid = stat_grid(N);
+  float* k0 = partial + (size_t)grid * 2 * kW;
+  float* k1 = k0 + kW;
   const DropArgs d = drop_args(dropout_p, seed);
-  BG_BY_DTYPE(dtype, (k_bn_act_fwd<T><<<grid, 256, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(x_prev),
-                                                                static_cast<T*>(y), N, a, shift, d)))
+  if (bn) {
+    BG_BY_DTYPE(dtype, (k_col_stats<T, 1, kW><<<grid, kStatWarps * 32, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(dy),
+                                                                                static_cast<const T*>(dy2), N, a, shift, d, partial)))
+    BG_LAUNCH_OK();
+    BnVectors v{const_cast<float*>(a), const_cast<float*>(shift), const_cast<float*>(mean), const_cast<float*>(invstd)};
+    k_bn_bwd_finalize<kW><<<kW / 64, kHidden, 0, stream>>>(partial, grid, N, v, dgamma, dbeta, accumulate, k0, k1);
+    BG_LAUNCH_OK();
+  } else {
+    BG_CUDA_OK(cudaMemsetAsync(k0, 0, 2 * kW * sizeof(float), stream));
+  }
+  const unsigned rgrid = grid_for(N * 32, 256, sm_count() * 8);
+  BG_BY_DTYPE(dtype, (k_sage_bwd_rows<T, kW><<<rgrid, 256, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(dy),
+                                                                        static_cast<const T*>(dy2), N, inv_norm, rowptr, a, shift, k0, k1, d,
+                                                                        static_cast<T*>(dz), static_cast<T*>(dz_scaled), static_cast<T*>(g_out))))
   BG_LAUNCH_OK();
   return BG_OK;
 }
+}  // extern "C++"
 
 int bg_sage_backward_rows(const void* u, const void* dy, const void* dy2, const float* inv_norm, const int32_t* rowptr,
                           int dtype, int64_t N, const float* a, const float* shift, const float* mean,
                           const float* invstd, float dropout_p, uint64_t seed, float* dgamma, float* dbeta,
                           int accumulate, void* dz, void* dz_scaled, void* g_out,
                           void* workspace, size_t workspace_bytes, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N <= 0) return fail(BG_ERR_INVALID, "bg_sage_backward_rows: needs at least one row");
-  if (!(dropout_p >= 0.f && dropout_p < 1.f)) return fail(BG_ERR_INVALID, "bg_sage_backward_rows: bad dropout_p");
-  if (!u || !dy || !dz || !a || !shift || !aligned16(u) || !aligned16(dy) || !aligned16(dz) || (dy2 && !aligned16(dy2)) ||
-      (dz_scaled && (!aligned16(dz_scaled) || !rowptr)) || (g_out && !aligned16(g_out)))
-    return fail(BG_ERR_INVALID, "bg_sage_backward_rows: bad pointer");
-  const bool bn = mean != nullptr;
-  if (bn && (!invstd || !dgamma || !dbeta)) return fail(BG_ERR_INVALID, "bg_sage_backward_rows: BatchNorm needs mean, invstd, dgamma, dbeta");
-  size_t need = 0;
-  bg_train_workspace_bytes(N, &need);
-  if (!workspace || workspace_bytes < need) return fail(BG_ERR_WORKSPACE, "bg_sage_backward_rows: workspace too small");
-  float* partial = static_cast<float*>(workspace);
-  const int grid = stat_grid(N);
-  float* k0 = partial + (size_t)grid * 2 * kHidden;
-  float* k1 = k0 + kHidden;
-  const DropArgs d = drop_args(dropout_p, seed);
-  if (bn) {
-    BG_BY_DTYPE(dtype, (k_col_stats<T, 1><<<grid, kStatWarps * 32, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(dy),
-                                                                            static_cast<const T*>(dy2), N, a, shift, d, partial)))
-    BG_LAUNCH_OK();
-    BnVectors v{const_cast<float*>(a), const_cast<float*>(shift), const_cast<float*>(mean), const_cast<float*>(invstd)};
-    k_bn_bwd_finalize<<<kFinalizeCtas, kHidden, 0, stream>>>(partial, grid, N, v, dgamma, dbeta, accumulate, k0, k1);
-    BG_LAUNCH_OK();
-  } else {
-    BG_CUDA_OK(cudaMemsetAsync(k0, 0, 2 * kHidden * sizeof(float), stream));
-  }
-  const unsigned rgrid = grid_for(N * 32, 256, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_sage_bwd_rows<T><<<rgrid, 256, 0, stream>>>(static_cast<const T*>(u), static_cast<const T*>(dy),
-                                                                    static_cast<const T*>(dy2), N, inv_norm, rowptr, a, shift, k0, k1, d,
-                                                                    static_cast<T*>(dz), static_cast<T*>(dz_scaled), static_cast<T*>(g_out))))
-  BG_LAUNCH_OK();
-  return BG_OK;
+  return sage_backward_rows_impl<kHidden>("bg_sage_backward_rows", u, dy, dy2, inv_norm, rowptr, dtype, N, a, shift, mean, invstd,
+                                          dropout_p, seed, dgamma, dbeta, accumulate, dz, dz_scaled, g_out, workspace,
+                                          workspace_bytes, stream_);
+}
+
+int bg_sage_backward_rows128(const void* u, const void* dy, const void* dy2, const float* inv_norm, const int32_t* rowptr,
+                             int dtype, int64_t N, const float* a, const float* shift, const float* mean,
+                             const float* invstd, float dropout_p, uint64_t seed, float* dgamma, float* dbeta,
+                             int accumulate, void* dz, void* dz_scaled, void* g_out,
+                             void* workspace, size_t workspace_bytes, void* stream_) {
+  return sage_backward_rows_impl<kW128>("bg_sage_backward_rows128", u, dy, dy2, inv_norm, rowptr, dtype, N, a, shift, mean,
+                                        invstd, dropout_p, seed, dgamma, dbeta, accumulate, dz, dz_scaled, g_out, workspace,
+                                        workspace_bytes, stream_);
 }
 
 int bg_transpose_chunks(const void* in, int dtype, int64_t n_rows, int32_t n_cols, int64_t ld, int32_t n_chunks,
@@ -1266,18 +1384,34 @@ int bg_colsum(const void* in, int dtype, int64_t rows, int32_t cols, int64_t ld,
   return BG_OK;
 }
 
-int bg_pool_backward(const float* dpooled, int64_t ldp, const int32_t* graph_ptr, int64_t G, int pool_mode, int64_t N,
-                     void* dx, int dtype, void* stream_) {
+extern "C++" {
+template <int kW>
+static int pool_backward_impl(const char* fn, const float* dpooled, int64_t ldp, const int32_t* graph_ptr, int64_t G, int pool_mode,
+                              int64_t N, void* dx, int dtype, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || G <= 0 || G >= 0x7fffffffLL || ldp < kHidden) return fail(BG_ERR_INVALID, "bg_pool_backward: bad size");
-  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail(BG_ERR_INVALID, "bg_pool_backward: bad pool_mode");
-  if (pool_mode == BG_POOL_SUPERNODE_WITH_POOLING && ldp < 2 * kHidden) return fail(BG_ERR_INVALID, "bg_pool_backward: the concatenated pooling needs dpooled [G, 1024]");
+  if (N < 0 || G <= 0 || G >= 0x7fffffffLL || ldp < kW) return fail_in(BG_ERR_INVALID, fn, "bad size");
+  if (pool_mode < BG_POOL_MEAN || pool_mode > BG_POOL_SUPERNODE_WITH_POOLING) return fail_in(BG_ERR_INVALID, fn, "bad pool_mode");
+  if (pool_mode == BG_POOL_SUPERNODE_WITH_POOLING && ldp < 2 * kW)
+    return fail_in(BG_ERR_INVALID, fn, kW == kHidden ? "the concatenated pooling needs dpooled [G, 1024]"
+                                                     : "the concatenated pooling needs dpooled [G, 256]");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
   if (N == 0) return BG_OK;
-  if (!dpooled || !graph_ptr || !dx || !aligned16(dx)) return fail(BG_ERR_INVALID, "bg_pool_backward: bad pointer");
+  if (!dpooled || !graph_ptr || !dx || !aligned16(dx)) return fail_in(BG_ERR_INVALID, fn, "bad pointer");
   const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_pool_bwd<T><<<grid, 256, 0, stream>>>(dpooled, ldp, graph_ptr, (int)G, pool_mode, N, static_cast<T*>(dx))))
+  BG_BY_DTYPE(dtype, (k_pool_bwd<T, kW><<<grid, 256, 0, stream>>>(dpooled, ldp, graph_ptr, (int)G, pool_mode, N, static_cast<T*>(dx))))
   BG_LAUNCH_OK();
   return BG_OK;
+}
+}  // extern "C++"
+
+int bg_pool_backward(const float* dpooled, int64_t ldp, const int32_t* graph_ptr, int64_t G, int pool_mode, int64_t N,
+                     void* dx, int dtype, void* stream_) {
+  return pool_backward_impl<kHidden>("bg_pool_backward", dpooled, ldp, graph_ptr, G, pool_mode, N, dx, dtype, stream_);
+}
+
+int bg_pool_backward128(const float* dpooled, int64_t ldp, const int32_t* graph_ptr, int64_t G, int pool_mode, int64_t N,
+                        void* dx, int dtype, void* stream_) {
+  return pool_backward_impl<kW128>("bg_pool_backward128", dpooled, ldp, graph_ptr, G, pool_mode, N, dx, dtype, stream_);
 }
 
 static inline int sgemm_splits(int64_t M, int64_t N, int64_t K) {

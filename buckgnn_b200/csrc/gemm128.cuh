@@ -19,6 +19,10 @@
 //              of output at a time, applies bias / normalize / BN / ReLU / skip in fp32 (one rounding of the result)
 //              and moves the rows through a 4 KB swizzled staging tile per warp, so that global loads and stores are
 //              coalesced (8 lanes per 128-byte row piece).
+// kMn (bg_wgrad128, the weight gradients of a 128-wide SAGE layer): both operands MN-major, read in place from row-major
+// [n_rows, 128] matrices (no transposed copies), the reduction over nodes.  Tile t = node chunk t: the CTA of rank 0
+// loads agg^T, rank 1 loads x^T as its 128 rows of the M = 256 A operand, both CTAs their 64-column half of dz as B, so
+// one tile yields [dWl^T ; dWr^T] of the chunk (fp32, plain epilogue) and k_reduce_wgrad128 sums the chunks.
 // The kernel streams: at K = 256 (fp16) a CTA pair reads 256 KB of operands per 256 x 128 x 256 MACs, so HBM, not
 // the tensor core, bounds it.  No setmaxnreg: every warp keeps the launch allocation (168 registers).
 #pragma once
@@ -55,6 +59,7 @@ struct alignas(64) Gemm128Params {
   float bias[kW128];                // epilogue vectors by value -> constant bank
   float scale[kW128];               // 1 when there is no BN
   float shift[kW128];               // 0 when there is no BN
+  int64_t chunk_k;                  // kMn: nodes per chunk (a multiple of k_elems_per_block)
 };
 
 // One epilogue warp: 32 TMEM lanes = 32 output rows of the tiles of parity g.  kPool as in k_gemm512 (last layer of a
@@ -208,9 +213,10 @@ BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base
   }
 }
 
-template <typename TOut, bool kRes, bool kPool>
+template <typename TOut, bool kRes, bool kPool, bool kMn = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 k_gemm128(const __grid_constant__ Gemm128Params p) {
+  static_assert(!kMn || (sizeof(TOut) == 4 && !kRes && !kPool), "weight-gradient mode: fp32 partials, plain epilogue");
   constexpr int kStages = kG128Stages;
   extern __shared__ uint8_t gemm128_smem_raw[];
   const uint32_t smem_base = (smem_u32(gemm128_smem_raw) + 1023u) & ~1023u;   // SWIZZLE_128B wants 1024 B
@@ -254,6 +260,25 @@ k_gemm128(const __grid_constant__ Gemm128Params p) {
     if (elect_one()) {
       uint32_t stage = 0, phase = 0;
       for (int tile = tile0; tile < p.n_tiles; tile += tile_stride) {
+        if constexpr (kMn) {                                    // node chunk `tile`: 128-byte column boxes x kblk nodes
+          const int32_t cols_per_box = p.k_elems_per_block;     // 64 (16-bit) / 32 (tf32) values = 128 B
+          const uint32_t box_bytes = (uint32_t)p.k_elems_per_block * 128u;
+          const void* map_a = &p.seg[rank].a;                   // rank 0: agg, rank 1: x
+          for (int kb = 0; kb < p.kblocks[0]; ++kb) {
+            mbar_wait(empty_bar(stage), phase ^ 1u, kTagEmpty);
+            const uint32_t sa = stages_u32 + stage * kG128StageBytes;
+            const int32_t node0 = (int32_t)((int64_t)tile * p.chunk_k + (int64_t)kb * p.k_elems_per_block);
+            if (rank == 0) mbar_arrive_expect_tx(full_bar(stage), 2 * kG128StageBytes);
+            else mbar_arrive_cluster(full_bar(stage), 0);
+            for (int j = 0; j < kW128 / cols_per_box; ++j)
+              tma_load_2d_cg2(sa + j * box_bytes, map_a, full_bar(stage), j * cols_per_box, node0);
+            for (int j = 0; j < kG128BRows / cols_per_box; ++j)
+              tma_load_2d_cg2(sa + kATileBytes + j * box_bytes, &p.seg[0].b, full_bar(stage),
+                              (int32_t)rank * kG128BRows + j * cols_per_box, node0);
+            if (++stage == kStages) { stage = 0; phase ^= 1u; }
+          }
+          continue;
+        }
         const int32_t row0 = tile * (2 * kTileM) + (int32_t)rank * kTileM;
         for (int s = 0; s < p.n_seg; ++s) {
           for (int kb = 0; kb < p.kblocks[s]; ++kb) {
@@ -272,8 +297,10 @@ k_gemm128(const __grid_constant__ Gemm128Params p) {
     __syncwarp();
   } else if (warp == 1 && rank == 0) {
     // ================================================================ MMA issuer (leader CTA)
-    const uint32_t idesc = umma_idesc(p.a_fmt, p.b_fmt, 2 * kTileM, kW128);
+    const uint32_t idesc = umma_idesc(p.a_fmt, p.b_fmt, 2 * kTileM, kW128) | (kMn ? (3u << 15) : 0u);   // a/b MN-major
     const bool tf32 = p.a_fmt == 2;
+    [[maybe_unused]] const uint32_t mn_lbo = (uint32_t)p.k_elems_per_block * 128u;  // bytes between 128-byte MN blocks
+    [[maybe_unused]] const uint32_t mn_kstep = tf32 ? 1024u : 2048u;                // one UMMA K step: 8 / 16 nodes
     uint32_t stage = 0, phase = 0, it = 0;
     for (int tile = tile0; tile < p.n_tiles; tile += tile_stride, ++it) {
       const uint32_t b = it & 1u;
@@ -292,8 +319,15 @@ k_gemm128(const __grid_constant__ Gemm128Params p) {
 #pragma unroll
             for (int k = 0; k < kStageKBytes / 32; ++k) {
               const uint32_t acc = (first && k == 0) ? 0u : 1u;
-              if (tf32) umma<2, true>(d, umma_smem_desc(sa + k * 32), umma_smem_desc(sb + k * 32), idesc, acc);
-              else umma<2, false>(d, umma_smem_desc(sa + k * 32), umma_smem_desc(sb + k * 32), idesc, acc);
+              if constexpr (kMn) {
+                const uint64_t da = umma_smem_desc_mn(sa + k * mn_kstep, mn_lbo, tf32);
+                const uint64_t db = umma_smem_desc_mn(sb + k * mn_kstep, mn_lbo, tf32);
+                if (tf32) umma<2, true>(d, da, db, idesc, acc);
+                else umma<2, false>(d, da, db, idesc, acc);
+              } else {
+                if (tf32) umma<2, true>(d, umma_smem_desc(sa + k * 32), umma_smem_desc(sb + k * 32), idesc, acc);
+                else umma<2, false>(d, umma_smem_desc(sa + k * 32), umma_smem_desc(sb + k * 32), idesc, acc);
+              }
             }
             umma_commit<2>(empty_bar(stage));                   // smem slot reusable once these MMAs retire
             if (s == p.n_seg - 1 && kb == nkb - 1) umma_commit<2>(tmem_full_bar(b));
@@ -338,9 +372,9 @@ static inline int make_operand_map_rows(CUtensorMap* map, const void* base, int6
   return r == CUDA_SUCCESS ? BG_OK : BG_ERR_CUDA;
 }
 
-template <typename TOut, bool kRes, bool kPool>
+template <typename TOut, bool kRes, bool kPool, bool kMn = false>
 static int launch_gemm128(const Gemm128Params& p, cudaStream_t stream) {
-  auto kern = k_gemm128<TOut, kRes, kPool>;
+  auto kern = k_gemm128<TOut, kRes, kPool, kMn>;
   static bool attr_set = false;
   if (!attr_set) {
     BG_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kG128SmemBytes));

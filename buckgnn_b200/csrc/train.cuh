@@ -12,6 +12,9 @@
 //   dagg = dz Wl, dx = dz Wr + A^T dagg (+ g for skip layers), dWl = dz^T agg, dWr = dz^T x  (bg_gemm512 on
 //   transposed / chunked operands, k_transpose_chunks + k_reduce_partials for the split-K over nodes).
 //
+// The row kernels are templates on the row width kW: 512, or 128 for a hidden_channels = 128 model (the `bg_*128` entry
+// points; its weight gradients run on bg_wgrad128, gemm128.cuh).
+//
 // All reductions are two-stage with a fixed order (no floating-point atomics): a training step is
 // bit-reproducible for a given seed.
 #pragma once
@@ -46,9 +49,38 @@ template <typename T> BG_DEVINL void row_load(const T* row, int lane, float (&v)
   for (int i = 0; i < 16; ++i) v[i] = 0.f;
   f.template accumulate<BG_AGGR_SUM>(v);
 }
-template <typename T> BG_DEVINL void lane_vec(const float* __restrict__ vec, int lane, float (&v)[16]) {
+// One row of kW columns per warp: 512 -> RowFrag (16 columns a lane, interleaved), 128 -> 4 consecutive columns a
+// lane (one 16-byte / 8-byte access).  The kernels below are templates on kW; their 512 instances are the kernels the
+// 512-wide step has always run.
+template <typename T, int kW> struct RowIO;
+template <typename T> struct RowIO<T, kHidden> {
+  static constexpr int kPer = 16;
+  static BG_DEVINL int col_of(int lane, int i) { return RowFrag<T>::col_of(lane, i); }
+  static BG_DEVINL void load(const T* row, int lane, float (&v)[16]) { row_load<T>(row, lane, v); }
+  static BG_DEVINL void store(T* row, int lane, const float (&v)[16]) { RowFrag<T>::store(row, lane, v); }
+};
+template <typename T> struct RowIO<T, 128> {
+  static constexpr int kPer = 4;
+  static BG_DEVINL int col_of(int lane, int i) { return 4 * lane + i; }
+  static BG_DEVINL void load(const T* row, int lane, float (&v)[4]) {
+    if constexpr (sizeof(T) == 4) {
+      const float4 q = *reinterpret_cast<const float4*>(row + 4 * lane);
+      v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+    } else {
+      const uint2 u = *reinterpret_cast<const uint2*>(row + 4 * lane);
+      v[0] = Pack16<T>::lo(u.x); v[1] = Pack16<T>::hi(u.x); v[2] = Pack16<T>::lo(u.y); v[3] = Pack16<T>::hi(u.y);
+    }
+  }
+  static BG_DEVINL void store(T* row, int lane, const float (&v)[4]) {
+    if constexpr (sizeof(T) == 4) *reinterpret_cast<float4*>(row + 4 * lane) = make_float4(v[0], v[1], v[2], v[3]);
+    else *reinterpret_cast<uint2*>(row + 4 * lane) = make_uint2(Pack16<T>::pack(v[0], v[1]), Pack16<T>::pack(v[2], v[3]));
+  }
+};
+
+template <typename T, int kW = kHidden>
+BG_DEVINL void lane_vec(const float* __restrict__ vec, int lane, float (&v)[RowIO<T, kW>::kPer]) {
 #pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = vec[RowFrag<T>::col_of(lane, i)];
+  for (int i = 0; i < RowIO<T, kW>::kPer; ++i) v[i] = vec[RowIO<T, kW>::col_of(lane, i)];
 }
 BG_DEVINL float warp_sum(float v) {
 #pragma unroll
@@ -58,86 +90,91 @@ BG_DEVINL float warp_sum(float v) {
 
 struct DropArgs { uint64_t seed; uint32_t thr; float inv_keep; };
 
-// g = dropout'(dy + dy2) for this lane's 16 columns of row r
-template <typename T>
+// g = dropout'(dy + dy2) for this lane's columns of row r (the dropout element index stays r * 512 + c at every width)
+template <typename T, int kW = kHidden>
 BG_DEVINL void load_upstream(const T* __restrict__ dy, const T* __restrict__ dy2, int64_t r, int lane, const DropArgs& d,
-                             float (&g)[16]) {
-  row_load<T>(dy + (size_t)r * kHidden, lane, g);
+                             float (&g)[RowIO<T, kW>::kPer]) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
+  IO::load(dy + (size_t)r * kW, lane, g);
   if (dy2) {
-    float t[16];
-    row_load<T>(dy2 + (size_t)r * kHidden, lane, t);
+    float t[kPer];
+    IO::load(dy2 + (size_t)r * kW, lane, t);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) g[i] += t[i];
+    for (int i = 0; i < kPer; ++i) g[i] += t[i];
   }
   if (d.thr) {
 #pragma unroll
-    for (int i = 0; i < 16; ++i)
-      g[i] = dropout_keep(d.seed, r, RowFrag<T>::col_of(lane, i), d.thr) ? g[i] * d.inv_keep : 0.f;
+    for (int i = 0; i < kPer; ++i)
+      g[i] = dropout_keep(d.seed, r, IO::col_of(lane, i), d.thr) ? g[i] * d.inv_keep : 0.f;
   }
 }
 
 // ------------------------------------------------------------------ column statistics
 // kMode 0: S1 = sum_r u, S2 = sum_r u^2                         (train-mode BatchNorm forward)
 // kMode 1: dv = g [a u + shift > 0]; S1 = sum dv, S2 = sum dv u  (BatchNorm backward)
-// partial [gridDim.x][2][512] f32; each CTA owns a contiguous chunk of rows
-template <typename T, int kMode>
+// partial [gridDim.x][2][kW] f32; each CTA owns a contiguous chunk of rows
+template <typename T, int kMode, int kW = kHidden>
 __global__ void __launch_bounds__(kStatWarps * 32)
 k_col_stats(const T* __restrict__ u, const T* __restrict__ dy, const T* __restrict__ dy2, int64_t N,
             const float* __restrict__ a, const float* __restrict__ shift, const DropArgs drop,
             float* __restrict__ partial) {
-  __shared__ float red[kStatWarps][2][kHidden];
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
+  __shared__ float red[kStatWarps][2][kW];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t chunk = (N + gridDim.x - 1) / gridDim.x;
   const int64_t r_beg = (int64_t)blockIdx.x * chunk, r_end = min(N, r_beg + chunk);
-  float s1[16], s2[16];
-  [[maybe_unused]] float av[16], sv[16];
+  float s1[kPer], s2[kPer];
+  [[maybe_unused]] float av[kPer], sv[kPer];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) s1[i] = s2[i] = 0.f;
-  if constexpr (kMode == 1) { lane_vec<T>(a, lane, av); lane_vec<T>(shift, lane, sv); }
+  for (int i = 0; i < kPer; ++i) s1[i] = s2[i] = 0.f;
+  if constexpr (kMode == 1) { lane_vec<T, kW>(a, lane, av); lane_vec<T, kW>(shift, lane, sv); }
   for (int64_t r = r_beg + warp; r < r_end; r += kStatWarps) {
-    float uv[16];
-    row_load<T>(u + (size_t)r * kHidden, lane, uv);
+    float uv[kPer];
+    IO::load(u + (size_t)r * kW, lane, uv);
     if constexpr (kMode == 0) {
 #pragma unroll
-      for (int i = 0; i < 16; ++i) { s1[i] += uv[i]; s2[i] = fmaf(uv[i], uv[i], s2[i]); }
+      for (int i = 0; i < kPer; ++i) { s1[i] += uv[i]; s2[i] = fmaf(uv[i], uv[i], s2[i]); }
     } else {
-      float g[16];
-      load_upstream<T>(dy, dy2, r, lane, drop, g);
+      float g[kPer];
+      load_upstream<T, kW>(dy, dy2, r, lane, drop, g);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) {
+      for (int i = 0; i < kPer; ++i) {
         const float dv = fmaf(av[i], uv[i], sv[i]) > 0.f ? g[i] : 0.f;
         s1[i] += dv; s2[i] = fmaf(dv, uv[i], s2[i]);
       }
     }
   }
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int c = RowFrag<T>::col_of(lane, i);
+  for (int i = 0; i < kPer; ++i) {
+    const int c = IO::col_of(lane, i);
     red[warp][0][c] = s1[i]; red[warp][1][c] = s2[i];
   }
   __syncthreads();
-  for (int c = threadIdx.x; c < 2 * kHidden; c += blockDim.x) {
-    const int k = c / kHidden, cc = c % kHidden;
+  for (int c = threadIdx.x; c < 2 * kW; c += blockDim.x) {
+    const int k = c / kW, cc = c % kW;
     float v = red[0][k][cc];
 #pragma unroll
     for (int w = 1; w < kStatWarps; ++w) v += red[w][k][cc];
-    partial[(size_t)blockIdx.x * 2 * kHidden + c] = v;
+    partial[(size_t)blockIdx.x * 2 * kW + c] = v;
   }
 }
 
-struct BnVectors {          // [512] f32 each, device
+struct BnVectors {          // [kW] f32 each, device
   float* a;                 // gamma * invstd          (1 without BatchNorm)
   float* shift;             // beta - mean * a         (0 without BatchNorm)
   float* mean;
   float* invstd;
 };
 
-// Finalize kernels: kFinalizeCtas CTAs x 512 threads.  CTA b owns columns [64 b, 64 b + 64); thread (g, cl) sums the
+// Finalize kernels: kFinalizeCtas (kW / 64) CTAs x 512 threads.  CTA b owns columns [64 b, 64 b + 64); thread (g, cl) sums the
 // partial slots p = g, g + 8, ... of column 64 b + cl in fp64 (four interleaved chains), the eight groups are added in
 // a fixed order through shared memory, and the threads of group 0 finish their column.  (Round 1 ran ONE CTA of 512
 // threads, each walking all ~300 slots of its column: 34 us per launch, 12 launches per training step -- the
 // dependent L2 round trips, not the arithmetic, were the cost.)
 constexpr int kFinalizeCtas = kHidden / 64;
+template <int kW = kHidden>
 BG_DEVINL bool sum_partials(const float* __restrict__ partial, int n_parts, int& c, double& s1, double& s2) {
   __shared__ double sh1[8][64], sh2[8][64];
   const int cl = threadIdx.x & 63, g = threadIdx.x >> 6;
@@ -149,15 +186,15 @@ BG_DEVINL bool sum_partials(const float* __restrict__ partial, int n_parts, int&
   for (; p + 24 < n_parts; p += 32) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      a1[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kHidden + c];
-      a2[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kHidden + kHidden + c];
+      a1[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kW + c];
+      a2[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kW + kW + c];
     }
   }
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     if (p + 8 * k < n_parts) {
-      a1[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kHidden + c];
-      a2[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kHidden + kHidden + c];
+      a1[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kW + c];
+      a2[k] += (double)partial[(size_t)(p + 8 * k) * 2 * kW + kW + c];
     }
   }
   sh1[g][cl] = (a1[0] + a1[1]) + (a1[2] + a1[3]);
@@ -171,13 +208,14 @@ BG_DEVINL bool sum_partials(const float* __restrict__ partial, int n_parts, int&
 
 // Batch mean / biased variance -> a, shift, mean, invstd; running statistics updated as torch.nn.BatchNorm1d does in
 // train mode (momentum, unbiased variance) -- Models/BuckGNN.py:163,451.
+template <int kW = kHidden>
 __global__ void __launch_bounds__(kHidden)
 k_bn_fwd_finalize(const float* __restrict__ partial, int n_parts, int64_t N, const float* __restrict__ gamma,
                   const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean,
                   float* __restrict__ running_var, long long* __restrict__ num_batches_tracked, BnVectors out) {
   int c;
   double s1, s2;
-  if (!sum_partials(partial, n_parts, c, s1, s2)) return;
+  if (!sum_partials<kW>(partial, n_parts, c, s1, s2)) return;
   const double mean = s1 / (double)N;
   double var = s2 / (double)N - mean * mean;
   if (var < 0.0) var = 0.0;
@@ -197,13 +235,14 @@ k_bn_fwd_finalize(const float* __restrict__ partial, int n_parts, int64_t N, con
 
 // dbeta = S1, dgamma = invstd (S2 - mean S1);  du = a dv - k0 - k1 u  with
 // k1 = a invstd dgamma / N,  k0 = a S1 / N - k1 mean
+template <int kW = kHidden>
 __global__ void __launch_bounds__(kHidden)
 k_bn_bwd_finalize(const float* __restrict__ partial, int n_parts, int64_t N, const BnVectors bn,
                   float* __restrict__ dgamma, float* __restrict__ dbeta, int accumulate,
                   float* __restrict__ k0, float* __restrict__ k1) {
   int c;
   double s1, s2;
-  if (!sum_partials(partial, n_parts, c, s1, s2)) return;
+  if (!sum_partials<kW>(partial, n_parts, c, s1, s2)) return;
   const double mean = bn.mean[c], invstd = bn.invstd[c], av = bn.a[c];
   const double dg = invstd * (s2 - mean * s1);
   if (accumulate) { dgamma[c] += (float)dg; dbeta[c] += (float)s1; }
@@ -214,57 +253,61 @@ k_bn_bwd_finalize(const float* __restrict__ partial, int n_parts, int64_t N, con
 }
 
 // ------------------------------------------------------------------ y = drop(relu(a u + shift) + x_prev)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_bn_act_fwd(const T* __restrict__ u, const T* __restrict__ x_prev, T* __restrict__ y, int64_t N,
              const float* __restrict__ a, const float* __restrict__ shift, const DropArgs drop) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  float av[16], sv[16];
-  lane_vec<T>(a, lane, av); lane_vec<T>(shift, lane, sv);
+  float av[kPer], sv[kPer];
+  lane_vec<T, kW>(a, lane, av); lane_vec<T, kW>(shift, lane, sv);
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += n_warps) {
-    float v[16];
-    row_load<T>(u + (size_t)r * kHidden, lane, v);
+    float v[kPer];
+    IO::load(u + (size_t)r * kW, lane, v);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = fmaxf(fmaf(av[i], v[i], sv[i]), 0.f);
+    for (int i = 0; i < kPer; ++i) v[i] = fmaxf(fmaf(av[i], v[i], sv[i]), 0.f);
     if (x_prev) {
-      float t[16];
-      row_load<T>(x_prev + (size_t)r * kHidden, lane, t);
+      float t[kPer];
+      IO::load(x_prev + (size_t)r * kW, lane, t);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] += t[i];
+      for (int i = 0; i < kPer; ++i) v[i] += t[i];
     }
     if (drop.thr) {
 #pragma unroll
-      for (int i = 0; i < 16; ++i)
-        v[i] = dropout_keep(drop.seed, r, RowFrag<T>::col_of(lane, i), drop.thr) ? v[i] * drop.inv_keep : 0.f;
+      for (int i = 0; i < kPer; ++i)
+        v[i] = dropout_keep(drop.seed, r, IO::col_of(lane, i), drop.thr) ? v[i] * drop.inv_keep : 0.f;
     }
-    RowFrag<T>::store(y + (size_t)r * kHidden, lane, v);
+    IO::store(y + (size_t)r * kW, lane, v);
   }
 }
 
 // ------------------------------------------------------------------ dz rows
 // dv = g [a u + shift > 0];  du = a dv - k0 - k1 u;  dz = inv_norm (du - u (u . du));
 // dz_scaled = dz / max(deg, 1) (mean aggregation: the row of A^T dagg's operand);  g_out = g (skip layers)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_sage_bwd_rows(const T* __restrict__ u, const T* __restrict__ dy, const T* __restrict__ dy2, int64_t N,
                 const float* __restrict__ inv_norm, const int32_t* __restrict__ rowptr,
                 const float* __restrict__ a, const float* __restrict__ shift, const float* __restrict__ k0,
                 const float* __restrict__ k1, const DropArgs drop, T* __restrict__ dz, T* __restrict__ dz_scaled,
                 T* __restrict__ g_out) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  float av[16], sv[16], k0v[16], k1v[16];
-  lane_vec<T>(a, lane, av); lane_vec<T>(shift, lane, sv);
-  lane_vec<T>(k0, lane, k0v); lane_vec<T>(k1, lane, k1v);
+  float av[kPer], sv[kPer], k0v[kPer], k1v[kPer];
+  lane_vec<T, kW>(a, lane, av); lane_vec<T, kW>(shift, lane, sv);
+  lane_vec<T, kW>(k0, lane, k0v); lane_vec<T, kW>(k1, lane, k1v);
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += n_warps) {
-    float uv[16], g[16];
-    row_load<T>(u + (size_t)r * kHidden, lane, uv);
-    load_upstream<T>(dy, dy2, r, lane, drop, g);
-    if (g_out) RowFrag<T>::store(g_out + (size_t)r * kHidden, lane, g);
+    float uv[kPer], g[kPer];
+    IO::load(u + (size_t)r * kW, lane, uv);
+    load_upstream<T, kW>(dy, dy2, r, lane, drop, g);
+    if (g_out) IO::store(g_out + (size_t)r * kW, lane, g);
     float dot = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < kPer; ++i) {
       const float dv = fmaf(av[i], uv[i], sv[i]) > 0.f ? g[i] : 0.f;
       g[i] = fmaf(av[i], dv, -fmaf(k1v[i], uv[i], k0v[i]));      // du
       dot = fmaf(uv[i], g[i], dot);
@@ -272,13 +315,13 @@ k_sage_bwd_rows(const T* __restrict__ u, const T* __restrict__ dy, const T* __re
     dot = warp_sum(dot);
     const float inr = inv_norm ? inv_norm[r] : 1.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) g[i] = inv_norm ? inr * fmaf(-uv[i], dot, g[i]) : g[i];
-    RowFrag<T>::store(dz + (size_t)r * kHidden, lane, g);
+    for (int i = 0; i < kPer; ++i) g[i] = inv_norm ? inr * fmaf(-uv[i], dot, g[i]) : g[i];
+    IO::store(dz + (size_t)r * kW, lane, g);
     if (dz_scaled) {
       const float id = 1.f / (float)max(rowptr[r + 1] - rowptr[r], 1);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) g[i] *= id;
-      RowFrag<T>::store(dz_scaled + (size_t)r * kHidden, lane, g);
+      for (int i = 0; i < kPer; ++i) g[i] *= id;
+      IO::store(dz_scaled + (size_t)r * kW, lane, g);
     }
   }
 }
@@ -322,6 +365,22 @@ __global__ void k_reduce_partials(const float* __restrict__ partial, int n_chunk
   }
 }
 
+// 128-wide weight gradients (bg_wgrad128): partial [n_chunks][256][128] f32 holds, per node chunk, [dWl^T ; dWr^T]
+// (row = input feature of lin_l / lin_r, column = output feature).  dW{l,r}[o, i] (+)= sum_s partial[s][{0,128} + i][o],
+// summed in chunk order.  Reads are coalesced along o; the 2 x 16 K scattered writes are small next to them.
+__global__ void __launch_bounds__(256)
+k_reduce_wgrad128(const float* __restrict__ partial, int n_chunks, float* __restrict__ dwl, float* __restrict__ dwr,
+                  int accumulate) {
+  const int64_t n = 2 * 128 * 128, stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const int which = (int)(t >> 14), i = (int)(t >> 7) & 127, o = (int)t & 127;
+    float v = 0.f;
+    for (int s = 0; s < n_chunks; ++s) v += partial[((size_t)s * 256 + which * 128 + i) * 128 + o];
+    float* out = (which ? dwr : dwl) + (size_t)o * 128 + i;
+    *out = accumulate ? *out + v : v;
+  }
+}
+
 // ------------------------------------------------------------------ generic loads by run-time dtype
 BG_DEVINL float load_as_float(const void* p, int dtype, size_t i) {
   if (dtype == BG_F32) return static_cast<const float*>(p)[i];
@@ -359,10 +418,12 @@ k_colsum_partial(const void* __restrict__ in, int dtype, int64_t rows, int cols,
 // 0 and cnt excludes it;  supernode_only: only the last node, w = 1;  supernode_with_pooling (dpooled is [G, 1024] =
 // cat[mean_no_super, super]): real nodes take the first half / (cnt - 1), the last node the second half.
 // (Models/BuckGNN.py:273-293 in reverse.)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_pool_bwd(const float* __restrict__ dpooled, int64_t ldp, const int32_t* __restrict__ graph_ptr, int G, int mode,
            int64_t N, T* __restrict__ dx) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += n_warps) {
@@ -375,11 +436,11 @@ k_pool_bwd(const float* __restrict__ dpooled, int64_t ldp, const int32_t* __rest
     if (mode == BG_POOL_MEAN) w = 1.f / (float)max(end - beg, (int64_t)1);
     else if (mode == BG_POOL_MEAN_NO_SUPER) w = last ? 0.f : 1.f / (float)max(end - beg - 1, (int64_t)1);
     else if (mode == BG_POOL_SUPERNODE_ONLY) w = last ? 1.f : 0.f;
-    else { w = last ? 1.f : 1.f / (float)max(end - beg - 1, (int64_t)1); off = last ? kHidden : 0; }   // cat[mean_no_super, super]
-    float v[16];
+    else { w = last ? 1.f : 1.f / (float)max(end - beg - 1, (int64_t)1); off = last ? kW : 0; }   // cat[mean_no_super, super]
+    float v[kPer];
 #pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = w * dpooled[(size_t)lo * ldp + off + RowFrag<T>::col_of(lane, i)];
-    RowFrag<T>::store(dx + (size_t)r * kHidden, lane, v);
+    for (int i = 0; i < kPer; ++i) v[i] = w * dpooled[(size_t)lo * ldp + off + IO::col_of(lane, i)];
+    IO::store(dx + (size_t)r * kW, lane, v);
   }
 }
 

@@ -17,6 +17,11 @@ In train mode (`model.train()`, as TRAIN_FINAL.py:289 does) the forward uses bat
 BatchNorm1d, applies Dropout and is differentiable: `loss.backward()` runs the backward kernels
 (`train.py`) and leaves `.grad` on the parameters that model_name uses.
 
+A hidden_channels = 128 model (the reference's default width) evaluates on its own 128-wide kernels.  It trains on them
+too when `model.native128_train` is set (a module attribute, default from BUCKGNN_NATIVE128_TRAIN=1 in the
+environment); otherwise, and for what the 128-wide step does not cover, training runs as the zero-padded 512-wide
+twin (narrow.py).
+
 Extra, non-reference keywords: `train_precision` in {"tf32", "bf16", "fp16"} (storage of the training
 step's activations and activation gradients; default tf32 = fp32 storage), and `precision` in {"auto", "fp16", "bf16", "tf32", "fp32"}
 selects how the tensor-core GEMMs read their operands (engine.PRECISION_FORMATS; fp32 =
@@ -26,6 +31,8 @@ sum/add whose hub rows can leave the fp16 range).
 from __future__ import annotations
 
 from typing import Dict, Optional
+
+import os
 
 import torch
 import torch.nn as nn
@@ -42,6 +49,9 @@ _SAGE_LISTS = {  # model_name -> (ModuleList attribute, aggr)      reference :12
 _POOLINGS = ("mean", "mean_no_super", "supernode_only", "supernode_with_pooling", "mlp", "mlp_no_super")
 # models whose eval forward at hidden_channels == 128 runs on the 128-wide kernels (the rest use narrow.WideTwin)
 _NATIVE128_MODELS = tuple(_SAGE_LISTS) + ("GraphSage_addAggr_Shared", "GraphSAGE_MLP")
+# train-mode forwards of the same models at hidden_channels == 128 on the 128-wide kernels (train.py at width 128)
+# instead of the twin.  Opt-in: BUCKGNN_NATIVE128_TRAIN=1 in the environment, or `model.native128_train = True`.
+NATIVE128_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_TRAIN", "0") not in ("", "0")
 
 
 class SAGEConv(nn.Module):
@@ -149,6 +159,7 @@ class BuckGNN(nn.Module):
         self.fold_encoder = fold_encoder      # fold node_encoder[4] into SAGE layer 0 (mean / sum / add aggregation)
         self.fuse_pool = fuse_pool            # last SAGE layer's epilogue sums its rows for the pooling layer (16-bit modes)
         self.fuse_aggregate = engine.FUSE_AGGREGATE_DEFAULT    # the aggregate operand gathered inside the update GEMM (opt-in)
+        self.native128_train = NATIVE128_TRAIN_DEFAULT         # hidden_channels 128: train on the 128-wide kernels (opt-in)
         self.output_dim = output_dim = _output_dim(prediction_type, use_z_coord, use_rotations)
         h = hidden_channels
         cat_dec = pooling_layer == "supernode_with_pooling" and prediction_type == "buckling"
@@ -351,6 +362,14 @@ class BuckGNN(nn.Module):
                 and self.model_name in _NATIVE128_MODELS and self.prediction_type == "buckling"
                 and self.pooling_layer in _POOLINGS)
 
+    def _trains_native128(self) -> bool:
+        """With `native128_train` on, train-mode forwards of the models `_runs_native128` covers run the training step
+        at width 128 on the module's own parameters (train.py); everything else at a width other than 512 trains as the
+        twin, flag or no flag."""
+        return (self.hidden_channels == 128 and self.training and bool(self.native128_train)
+                and self.model_name in _NATIVE128_MODELS and self.prediction_type == "buckling"
+                and self.pooling_layer in _POOLINGS)
+
     def forward(self, x, edge_index, edge_attr, batch=None, mask=None):
         self._check_supported(x)
         self._ran_native128 = False
@@ -359,7 +378,17 @@ class BuckGNN(nn.Module):
                 pred = self._forward_cuda(x, edge_index, batch, width=128)
             self._ran_native128 = True
             return pred.squeeze(), batch
+        if self._trains_native128():
+            from . import train
+            pred = train.forward_train(self, x, edge_index, batch, edge_attr=edge_attr)
+            self._pack_sig = None                # BatchNorm statistics changed: the next native eval forward repacks
+            return pred.squeeze(), batch
         if self.hidden_channels != 512:
+            if self.training and getattr(self, "_grad_sync", None) is not None:
+                # the twin's parameters are not the module's own: the installed GradSync would never see a gradient
+                raise NotImplementedError("buckgnn_b200: this model trains as the zero-padded 512-wide twin, which "
+                                          "enable_gradient_sync does not cover; use dist.allreduce_gradients("
+                                          "model.parameters()) after backward() instead")
             # TRAIN_FINAL.py:55,71 / the constructor default use 128: runs as the exact zero-padded 512-wide twin.
             # 129..255 build no encoder in the reference (Models/BuckGNN.py:41,67): the same AttributeError surfaces here.
             if self._wide is None:
@@ -423,9 +452,10 @@ class BuckGNN(nn.Module):
         """Multi-GPU training (BASELINE.json configs[3]): all-reduce (mean) the gradients of this model's trainable
         parameters over `group`, bucketed per layer and overlapped with the backward pass (dist.GradSync).  Call once
         after `.to(device)`, on every rank; `loss.backward()` then leaves the REDUCED gradients in `.grad`."""
-        if self.hidden_channels != 512:
-            raise NotImplementedError("buckgnn_b200: overlapped gradient sync is built for hidden_channels=512; "
-                                      "use dist.allreduce_gradients(model.parameters()) after backward() instead")
+        if self.hidden_channels != 512 and not (self.hidden_channels == 128 and self.native128_train):
+            raise NotImplementedError("buckgnn_b200: overlapped gradient sync is built for hidden_channels=512, and for "
+                                      "128 with native128_train on; use dist.allreduce_gradients(model.parameters()) "
+                                      "after backward() instead")
         from . import train
         from .dist import GradSync
         self._grad_sync = GradSync(train.trainable_parameters(self), next(self.parameters()).device, group)

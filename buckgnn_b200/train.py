@@ -17,6 +17,11 @@ Per layer (Models/BuckGNN.py:447-458, train mode)
               dx = dz Wr + A^T dagg  (+ g on skip layers) bg_sage_aggregate over the CSR keyed by source + bg_gemm512
 The encoder's first two Linears, the decoder and their gradients run on `bg_sgemm` (fp32 CUDA cores).
 
+Width: the step runs at the model's hidden_channels, 512 or 128 (`BuckGNN.native128_train`: a hidden_channels = 128
+model trains on its own 128-wide kernels -- bg_gemm128, bg_wgrad128 and the `*128` row kernels -- instead of the
+zero-padded 512-wide twin of narrow.py).  At 128 the encoder and decoder are the reference's 2-layer MLPs
+(Models/BuckGNN.py:41-65), all on bg_sgemm.
+
 Precision: `train_precision` in {"tf32" (default; fp32 storage), "bf16", "fp16"}: activations, saved tensors and
 gradients of activations are stored in that format, weight gradients and all reductions are fp32.
 """
@@ -60,10 +65,11 @@ def colsum(src, code, rows, cols, ld, out, accumulate=False):
     capi.colsum(src.data_ptr(), code, rows, cols, ld, out.data_ptr(), accumulate, ws.data_ptr(), nbytes, _stream())
 
 
-def split_k_layout(n_rows: int):
-    """(chunks, chunk_k) of the split over nodes for the weight-gradient GEMMs: one 512 x 512 product per CTA
-    pair of the 148-SM part when there is enough work, K per chunk a multiple of 64."""
-    chunks = max(1, min(37, -(-n_rows // 1024)))
+def split_k_layout(n_rows: int, max_chunks: int = 37):
+    """(chunks, chunk_k) of the split over nodes for the weight-gradient GEMMs: one 512 x 512 product (width 128:
+    max_chunks = 74, one 256 x 128 tile) per CTA pair of the 148-SM part when there is enough work, K per chunk a
+    multiple of 64."""
+    chunks = max(1, min(max_chunks, -(-n_rows // 1024)))
     chunk_k = -(-(-(-n_rows // chunks)) // 64) * 64
     return chunks, chunk_k
 
@@ -106,6 +112,24 @@ def weight_grad_mn(dz: torch.Tensor, act: torch.Tensor, code: int, n_rows: int, 
         capi.wgrad512(dz.data_ptr(), dz.shape[1], act.data_ptr(), act.shape[1], act.shape[1], code, n_rows, chunks,
                       chunk_k, partial.data_ptr(), _stream())
     capi.reduce_partials(partial.data_ptr(), chunks, 512 * 512, out.data_ptr(), accumulate, _stream())
+
+
+def sage_weight_grads(dz: torch.Tensor, agg: torch.Tensor, x: torch.Tensor, code: int, n_rows: int, dwl: torch.Tensor,
+                      acc_l: bool, dwr: torch.Tensor, acc_r: bool) -> None:
+    """dWl (+)= dz^T agg and dWr (+)= dz^T x of one SAGE layer at the rows' width: two bg_wgrad512 products at 512,
+    one bg_wgrad128 launch for both at 128."""
+    width = dz.shape[1]
+    if width == 512:
+        weight_grad_mn(dz, agg, code, n_rows, dwl, acc_l)
+        weight_grad_mn(dz, x, code, n_rows, dwr, acc_r)
+        return
+    if acc_l != acc_r:
+        raise RuntimeError("buckgnn_b200: lin_l and lin_r of a layer accumulate together")
+    chunks, chunk_k = split_k_layout(n_rows, max_chunks=74)
+    partial = _f32((chunks * 256, 128), dz.device)
+    with engine.TIMERS.span("train_wgrad_gemm"):
+        capi.wgrad128(dz.data_ptr(), agg.data_ptr(), x.data_ptr(), code, n_rows, chunks, chunk_k, partial.data_ptr(),
+                      dwl.data_ptr(), dwr.data_ptr(), acc_l, _stream())
 
 
 def transposed_pack(weight: torch.Tensor, precision: str) -> engine.LinearPack:
@@ -180,14 +204,24 @@ class GradStore:
 
 
 # ----------------------------------------------------------------------------- shared pieces: encoders and head
-def encoder_forward_train(enc, inp: torch.Tensor, prec: str, bias3_host: torch.Tensor):
+def encoder_forward_train(enc, inp: torch.Tensor, prec: str, bias3_host: torch.Tensor, width: int = 512):
     """node_encoder / edge_encoder (Models/BuckGNN.py:68-82): the two narrow Linears on bg_sgemm (fp32), the
-    128 -> 512 one on the tensor cores.  Returns (h1 [n,64] f32, h2 [n,128], out [n,512])."""
+    128 -> 512 one on the tensor cores.  Returns (h1 [n,64] f32, h2 [n,128], out [n,512]).
+    width 128: the 2-layer encoder Linear(F,64) ReLU Linear(64,128) (:41-48), both on bg_sgemm; returns
+    (h1 [n,64] f32, None, out [n,128])."""
     dev, n, f = inp.device, inp.shape[0], inp.shape[1]
     code = engine.PRECISION_FORMATS[prec][0]
     F32 = capi.BG_F32
     w1, b1 = enc[0].weight.detach().float().contiguous(), enc[0].bias.detach().float().contiguous()
     w2, b2 = enc[2].weight.detach().float().contiguous(), enc[2].bias.detach().float().contiguous()
+    if width == 128:
+        with engine.TIMERS.span("train_encoder"):
+            h1 = _f32((n, 64), dev)
+            sgemm(inp, F32, f, 1, w1, F32, 1, f, n, 64, f, h1, F32, 64, bias=b1, relu=True)
+            out = Activation(n, 128, prec, dev)
+            sgemm(h1, F32, 64, 1, w2, F32, 1, 64, n, 128, 64, out.data, code, 128, bias=b2)
+            out.refresh_split()
+        return h1, None, out
     with engine.TIMERS.span("train_encoder"):
         h1 = _f32((n, 64), dev)
         sgemm(inp, F32, f, 1, w1, F32, 1, f, n, 64, f, h1, F32, 64, bias=b1, relu=True)
@@ -200,14 +234,26 @@ def encoder_forward_train(enc, inp: torch.Tensor, prec: str, bias3_host: torch.T
     return h1, h2, out
 
 
-def encoder_backward(enc, inp: torch.Tensor, h1: torch.Tensor, h2: Activation, dout: Activation, prec: str,
+def encoder_backward(enc, inp: torch.Tensor, h1: torch.Tensor, h2: Optional[Activation], dout: Activation, prec: str,
                      grads: GradStore) -> None:
-    """Gradients of the three encoder Linears given d(out) [n, 512]."""
+    """Gradients of the three encoder Linears given d(out) [n, 512] (of the two given d(out) [n, 128] at width 128)."""
     dev, n, f = inp.device, inp.shape[0], inp.shape[1]
     code = engine.PRECISION_FORMATS[prec][0]
     F32 = capi.BG_F32
     s = _stream()
     dx0 = dout.data
+    if dx0.shape[1] == 128:
+        with engine.TIMERS.span("train_encoder_bwd"):
+            w2 = enc[2].weight.detach().float().contiguous()          # [128, 64]
+            dw2e, _ = grads.get(enc[2].weight); db2e, _ = grads.get(enc[2].bias)
+            sgemm(dx0, code, 1, 128, h1, F32, 64, 1, 128, 64, n, dw2e, F32, 64)
+            colsum(dx0, code, n, 128, 128, db2e)
+            dh1 = _f32((n, 64), dev)
+            sgemm(dx0, code, 128, 1, w2, F32, 64, 1, n, 64, 128, dh1, F32, 64, mask=h1, mask_ld=64)
+            dw1e, _ = grads.get(enc[0].weight); db1e, _ = grads.get(enc[0].bias)
+            sgemm(dh1, F32, 1, 64, inp, F32, f, 1, 64, f, n, dw1e, F32, f)
+            colsum(dh1, F32, n, 64, 64, db1e)
+        return
     with engine.TIMERS.span("train_encoder_bwd"):
         w3 = enc[4].weight.detach().float().contiguous()          # [512, 128]
         w2 = enc[2].weight.detach().float().contiguous()
@@ -233,10 +279,90 @@ def encoder_backward(enc, inp: torch.Tensor, h1: torch.Tensor, h2: Activation, d
         colsum(dh1, F32, n, 64, 64, db1e)
 
 
+def _decoder128_embedded(dec) -> dict:
+    """The 2-layer decoder Linear(in,64) ReLU Linear(64,out) of a hidden_channels = 128 model in the 3-layer form
+    bg_pool_head128 takes (include/buckgnn_b200.h): w1 = [W1; 0], w2 = [I64 | 0], w3 = W2."""
+    f32 = lambda t: t.detach().float().contiguous()
+    dev = dec[0].weight.device
+    w1 = torch.zeros((128, dec[0].in_features), dtype=torch.float32, device=dev)
+    b1 = torch.zeros(128, dtype=torch.float32, device=dev)
+    w1[:64], b1[:64] = f32(dec[0].weight), f32(dec[0].bias)
+    w2 = torch.zeros((64, 128), dtype=torch.float32, device=dev)
+    w2[:, :64] = torch.eye(64, device=dev)
+    return {"w1": w1, "b1": b1, "w2": w2, "b2": torch.zeros(64, dtype=torch.float32, device=dev),
+            "w3": f32(dec[2].weight), "b3": f32(dec[2].bias)}
+
+
+def _head_forward_train128(model, cur: Activation, idx, sv) -> torch.Tensor:
+    """head_forward_train at width 128: bg_pool_head128's pooled feature, MLPPooling Linear(128,128) and the 2-layer
+    decoder Linear(128 | 256, 64) ReLU Linear(64, out) on bg_sgemm.  sv.h1d is the decoder's hidden layer [G, 64];
+    there is no second one (sv.h2d = None)."""
+    dev = cur.data.device
+    dec = model.decoder
+    F32 = capi.BG_F32
+    with engine.TIMERS.span("pool_head"):
+        _, raw = engine.pool_head(cur, idx, _decoder128_embedded(dec), model.output_dim, want_pooled=True,
+                                  pooling=model.pooling_layer)
+        g_count, in_dim = raw.shape
+        sv.mlp = None
+        dec_in = raw
+        if model.pooling_layer in ("mlp", "mlp_no_super"):                     # MLPPooling (:568-581)
+            lin = model.pooling_mpl.mlp[0]
+            wp, bp = lin.weight.detach().float().contiguous(), lin.bias.detach().float().contiguous()
+            dec_in = _f32((g_count, 128), dev)
+            sgemm(raw, F32, 128, 1, wp, F32, 1, 128, g_count, 128, 128, dec_in, F32, 128, bias=bp, relu=True)
+            sv.mlp = (lin, wp)
+        decw = {"w1": dec[0].weight.detach().float().contiguous(), "b1": dec[0].bias.detach().float().contiguous(),
+                "w2": dec[2].weight.detach().float().contiguous(), "b2": dec[2].bias.detach().float().contiguous()}
+        out_dim = model.output_dim
+        h1d, pred = _f32((g_count, 64), dev), _f32((g_count, out_dim), dev)
+        sgemm(dec_in, F32, in_dim, 1, decw["w1"], F32, 1, in_dim, g_count, 64, in_dim, h1d, F32, 64, bias=decw["b1"], relu=True)
+        sgemm(h1d, F32, 64, 1, decw["w2"], F32, 1, 64, g_count, out_dim, 64, pred, F32, out_dim, bias=decw["b2"])
+    sv.decw, sv.raw, sv.dec_in, sv.h1d, sv.h2d = decw, raw, dec_in, h1d, None
+    return pred
+
+
+def _head_backward128(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
+    """head_backward at width 128: returns d(last layer output) [n, 128]."""
+    dev = dpred.device
+    code = engine.PRECISION_FORMATS[prec][0]
+    F32 = capi.BG_F32
+    g_count, out_dim = sv.raw.shape[0], model.output_dim
+    in_dim = sv.dec_in.shape[1]
+    d, dec = sv.decw, model.decoder
+    h1d, dec_in = sv.h1d, sv.dec_in
+    with engine.TIMERS.span("train_head_bwd"):
+        dw2, _ = grads.get(dec[2].weight); db2, _ = grads.get(dec[2].bias)
+        sgemm(dpred, F32, 1, out_dim, h1d, F32, 64, 1, out_dim, 64, g_count, dw2, F32, 64)
+        colsum(dpred, F32, g_count, out_dim, out_dim, db2)
+        dh1d = _f32((g_count, 64), dev)
+        sgemm(dpred, F32, out_dim, 1, d["w2"], F32, 64, 1, g_count, 64, out_dim, dh1d, F32, 64, mask=h1d, mask_ld=64)
+        dw1, _ = grads.get(dec[0].weight); db1, _ = grads.get(dec[0].bias)
+        sgemm(dh1d, F32, 1, 64, dec_in, F32, in_dim, 1, 64, in_dim, g_count, dw1, F32, in_dim)
+        colsum(dh1d, F32, g_count, 64, 64, db1)
+        dpooled = _f32((g_count, in_dim), dev)
+        if sv.mlp is None:
+            sgemm(dh1d, F32, 64, 1, d["w1"], F32, in_dim, 1, g_count, in_dim, 64, dpooled, F32, in_dim)
+        else:                                                   # through relu(Linear(128, 128)) of MLPPooling
+            lin, wp = sv.mlp
+            dpm = _f32((g_count, 128), dev)
+            sgemm(dh1d, F32, 64, 1, d["w1"], F32, 128, 1, g_count, 128, 64, dpm, F32, 128, mask=dec_in, mask_ld=128)
+            dwp, _ = grads.get(lin.weight); dbp, _ = grads.get(lin.bias)
+            sgemm(dpm, F32, 1, 128, sv.raw, F32, 128, 1, 128, 128, g_count, dwp, F32, 128)
+            colsum(dpm, F32, g_count, 128, 128, dbp)
+            sgemm(dpm, F32, 128, 1, wp, F32, 128, 1, g_count, 128, 128, dpooled, F32, 128)
+        dcur = Activation(n, 128, prec, dev)
+        capi.pool_backward(dpooled.data_ptr(), in_dim, sv.idx.graph_ptr.data_ptr(), g_count,
+                           capi.POOL_MODES[model.pooling_layer], n, dcur.data.data_ptr(), code, _stream(), width=128)
+    return dcur
+
+
 def head_forward_train(model, cur: Activation, idx, sv) -> torch.Tensor:
     """get_pooling_layer + decoder (Models/BuckGNN.py:246-307, 515-516): the pooled feature comes from bg_pool_head
     (its own decoder output is not used here); MLPPooling and the decoder run on bg_sgemm so that their hidden
     layers are kept for the backward pass."""
+    if cur.data.shape[1] == 128:
+        return _head_forward_train128(model, cur, idx, sv)
     dev = cur.data.device
     dec = model.decoder
     decw = {"w1": dec[0].weight.detach(), "b1": dec[0].bias.detach(), "w2": dec[2].weight.detach(),
@@ -265,7 +391,9 @@ def head_forward_train(model, cur: Activation, idx, sv) -> torch.Tensor:
 
 
 def head_backward(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
-    """Decoder (+ MLPPooling) and pooling backward: returns d(last layer output) [n, 512]."""
+    """Decoder (+ MLPPooling) and pooling backward: returns d(last layer output) [n, 512] ([n, 128] at width 128)."""
+    if sv.h2d is None:
+        return _head_backward128(model, sv, dpred, n, prec, grads)
     dev = dpred.device
     code = engine.PRECISION_FORMATS[prec][0]
     F32 = capi.BG_F32
@@ -369,6 +497,11 @@ class SageTrainFunction(torch.autograd.Function):
         s = _stream()
         x = x.detach().to(torch.float32).contiguous()
         n = x.shape[0]
+        W = model.hidden_channels                          # 512, or 128 (BuckGNN.native128_train)
+        if W not in (512, 128):
+            raise NotImplementedError(f"buckgnn_b200: the training step runs at width 512 or 128, not {W}")
+        if W == 128 and is_node_level(model):
+            raise NotImplementedError("buckgnn_b200: the 128-wide training step has graph-level heads only")
         convs = model._sage_layers()
         L = len(convs)
         aggr = convs[0][0].aggr if convs else "mean"      # no layers: the default model_name (encoder -> pool -> decoder)
@@ -380,12 +513,12 @@ class SageTrainFunction(torch.autograd.Function):
         for c, _ in convs:
             if all(c is not q for q in uniq_convs):
                 uniq_convs.append(c)
-        biases = torch.stack([enc[4].bias.detach().float()] + [c.lin_l.bias.detach().float() for c in uniq_convs]).cpu()
+        biases = torch.stack([enc[-1].bias.detach().float()] + [c.lin_l.bias.detach().float() for c in uniq_convs]).cpu()
         bias_of = {id(c): biases[1 + k] for k, c in enumerate(uniq_convs)}
 
         sv = _Saved()
         sv.model, sv.prec, sv.n, sv.x, sv.seed, sv.p_drop, sv.aggr = model, prec, n, x, seed, p_drop, aggr
-        sv.h1, sv.h2, cur = encoder_forward_train(enc, x, prec, biases[0])          # Models/BuckGNN.py:323
+        sv.h1, sv.h2, cur = encoder_forward_train(enc, x, prec, biases[0], width=W)  # Models/BuckGNN.py:323
         idx = pending.finish()
         sv.idx = idx
         sv.edge_index = pending.edge_index
@@ -394,22 +527,22 @@ class SageTrainFunction(torch.autograd.Function):
         sv.layers = []
         ws_bytes = capi.train_workspace_bytes(n)
         ws = _ws(ws_bytes, dev)
-        ones = torch.ones(512, dtype=torch.float32, device=dev)
-        zeros = torch.zeros(512, dtype=torch.float32, device=dev)
+        ones = torch.ones(W, dtype=torch.float32, device=dev)
+        zeros = torch.zeros(W, dtype=torch.float32, device=dev)
         for i, (conv, bn) in enumerate(convs):
             if id(conv) not in packs:
                 packs[id(conv)] = (engine.pack_linear(conv.lin_l.weight, prec), engine.pack_linear(conv.lin_r.weight, prec))
             wl, wr = packs[id(conv)]
-            agg = Activation(n, 512, prec, dev)
+            agg = Activation(n, W, prec, dev)
             engine.aggregate(cur, agg, idx, aggr)
-            u = Activation(n, 512, prec, dev)
+            u = Activation(n, W, prec, dev)
             inv_norm = _f32((n,), dev)
             with engine.TIMERS.span("train_update_gemm"):
-                engine.gemm512(engine._segments(agg, wl) + engine._segments(cur, wr), n, prec, u,
-                               bias=bias_of[id(conv)].data_ptr(), normalize=True, inv_norm_out=inv_norm.data_ptr())
+                engine.gemm(engine._segments(agg, wl) + engine._segments(cur, wr), n, prec, u,
+                            bias=bias_of[id(conv)].data_ptr(), normalize=True, inv_norm_out=inv_norm.data_ptr())
             vec = None
             if bn is not None:
-                vec = _f32((4, 512), dev)              # a, shift, mean, invstd
+                vec = _f32((4, W), dev)                # a, shift, mean, invstd
                 track = bn.track_running_stats and bn.running_mean is not None
                 momentum = 0.1 if bn.momentum is None else float(bn.momentum)
                 with engine.TIMERS.span("train_bn_stats"):
@@ -418,15 +551,15 @@ class SageTrainFunction(torch.autograd.Function):
                                         bn.running_var.data_ptr() if track else None,
                                         bn.num_batches_tracked.data_ptr() if track else None,
                                         vec[0].data_ptr(), vec[1].data_ptr(), vec[2].data_ptr(), vec[3].data_ptr(),
-                                        ws.data_ptr(), ws_bytes, s)
+                                        ws.data_ptr(), ws_bytes, s, width=W)
                 a_vec, shift_vec = vec[0], vec[1]
             else:
                 a_vec, shift_vec = ones, zeros
             residual = 0 < i < L - 1
-            y = Activation(n, 512, prec, dev)
+            y = Activation(n, W, prec, dev)
             with engine.TIMERS.span("train_bn_act"):
                 capi.bn_act_forward(u.data.data_ptr(), cur.data.data_ptr() if residual else None, y.data.data_ptr(), code, n,
-                                    a_vec.data_ptr(), shift_vec.data_ptr(), p_drop, layer_seed(seed, i), s)
+                                    a_vec.data_ptr(), shift_vec.data_ptr(), p_drop, layer_seed(seed, i), s, width=W)
             y.refresh_split()
             sv.layers.append((conv, bn, cur, agg, u, inv_norm, vec, residual))
             cur = y
@@ -461,11 +594,12 @@ class SageTrainFunction(torch.autograd.Function):
         tpacks = {}
         mean = sv.aggr == "mean"
         L = len(sv.layers)
+        W = model.hidden_channels
         for i in range(L - 1, -1, -1):
             conv, bn, x_in, agg, u, inv_norm, vec, residual = sv.layers[i]
-            dz = Activation(n, 512, prec, dev)
-            dzs = Activation(n, 512, prec, dev) if mean else dz
-            g = Activation(n, 512, prec, dev) if residual else None
+            dz = Activation(n, W, prec, dev)
+            dzs = Activation(n, W, prec, dev) if mean else dz
+            g = Activation(n, W, prec, dev) if residual else None
             if bn is not None:
                 dgam, acc_g = grads.get(bn.weight); dbet, _ = grads.get(bn.bias)
                 a_vec, shift_vec, mean_vec, invstd_vec = vec[0], vec[1], vec[2], vec[3]
@@ -479,7 +613,7 @@ class SageTrainFunction(torch.autograd.Function):
                                         a_vec.data_ptr(), shift_vec.data_ptr(), _p(mean_vec), _p(invstd_vec), sv.p_drop,
                                         layer_seed(sv.seed, i), _p(dgam), _p(dbet), acc_g, dz.data.data_ptr(),
                                         dzs.data.data_ptr() if mean else None, None if g is None else g.data.data_ptr(),
-                                        ws.data_ptr(), ws_bytes, s)
+                                        ws.data_ptr(), ws_bytes, s, width=W)
             dz.refresh_split()
             if mean:
                 dzs.refresh_split()
@@ -487,33 +621,33 @@ class SageTrainFunction(torch.autograd.Function):
             with engine.TIMERS.span("train_wgrad"):
                 dwl, acc_l = grads.get(conv.lin_l.weight)
                 dwr, acc_r = grads.get(conv.lin_r.weight)
-                weight_grad_mn(dz.data, agg.data, code, n, dwl, acc_l)
-                weight_grad_mn(dz.data, x_in.data, code, n, dwr, acc_r)
+                sage_weight_grads(dz.data, agg.data, x_in.data, code, n, dwl, acc_l, dwr, acc_r)
                 dbl, acc_b = grads.get(conv.lin_l.bias)
-                colsum(dz.data, code, n, 512, 512, dbl, accumulate=acc_b)
+                colsum(dz.data, code, n, W, W, dbl, accumulate=acc_b)
             # input gradient: dx = dz Wr + A^T (dz/deg Wl)  (+ g, added by the next iteration through dy2)
             if id(conv) not in tpacks:
                 tpacks[id(conv)] = (transposed_pack(conv.lin_l.weight, prec), transposed_pack(conv.lin_r.weight, prec))
             wlt, wrt = tpacks[id(conv)]
-            dagg = Activation(n, 512, prec, dev)
+            dagg = Activation(n, W, prec, dev)
             with engine.TIMERS.span("train_dgrad_gemm"):
-                engine.gemm512(engine._segments(dzs, wlt), n, prec, dagg)
-            sbuf = Activation(n, 512, prec, dev)
+                engine.gemm(engine._segments(dzs, wlt), n, prec, dagg)
+            sbuf = Activation(n, W, prec, dev)
             if sv.aggr == "max":                     # the gradient goes to the neighbours that attain the maximum
-                wtmp = Activation(n, 512, prec, dev)
+                wtmp = Activation(n, W, prec, dev)
                 mb = capi.max_bwd_workspace_bytes(idx.n_big, idx_t.n_big)
                 mws = _ws(mb, dev)
                 with engine.TIMERS.span("train_max_bwd"):
                     capi.max_aggregate_backward(x_in.data.data_ptr(), agg.data.data_ptr(), dagg.data.data_ptr(), code, n,
                                                 idx.rowptr.data_ptr(), idx.col.data_ptr(), idx.big_rows.data_ptr(), idx.n_big,
                                                 idx_t.rowptr.data_ptr(), idx_t.col.data_ptr(), idx_t.big_rows.data_ptr(),
-                                                idx_t.n_big, wtmp.data.data_ptr(), sbuf.data.data_ptr(), mws.data_ptr(), mb, s)
+                                                idx_t.n_big, wtmp.data.data_ptr(), sbuf.data.data_ptr(), mws.data_ptr(), mb, s,
+                                                width=W)
                 sbuf.refresh_split()
             else:
                 engine.aggregate(dagg, sbuf, idx_t, "sum")
-            dx = Activation(n, 512, prec, dev)
+            dx = Activation(n, W, prec, dev)
             with engine.TIMERS.span("train_dgrad_gemm"):
-                engine.gemm512(engine._segments(dz, wrt), n, prec, dx, residual=sbuf.data.data_ptr(), ldr=512)
+                engine.gemm(engine._segments(dz, wrt), n, prec, dx, residual=sbuf.data.data_ptr(), ldr=W)
             if first_use[id(conv)] == i:
                 grads.done([conv.lin_l.weight, conv.lin_l.bias, conv.lin_r.weight] +
                            ([bn.weight, bn.bias] if bn is not None else []))

@@ -450,6 +450,43 @@ int bg_max_aggregate_backward(const void* x, const void* agg, const void* dagg, 
                               const int32_t* rowptr_src, const int32_t* col_src, const int32_t* big_rows_src, int32_t n_big_src,
                               void* w_scratch, void* dx, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------ training step at width 128
+ * The same layer step for a hidden_channels = 128 model on rows [N, 128] (BuckGNN.native128_train): every argument and
+ * rule is the one of the 512-wide entry point above, with 128 for 512 --
+ *   bg_bn_batch_stats128, bg_bn_act_forward128, bg_sage_backward_rows128: u / x_prev / y / dy / dy2 / dz / dz_scaled /
+ *     g_out [N, 128]; the BatchNorm vectors [128]; workspace from bg_train_workspace_bytes(N) (as at 512).  The dropout
+ *     element index stays r*512 + c, so the mask is the first 128 columns of the 512-wide one (bg_dropout_mask).
+ *   bg_pool_backward128: dx [N, 128]; dpooled [G, >= 128] (ld = ldp), [G, 256] for BG_POOL_SUPERNODE_WITH_POOLING.
+ *   bg_max_aggregate_backward128: x, agg, dagg, w_scratch, dx [N, 128]; workspace from bg_max_bwd_workspace_bytes.
+ * bg_wgrad128: both weight gradients of a 128-wide SAGE layer in one tcgen05 launch,
+ *     dwl[o, i] (+)= sum_n dz[n, o] agg[n, i],   dwr[o, i] (+)= sum_n dz[n, o] x[n, i]     (f32 [128, 128] each)
+ *   dz, agg, x: contiguous [n_rows, 128] of `dtype`, read in place as MN-major operands (no transposed copies; f32 =
+ *   tf32 operands with the 32-byte-atom swizzle).  Split over the nodes as bg_wgrad512: chunk s covers rows
+ *   [s*chunk_k, (s+1)*chunk_k), chunk_k a multiple of 64 (16-bit) / 32 (tf32), n_chunks*chunk_k >= n_rows; one
+ *   256 x 128 tile [dWl^T ; dWr^T] per chunk and CTA pair goes to partial ([n_chunks * 256, 128] f32, caller-owned),
+ *   then a second kernel sums the chunks in order and transposes.  accumulate != 0 adds into dwl / dwr.  No
+ *   floating-point atomics: repeated calls are bit-identical. */
+int bg_bn_batch_stats128(const void* u, int dtype, int64_t n_rows, const float* gamma, const float* beta, float eps,
+                         float momentum, float* running_mean, float* running_var, int64_t* num_batches_tracked,
+                         float* a_out, float* shift_out, float* mean_out, float* invstd_out,
+                         void* workspace, size_t workspace_bytes, void* stream);
+int bg_bn_act_forward128(const void* u, const void* x_prev, void* y, int dtype, int64_t n_rows, const float* a,
+                         const float* shift, float dropout_p, uint64_t seed, void* stream);
+int bg_sage_backward_rows128(const void* u, const void* dy, const void* dy2, const float* inv_norm, const int32_t* rowptr,
+                             int dtype, int64_t n_rows, const float* a, const float* shift, const float* mean,
+                             const float* invstd, float dropout_p, uint64_t seed, float* dgamma, float* dbeta,
+                             int accumulate, void* dz, void* dz_scaled, void* g_out,
+                             void* workspace, size_t workspace_bytes, void* stream);
+int bg_pool_backward128(const float* dpooled, int64_t ldp, const int32_t* graph_ptr, int64_t n_graphs, int pool_mode,
+                        int64_t n_nodes, void* dx, int dtype, void* stream);
+int bg_max_aggregate_backward128(const void* x, const void* agg, const void* dagg, int dtype, int64_t n_nodes,
+                                 const int32_t* rowptr_tgt, const int32_t* col_tgt, const int32_t* big_rows_tgt,
+                                 int32_t n_big_tgt, const int32_t* rowptr_src, const int32_t* col_src,
+                                 const int32_t* big_rows_src, int32_t n_big_src,
+                                 void* w_scratch, void* dx, void* workspace, size_t workspace_bytes, void* stream);
+int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64_t n_rows, int32_t n_chunks,
+                int64_t chunk_k, float* partial, float* dwl, float* dwr, int accumulate, void* stream);
+
 /* Device-side collate (SURVEY.md section 8 row f1): PyG `DataLoader` / `Batch.from_data_list` for a dataset kept in HBM in
  * concatenated form -- x_all [sum n, F], ei_all [2, E_all] with node ids LOCAL to their graph (as
  * GraphCreate.py:417-432 emits them), ea_all [E_all, Fe], y_all [G_all], node_ptr / edge_ptr [G_all+1] int64.
