@@ -30,7 +30,7 @@ EXPORTED_SYMBOLS = (
     "bg_csr_max_big_rows", "bg_csr_workspace_bytes", "bg_csr_build",
     "bg_batch_info", "bg_graph_ptr_build", "bg_publish_words", "bg_encoder_front",
     "bg_aggregate_workspace_bytes", "bg_hubfold_workspace_bytes", "bg_sage_aggregate", "bg_gemm512",
-    "bg_sage_fused512", "bg_sage_aggregate_hubs", "bg_gemm128", "bg_pool_head128", "bg_pool_head_blocks128",
+    "bg_sage_fused512", "bg_sage_aggregate_hubs", "bg_gemm128", "bg_gemm128_gathered", "bg_pool_head128", "bg_pool_head_blocks128",
     "bg_wgrad512", "bg_pool_workspace_bytes", "bg_pool_head", "bg_pool_block_flags", "bg_pool_head_blocks", "bg_cast_f32", "bg_split_tf32",
     "bg_expand_rowptr", "bg_add",
     "bg_train_workspace_bytes", "bg_bn_batch_stats", "bg_bn_act_forward", "bg_sage_backward_rows",
@@ -98,6 +98,8 @@ _SIGNATURES = {
     "bg_sage_aggregate_hubs": (C.c_int, [_P, C.c_int, _P, _P, _P, _I32, C.c_int, _P, _P, C.c_size_t, _P]),
     "bg_gemm128": (C.c_int, [C.POINTER(GemmSegment), _I32, _I64, C.c_int, C.c_int, C.POINTER(Epilogue), _P,
                              C.c_int, _I64, C.c_int, _P]),
+    "bg_gemm128_gathered": (C.c_int, [C.POINTER(GemmSegment), _I32, _I64, C.c_int, C.c_int, C.POINTER(Epilogue), _P,
+                                      C.c_int, _I64, C.c_int, _P]),
     "bg_pool_head128": (C.c_int, [_P, C.c_int, _I64, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _P, _P,
                                   _P, C.c_size_t, _P, _P]),
     "bg_pool_head_blocks128": (C.c_int, [_P, C.c_int, _I64, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _P,
@@ -292,6 +294,22 @@ def gemm128(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=
                    gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
     _check(load().bg_gemm128(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group, stream),
            "bg_gemm128")
+
+
+def gemm128_gathered(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
+                     bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
+                     gather=(), gather_ld=128, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+    """bg_gemm128_gathered: gemm128 plus up to two (matrix_ptr, index_ptr) pairs of gathered pre-activation addends,
+    [*, 128] rows of the output dtype with leading dimension gather_ld.  The library rejects them together with
+    normalize, residual or pool fusion."""
+    n = len(segments)
+    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
+    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
+    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
+    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
+                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
+    _check(load().bg_gemm128_gathered(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group,
+                                      stream), "bg_gemm128_gathered")
 
 
 def sage_fused512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, x, ldx, rowptr, col, aggr, hub_agg=None,

@@ -665,39 +665,53 @@ int bg_sage_fused512(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int 
   return gemm512_impl(segs, n_seg, m, a_dtype, b_dtype, epi, fuse, out, out_dtype, ldo, 2, stream_);
 }
 
-int bg_gemm128(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtype, int b_dtype,
-               const bg_epilogue* epi, void* out, int out_dtype, int64_t ldo, int cta_group, void* stream_) {
+// bg_gemm128 and bg_gemm128_gathered: the gathered addends are only accepted through the second entry point
+static int gemm128_impl(const char* fn, bool gathered, const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtype,
+                        int b_dtype, const bg_epilogue* epi, void* out, int out_dtype, int64_t ldo, int cta_group,
+                        void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   // every argument is checked before the first CUDA call
-  if (!segs || n_seg < 1 || n_seg > BG_MAX_GEMM_SEGMENTS) return fail(BG_ERR_INVALID, "bg_gemm128: bad segment count");
-  if (m < 0 || m >= 0x7fffffffLL) return fail(BG_ERR_INVALID, "bg_gemm128: bad m");
+  if (!segs || n_seg < 1 || n_seg > BG_MAX_GEMM_SEGMENTS) return fail_in(BG_ERR_INVALID, fn, "bad segment count");
+  if (m < 0 || m >= 0x7fffffffLL) return fail_in(BG_ERR_INVALID, fn, "bad m");
   const int a_fmt = umma_format_of(a_dtype), b_fmt = umma_format_of(b_dtype);
   if (a_fmt < 0 || b_fmt < 0 || a_fmt != b_fmt)
-    return fail(BG_ERR_INVALID, "bg_gemm128: a_dtype and b_dtype must be the same (bf16, f16 or f32)");
-  if (umma_format_of(out_dtype) < 0) return fail(BG_ERR_INVALID, "bg_gemm128: bad out_dtype");
-  if (cta_group != 2) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: only cta_group = 2 is built");
+    return fail_in(BG_ERR_INVALID, fn, "a_dtype and b_dtype must be the same (bf16, f16 or f32)");
+  if (umma_format_of(out_dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad out_dtype");
+  if (cta_group != 2) return fail_in(BG_ERR_UNSUPPORTED, fn, "only cta_group = 2 is built");
   const bool tf32 = a_fmt == 2;
   const int esz = tf32 ? 4 : 2, osz = out_dtype == BG_F32 ? 4 : 2;
   const int kblk = kStageKBytes / esz;
-  if (!out || !aligned16(out) || (ldo * osz) % 16 != 0 || ldo < kW128) return fail(BG_ERR_INVALID, "bg_gemm128: bad out/ldo");
+  if (!out || !aligned16(out) || (ldo * osz) % 16 != 0 || ldo < kW128) return fail_in(BG_ERR_INVALID, fn, "bad out/ldo");
   for (int s = 0; s < n_seg; ++s) {
     const bg_gemm_segment& g = segs[s];
-    if (!g.a || !g.b) return fail(BG_ERR_INVALID, "bg_gemm128: null operand");
-    if (g.k <= 0 || g.k % kblk != 0) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: k must be a positive multiple of 64 (16-bit) / 32 (tf32)");
-    if (g.b_groups > 1) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: b_groups is not built at width 128");
+    if (!g.a || !g.b) return fail_in(BG_ERR_INVALID, fn, "null operand");
+    if (g.k <= 0 || g.k % kblk != 0) return fail_in(BG_ERR_UNSUPPORTED, fn, "k must be a positive multiple of 64 (16-bit) / 32 (tf32)");
+    if (g.b_groups > 1) return fail_in(BG_ERR_UNSUPPORTED, fn, "b_groups is not built at width 128");
     if (!aligned16(g.a) || (g.lda * esz) % 16 != 0 || g.lda < g.k || !aligned16(g.b) || (g.ldb * esz) % 16 != 0 || g.ldb < g.k)
-      return fail(BG_ERR_INVALID, "bg_gemm128: operand alignment / leading dimension");
+      return fail_in(BG_ERR_INVALID, fn, "operand alignment / leading dimension");
   }
+  int n_gather = 0;
   if (epi) {
-    if (epi->gather[0] || epi->gather[1]) return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: gathered addends are not built at width 128");
+    if (!gathered && (epi->gather[0] || epi->gather[1]))
+      return fail_in(BG_ERR_UNSUPPORTED, fn, "gathered addends are not built here (use bg_gemm128_gathered)");
+    if (gathered) {
+      if (!epi->gather[0] && epi->gather[1]) return fail_in(BG_ERR_INVALID, fn, "gather[1] without gather[0]");
+      for (int k = 0; k < 2 && epi->gather[k]; ++k) {
+        if (!epi->gather_idx[k] || !aligned16(epi->gather[k]) || epi->gather_ld < kW128 || (epi->gather_ld * osz) % 16 != 0)
+          return fail_in(BG_ERR_INVALID, fn, "bad gather operand (null index, misaligned, or gather_ld < 128 / rows not 16-byte aligned)");
+        n_gather = k + 1;
+      }
+      if (n_gather > 0 && (epi->normalize || epi->residual || epi->pool_block_sums || epi->pool_block_keep))
+        return fail_in(BG_ERR_UNSUPPORTED, fn, "gathered addends cannot be combined with normalize, residual or pool fusion");
+    }
     if (epi->residual && (!aligned16(epi->residual) || (epi->ldr * osz) % 16 != 0 || epi->ldr < kW128))
-      return fail(BG_ERR_INVALID, "bg_gemm128: bad residual/ldr");
-    if (epi->bn_scale_host && !epi->bn_shift_host) return fail(BG_ERR_INVALID, "bg_gemm128: bn_scale without bn_shift");
-    if (epi->inv_norm_out && !epi->normalize) return fail(BG_ERR_INVALID, "bg_gemm128: inv_norm_out needs normalize");
+      return fail_in(BG_ERR_INVALID, fn, "bad residual/ldr");
+    if (epi->bn_scale_host && !epi->bn_shift_host) return fail_in(BG_ERR_INVALID, fn, "bn_scale without bn_shift");
+    if (epi->inv_norm_out && !epi->normalize) return fail_in(BG_ERR_INVALID, fn, "inv_norm_out needs normalize");
     if ((epi->pool_block_sums != nullptr) != (epi->pool_block_keep != nullptr))
-      return fail(BG_ERR_INVALID, "bg_gemm128: pool_block_sums and pool_block_keep go together");
+      return fail_in(BG_ERR_INVALID, fn, "pool_block_sums and pool_block_keep go together");
     if (epi->pool_block_sums && (!epi->normalize || out_dtype == BG_F32 || epi->residual || !aligned16(epi->pool_block_sums)))
-      return fail(BG_ERR_UNSUPPORTED, "bg_gemm128: the pool-fused epilogue needs normalize, a 16-bit output and no residual");
+      return fail_in(BG_ERR_UNSUPPORTED, fn, "the pool-fused epilogue needs normalize, a 16-bit output and no residual");
   }
   if (m == 0) return BG_OK;
   Gemm128Params p;
@@ -706,7 +720,7 @@ int bg_gemm128(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtyp
     const bg_gemm_segment& g = segs[s];
     int rc = make_operand_map(&p.seg[s].a, g.a, m, g.k, g.lda, (uint32_t)a_fmt);
     if (rc == BG_OK) rc = make_operand_map_rows(&p.seg[s].b, g.b, kW128, g.k, g.ldb, (uint32_t)b_fmt, kG128BRows);
-    if (rc != BG_OK) return fail(rc, "bg_gemm128: cuTensorMapEncodeTiled failed");
+    if (rc != BG_OK) return fail_in(rc, fn, "cuTensorMapEncodeTiled failed");
     p.kblocks[s] = g.k / kblk;
   }
   p.n_seg = n_seg;
@@ -725,17 +739,35 @@ int bg_gemm128(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtyp
     p.residual = epi->residual; p.ldr = epi->ldr;
     p.inv_norm_out = epi->inv_norm_out;
     p.pool_sums = epi->pool_block_sums; p.pool_keep = epi->pool_block_keep;
+    for (int k = 0; k < n_gather; ++k) { p.gather[k] = epi->gather[k]; p.gidx[k] = epi->gather_idx[k]; }
+    p.n_gather = n_gather;
+    p.gather_ld = epi->gather_ld;
   }
   p.out = out; p.ldo = ldo;
   if (p.pool_sums)
     return out_dtype == BG_BF16 ? launch_gemm128<__nv_bfloat16, false, true>(p, stream)
                                 : launch_gemm128<__half, false, true>(p, stream);
+  if (n_gather > 0)
+    return out_dtype == BG_BF16 ? launch_gemm128<__nv_bfloat16, false, false, false, true>(p, stream)
+         : out_dtype == BG_F16  ? launch_gemm128<__half, false, false, false, true>(p, stream)
+                                : launch_gemm128<float, false, false, false, true>(p, stream);
 #define BG_GEMM128_OUT(RES)                                                              \
   (out_dtype == BG_BF16 ? launch_gemm128<__nv_bfloat16, RES, false>(p, stream)           \
    : out_dtype == BG_F16 ? launch_gemm128<__half, RES, false>(p, stream)                 \
                          : launch_gemm128<float, RES, false>(p, stream))
   return p.residual ? BG_GEMM128_OUT(true) : BG_GEMM128_OUT(false);
 #undef BG_GEMM128_OUT
+}
+
+int bg_gemm128(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtype, int b_dtype,
+               const bg_epilogue* epi, void* out, int out_dtype, int64_t ldo, int cta_group, void* stream_) {
+  return gemm128_impl("bg_gemm128", false, segs, n_seg, m, a_dtype, b_dtype, epi, out, out_dtype, ldo, cta_group, stream_);
+}
+
+int bg_gemm128_gathered(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, int a_dtype, int b_dtype,
+                        const bg_epilogue* epi, void* out, int out_dtype, int64_t ldo, int cta_group, void* stream_) {
+  return gemm128_impl("bg_gemm128_gathered", true, segs, n_seg, m, a_dtype, b_dtype, epi, out, out_dtype, ldo, cta_group,
+                      stream_);
 }
 
 int bg_sage_aggregate_hubs(const void* x, int dtype, const int32_t* rowptr, const int32_t* col, const int32_t* big_rows,

@@ -19,6 +19,10 @@
 //              of output at a time, applies bias / normalize / BN / ReLU / skip in fp32 (one rounding of the result)
 //              and moves the rows through a 4 KB swizzled staging tile per warp, so that global loads and stores are
 //              coalesced (8 lanes per 128-byte row piece).
+// kGather (bg_gemm128_gathered, the edge GEMMs of a 128-wide EA-GNN layer): up to two rows G_k[gidx_k[m], 0:128] of
+// the output dtype are added to output row m before the activation, out = relu(acc + bias + G_0[i0] + G_1[i1]), in fp32
+// with one rounding of the result.  They travel like the skip rows (8 lanes per 128-byte row piece, through the staging
+// tile), the row index read once per row and broadcast by shuffle.
 // kMn (bg_wgrad128, the weight gradients of a 128-wide SAGE layer): both operands MN-major, read in place from row-major
 // [n_rows, 128] matrices (no transposed copies), the reduction over nodes.  Tile t = node chunk t: the CTA of rank 0
 // loads agg^T, rank 1 loads x^T as its 128 rows of the M = 256 A operand, both CTAs their 64-column half of dz as B, so
@@ -60,16 +64,22 @@ struct alignas(64) Gemm128Params {
   float scale[kW128];               // 1 when there is no BN
   float shift[kW128];               // 0 when there is no BN
   int64_t chunk_k;                  // kMn: nodes per chunk (a multiple of k_elems_per_block)
+  // kGather (appended: the fields above keep their constant-bank offsets)
+  const void* gather[2];            // [*, 128] row-major matrices of the output dtype, ld = gather_ld
+  const int32_t* gidx[2];           // [M] row index into gather[k]
+  int32_t n_gather;                 // 1 or 2
+  int64_t gather_ld;
 };
 
 // One epilogue warp: 32 TMEM lanes = 32 output rows of the tiles of parity g.  kPool as in k_gemm512 (last layer of a
 // graph-level model, 16-bit output): per 32-row block and column the fp32 sum of the stored (rounded) values goes to
 // pool_sums, and only the blocks flagged in pool_keep are stored.
-template <typename TOut, bool kRes, bool kPool>
+template <typename TOut, bool kRes, bool kPool, bool kGather = false>
 BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base, const uint32_t stage_u32,
                                 const uint32_t tmem_full_bar, const uint32_t tmem_empty_bar, const uint32_t rank,
                                 const int tile0, const int tile_stride, const int g) {
   static_assert(!kPool || (sizeof(TOut) == 2 && !kRes), "pool-fused epilogue: 16-bit output, no skip rows");
+  static_assert(!kGather || (!kRes && !kPool), "gathered addends: no skip rows, no pool fusion");
   constexpr bool kOut16 = sizeof(TOut) == 2;
   constexpr size_t esz = sizeof(TOut);
   constexpr int kChunkCols = 128 / (int)esz;                    // output columns per 128-byte row piece: 64 / 32
@@ -97,6 +107,13 @@ BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base
     [[maybe_unused]] const char* res_base = nullptr;
     if constexpr (kRes)
       res_base = reinterpret_cast<const char*>(p.residual) + (size_t)(warp_row0 + r4) * p.ldr * esz + piece * 16;
+    // kGather: gathered rows of one 128-byte chunk in the same layout, one matrix at a time (G_1 is loaded only after
+    // G_0 has been folded into the accumulator registers: holding both would spill the 16-bit instances)
+    [[maybe_unused]] int32_t gi[2] = {0, 0};
+    [[maybe_unused]] uint4 gpre[kGather ? 8 : 1];
+    if constexpr (kGather) {
+      if (m_row < p.m) { gi[0] = p.gidx[0][m_row]; if (p.n_gather > 1) gi[1] = p.gidx[1][m_row]; }
+    }
     auto fetch = [&](int ch) {
       if constexpr (kRes) {
 #pragma unroll
@@ -105,7 +122,27 @@ BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base
                                             : make_uint4(0u, 0u, 0u, 0u);
       }
     };
+    [[maybe_unused]] auto fetch_gather = [&](int k, int ch) {
+      const char* g_base = reinterpret_cast<const char*>(p.gather[k]) + piece * 16 + ch * 128;
+#pragma unroll
+      for (int t = 0; t < 8; ++t) {
+        const int32_t n = __shfl_sync(0xffffffffu, gi[k], t * 4 + r4);
+        gpre[t] = (t * 4 + r4 < rows_here) ? ldg_nc_v4(g_base + (size_t)n * p.gather_ld * esz) : make_uint4(0u, 0u, 0u, 0u);
+      }
+    };
+    // adds the 16-byte piece `u` of a gathered row (kPer values of the output dtype) to v[0..kPer) in fp32
+    [[maybe_unused]] auto add_piece = [&](float* v, const uint4 u) {
+      const uint32_t au[4] = {u.x, u.y, u.z, u.w};
+      if constexpr (kOut16) {
+#pragma unroll
+        for (int e = 0; e < 4; ++e) Pack16<TOut>::add2(v[2 * e], v[2 * e + 1], au[e]);
+      } else {
+#pragma unroll
+        for (int e = 0; e < 4; ++e) v[e] += __uint_as_float(au[e]);
+      }
+    };
     fetch(0);                                                   // in flight while the MMAs run
+    if constexpr (kGather) fetch_gather(0, 0);
 
     mbar_wait(tmem_full_bar, j & 1u, kTagTmemFull);
     tc_fence_after();
@@ -148,15 +185,46 @@ BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base
         if (rank == 0) mbar_arrive(tmem_empty_bar);
         else mbar_arrive_cluster(tmem_empty_bar, 0);
       }
+      if constexpr (kGather) {                                  // G_0 joins the accumulator registers, G_1 waits staged
+        auto stage = [&]() {
+#pragma unroll
+          for (int t = 0; t < 8; ++t) sts_v4(((t & 1) ? coop_odd : coop_even) + (uint32_t)(t >> 1) * 1024u, gpre[t]);
+          __syncwarp();
+        };
+        stage();
+#pragma unroll
+        for (int jp = 0; jp < 8; ++jp) {
+          float a[kPer];
+#pragma unroll
+          for (int e = 0; e < kPer; ++e) a[e] = __uint_as_float(r[jp * kPer + e]);
+          add_piece(a, lds_v4(my_row + (((uint32_t)jp ^ my_sw) << 4)));
+#pragma unroll
+          for (int e = 0; e < kPer; ++e) r[jp * kPer + e] = __float_as_uint(a[e]);
+        }
+        __syncwarp();
+        if (p.n_gather > 1) { fetch_gather(1, ch); stage(); }
+        if (ch + 1 < kChunks) fetch_gather(0, ch + 1);
+      }
 #pragma unroll
       for (int jp = 0; jp < 8; ++jp) {                          // 16-byte pieces of this thread's 128-byte row chunk
         const uint32_t addr = my_row + (((uint32_t)jp ^ my_sw) << 4);
         const int c0 = ch * kChunkCols + jp * kPer;
         float v[kPer];
+        if constexpr (kGather) {                                // acc + G_0 + bias + G_1 before the activation
 #pragma unroll
-        for (int e = 0; e < kPer; ++e) {
-          v[e] = fmaf((__uint_as_float(r[jp * kPer + e]) + p.bias[c0 + e]) * inv, p.scale[c0 + e], p.shift[c0 + e]);
-          if (p.relu) v[e] = fmaxf(v[e], 0.f);
+          for (int e = 0; e < kPer; ++e) v[e] = __uint_as_float(r[jp * kPer + e]) + p.bias[c0 + e];
+          if (p.n_gather > 1) add_piece(v, lds_v4(addr));
+#pragma unroll
+          for (int e = 0; e < kPer; ++e) {
+            v[e] = fmaf(v[e] * inv, p.scale[c0 + e], p.shift[c0 + e]);
+            if (p.relu) v[e] = fmaxf(v[e], 0.f);
+          }
+        } else {
+#pragma unroll
+          for (int e = 0; e < kPer; ++e) {
+            v[e] = fmaf((__uint_as_float(r[jp * kPer + e]) + p.bias[c0 + e]) * inv, p.scale[c0 + e], p.shift[c0 + e]);
+            if (p.relu) v[e] = fmaxf(v[e], 0.f);
+          }
         }
         if constexpr (kRes) {                                   // skip rows enter after the activation
           const uint4 ad = lds_v4(addr);
@@ -213,10 +281,10 @@ BG_DEVINL void epilogue128_warp(const Gemm128Params& p, const uint32_t tmem_base
   }
 }
 
-template <typename TOut, bool kRes, bool kPool, bool kMn = false>
+template <typename TOut, bool kRes, bool kPool, bool kMn = false, bool kGather = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 k_gemm128(const __grid_constant__ Gemm128Params p) {
-  static_assert(!kMn || (sizeof(TOut) == 4 && !kRes && !kPool), "weight-gradient mode: fp32 partials, plain epilogue");
+  static_assert(!kMn || (sizeof(TOut) == 4 && !kRes && !kPool && !kGather), "weight-gradient mode: fp32 partials, plain epilogue");
   constexpr int kStages = kG128Stages;
   extern __shared__ uint8_t gemm128_smem_raw[];
   const uint32_t smem_base = (smem_u32(gemm128_smem_raw) + 1023u) & ~1023u;   // SWIZZLE_128B wants 1024 B
@@ -342,7 +410,7 @@ k_gemm128(const __grid_constant__ Gemm128Params p) {
   } else if (warp >= kEpiFirstWarp && warp < kEpiFirstWarp + kEpiWarps) {
     // ================================================================ epilogue warps 4..11
     const int ew = warp - kEpiFirstWarp, g = ew >> 2;
-    epilogue128_warp<TOut, kRes, kPool>(p, tmem_base, epi_u32 + (uint32_t)ew * kEpiStageBytes, tmem_full_bar(g),
+    epilogue128_warp<TOut, kRes, kPool, kGather>(p, tmem_base, epi_u32 + (uint32_t)ew * kEpiStageBytes, tmem_full_bar(g),
                                         tmem_empty_bar(g), rank, tile0, tile_stride, g);
   }
 
@@ -372,9 +440,9 @@ static inline int make_operand_map_rows(CUtensorMap* map, const void* base, int6
   return r == CUDA_SUCCESS ? BG_OK : BG_ERR_CUDA;
 }
 
-template <typename TOut, bool kRes, bool kPool, bool kMn = false>
+template <typename TOut, bool kRes, bool kPool, bool kMn = false, bool kGather = false>
 static int launch_gemm128(const Gemm128Params& p, cudaStream_t stream) {
-  auto kern = k_gemm128<TOut, kRes, kPool, kMn>;
+  auto kern = k_gemm128<TOut, kRes, kPool, kMn, kGather>;
   static bool attr_set = false;
   if (!attr_set) {
     BG_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kG128SmemBytes));

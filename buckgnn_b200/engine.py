@@ -314,12 +314,13 @@ def gemm512(segs, m: int, precision: str, out: Activation, *, cta_group: int = 2
 
 def gemm(segs, m: int, precision: str, out: Activation, *, cta_group: int = 2, **epi) -> None:
     """The update GEMM for the width of `out`: bg_gemm128 for 128-wide rows (a hidden_channels = 128 model on its own
-    kernels), else bg_gemm512."""
+    kernels; bg_gemm128_gathered when there are gathered addends), else bg_gemm512."""
     if out.data.shape[1] != 128:
         return gemm512(segs, m, precision, out, cta_group=cta_group, **epi)
     a_code, b_code = PRECISION_FORMATS[precision]
-    capi.gemm128(segs, m, a_code, b_code, out.data.data_ptr(), out.code, out.data.shape[1], _stream(),
-                 cta_group=cta_group, **epi)
+    fn = capi.gemm128_gathered if epi.get("gather") else capi.gemm128
+    fn(segs, m, a_code, b_code, out.data.data_ptr(), out.code, out.data.shape[1], _stream(),
+       cta_group=cta_group, **epi)
     out.refresh_split()
 
 
@@ -598,8 +599,9 @@ class GNBlockPack:
     wb2: LinearPack; bb2: torch.Tensor
 
 
-def pack_gnblock(blk, precision: str) -> GNBlockPack:
-    h = 512
+def pack_gnblock(blk, precision: str, width: int = 512) -> GNBlockPack:
+    """`width`: the block's hidden width (512, or 128 for a hidden_channels = 128 model on the 128-wide kernels)."""
+    h = width
     dev = blk.edge_mlp[0].weight.device
     d64 = lambda t: t.detach().to(torch.float64).cpu()
     W1, b1 = d64(blk.edge_mlp[0].weight), d64(blk.edge_mlp[0].bias)
@@ -649,8 +651,8 @@ def add_into(out: Activation, a: Activation, b: Activation) -> None:
 class GNBlockBuffers:
     """Scratch activations of the EA-GNN layer loop (allocated once per forward)."""
 
-    def __init__(self, n: int, e: int, precision: str, device):
-        mk = lambda rows: Activation(rows, 512, precision, device)
+    def __init__(self, n: int, e: int, precision: str, device, width: int = 512):
+        mk = lambda rows: Activation(rows, width, precision, device)
         self.P, self.Q, self.R, self.mh, self.g1, self.xg, self.t, self.s, self.x_alt = (mk(n) for _ in range(9))
         self.he, self.hm, self.e_alt = (mk(max(e, 1)) for _ in range(3))
 
@@ -659,10 +661,12 @@ def gnblock_layer(x: Activation, e: Activation, buf: GNBlockBuffers, idx: GraphI
                   w: GNBlockPack, *, skip: bool, need_edges_out: bool, cta_group: int = 2):
     """One iteration of the EA-GNN loop (Models/BuckGNN.py:378-387): returns (x_next, e_next).
     Edge tensors live in CSR order keyed by `row = edge_index[0]` (idx built with key_row=0), so
-    scatter_mean(messages, row) is a segmented mean over contiguous slots."""
+    scatter_mean(messages, row) is a segmented mean over contiguous slots.  The row width (512, or 128 for a
+    hidden_channels = 128 model) is that of `x`; `gemm` picks the kernel for it."""
     prec, n, ne = x.precision, idx.n_nodes, idx.n_edges
+    width = x.data.shape[1]
     hp = lambda t: t.data_ptr()
-    G = lambda out, segs, m, **kw: gemm512(segs, m, prec, out, cta_group=cta_group, **kw)
+    G = lambda out, segs, m, **kw: gemm(segs, m, prec, out, cta_group=cta_group, **kw)
     with TIMERS.span("gn_node_gemms"):
         G(buf.P, _segments(x, w.w1a), n)
         G(buf.Q, _segments(x, w.w1b), n)
@@ -676,7 +680,7 @@ def gnblock_layer(x: Activation, e: Activation, buf: GNBlockBuffers, idx: GraphI
         if need_edges_out:
             e_next = buf.e_alt
             G(e_next, _segments(buf.he, w.w2), ne, bias=hp(w.b2),
-              residual=e.data.data_ptr() if skip else None, ldr=512)
+              residual=e.data.data_ptr() if skip else None, ldr=width)
         # phi layer 1 (+ReLU) on e1 = h_e W2^T + b2, folded
         G(buf.hm, _segments(buf.he, w.w3c), ne, bias=hp(w.b3c), relu=True,
           gather=[(buf.R.data.data_ptr(), idx.col.data_ptr())])
@@ -686,7 +690,7 @@ def gnblock_layer(x: Activation, e: Activation, buf: GNBlockBuffers, idx: GraphI
     with TIMERS.span("gn_segment_mean"):
         capi.sage_aggregate(buf.hm.data.data_ptr(), buf.mh.data.data_ptr(), buf.hm.code, n, idx.rowptr.data_ptr(),
                             ex.iota.data_ptr(), idx.big_rows.data_ptr(), idx.n_big, capi.BG_AGGR_MEAN,
-                            ws.data_ptr(), ws_bytes, _stream())
+                            ws.data_ptr(), ws_bytes, _stream(), width=width)
     buf.mh.refresh_split()
     with TIMERS.span("gn_node_gemms"):
         gate_segs = _segments(ex.nonempty, w.wgate)[:2]      # the indicator is exact in tf32: its lo part is 0
@@ -697,7 +701,7 @@ def gnblock_layer(x: Activation, e: Activation, buf: GNBlockBuffers, idx: GraphI
         if skip:                                   # x_next = xg + beta(xg) + x_prev
             add_into(buf.s, buf.xg, x)
             res = buf.s
-        G(buf.x_alt, _segments(buf.t, w.wb2), n, bias=hp(w.bb2), residual=res.data.data_ptr(), ldr=512)
+        G(buf.x_alt, _segments(buf.t, w.wb2), n, bias=hp(w.bb2), residual=res.data.data_ptr(), ldr=width)
     x_next = buf.x_alt
     buf.x_alt = x                                  # ping-pong
     if e_next is not None:

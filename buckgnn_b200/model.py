@@ -17,10 +17,11 @@ In train mode (`model.train()`, as TRAIN_FINAL.py:289 does) the forward uses bat
 BatchNorm1d, applies Dropout and is differentiable: `loss.backward()` runs the backward kernels
 (`train.py`) and leaves `.grad` on the parameters that model_name uses.
 
-A hidden_channels = 128 model (the reference's default width) evaluates on its own 128-wide kernels.  It trains on them
-too when `model.native128_train` is set (a module attribute, default from BUCKGNN_NATIVE128_TRAIN=1 in the
-environment); otherwise, and for what the 128-wide step does not cover, training runs as the zero-padded 512-wide
-twin (narrow.py).
+A hidden_channels = 128 GraphSAGE model (the reference's default width) evaluates on its own 128-wide kernels.  It
+trains on them too when `model.native128_train` is set (a module attribute, default from BUCKGNN_NATIVE128_TRAIN=1 in
+the environment); otherwise, and for what the 128-wide step does not cover, training runs as the zero-padded 512-wide
+twin (narrow.py).  A 128-wide EA_GNN / EA_GNN_Shared model evaluates on the 128-wide kernels when
+`model.native128_eagnn` is set (default from BUCKGNN_NATIVE128_EAGNN=1); it always trains as the twin.
 
 Extra, non-reference keywords: `train_precision` in {"tf32", "bf16", "fp16"} (storage of the training
 step's activations and activation gradients; default tf32 = fp32 storage), and `precision` in {"auto", "fp16", "bf16", "tf32", "fp32"}
@@ -52,6 +53,11 @@ _NATIVE128_MODELS = tuple(_SAGE_LISTS) + ("GraphSage_addAggr_Shared", "GraphSAGE
 # train-mode forwards of the same models at hidden_channels == 128 on the 128-wide kernels (train.py at width 128)
 # instead of the twin.  Opt-in: BUCKGNN_NATIVE128_TRAIN=1 in the environment, or `model.native128_train = True`.
 NATIVE128_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_TRAIN", "0") not in ("", "0")
+# EA-GNN models whose eval forward at hidden_channels == 128 runs on the 128-wide kernels (bg_gemm128_gathered for the
+# edge GEMMs) instead of the twin.  Opt-in: BUCKGNN_NATIVE128_EAGNN=1 in the environment, or
+# `model.native128_eagnn = True`.
+_NATIVE128_EAGNN_MODELS = ("EA_GNN", "EA_GNN_Shared")
+NATIVE128_EAGNN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN", "0") not in ("", "0")
 
 
 class SAGEConv(nn.Module):
@@ -160,6 +166,7 @@ class BuckGNN(nn.Module):
         self.fuse_pool = fuse_pool            # last SAGE layer's epilogue sums its rows for the pooling layer (16-bit modes)
         self.fuse_aggregate = engine.FUSE_AGGREGATE_DEFAULT    # the aggregate operand gathered inside the update GEMM (opt-in)
         self.native128_train = NATIVE128_TRAIN_DEFAULT         # hidden_channels 128: train on the 128-wide kernels (opt-in)
+        self.native128_eagnn = NATIVE128_EAGNN_DEFAULT         # hidden_channels 128: EA-GNN eval on the 128-wide kernels (opt-in)
         self.output_dim = output_dim = _output_dim(prediction_type, use_z_coord, use_rotations)
         h = hidden_channels
         cat_dec = pooling_layer == "supernode_with_pooling" and prediction_type == "buckling"
@@ -337,6 +344,15 @@ class BuckGNN(nn.Module):
             if not all(bool(torch.isfinite(t).all()) for pk in (folded.wl3, folded.wr3, folded.wgate) for t in pk.parts):
                 folded = None
         packs["layer0_folded"] = folded
+        if self.model_name in _NATIVE128_EAGNN_MODELS:      # the edge encoder by the same [I; 0] embedding
+            ee = self.edge_encoder
+            packs["edge_enc"] = {"w1": f32(ee[0].weight), "b1": f32(ee[0].bias), "w2": w2, "b2": zeros(128),
+                                 "b3_host": engine.host_vector(ee[2].bias)}
+            packs["edge_enc_w3"] = engine.pack_linear(torch.nn.functional.pad(f32(ee[2].weight), (0, 64)), prec)
+            if self.model_name == "EA_GNN_Shared":
+                packs["gn"] = [engine.pack_gnblock(self.shared_gn_block, prec, width=128)] * self.num_layers
+            else:
+                packs["gn"] = [engine.pack_gnblock(b, prec, width=128) for b in self.gn_blocks]
         self._packs, self._pack_sig = packs, sig
         return packs
 
@@ -357,10 +373,14 @@ class BuckGNN(nn.Module):
 
     def _runs_native128(self) -> bool:
         """hidden_channels == 128 eval forwards of the GraphSAGE models with a graph-level head run on the 128-wide
-        kernels; everything else at a width other than 512 runs on the zero-padded twin (narrow.py)."""
-        return (self.hidden_channels == 128 and not self.training and not self.fuse_aggregate
-                and self.model_name in _NATIVE128_MODELS and self.prediction_type == "buckling"
-                and self.pooling_layer in _POOLINGS)
+        kernels, and those of EA_GNN / EA_GNN_Shared too when `native128_eagnn` is on; everything else at a width other
+        than 512 runs on the zero-padded twin (narrow.py)."""
+        if (self.hidden_channels != 128 or self.training or self.prediction_type != "buckling"
+                or self.pooling_layer not in _POOLINGS):
+            return False
+        if self.model_name in _NATIVE128_EAGNN_MODELS:
+            return bool(self.native128_eagnn)
+        return not self.fuse_aggregate and self.model_name in _NATIVE128_MODELS
 
     def _trains_native128(self) -> bool:
         """With `native128_train` on, train-mode forwards of the models `_runs_native128` covers run the training step
@@ -375,7 +395,10 @@ class BuckGNN(nn.Module):
         self._ran_native128 = False
         if self._runs_native128():
             with torch.no_grad():
-                pred = self._forward_cuda(x, edge_index, batch, width=128)
+                if self.model_name in _NATIVE128_EAGNN_MODELS:
+                    pred = self._forward_cuda_eagnn(x, edge_index, edge_attr, batch, width=128)
+                else:
+                    pred = self._forward_cuda(x, edge_index, batch, width=128)
             self._ran_native128 = True
             return pred.squeeze(), batch
         if self._trains_native128():
@@ -498,9 +521,10 @@ class BuckGNN(nn.Module):
             return _Fill
         return engine.begin_graph_index(edge_index, batch, n)
 
-    def _forward_cuda_eagnn(self, x, edge_index, edge_attr, batch, node_level=False):
-        """EA-GNN / "CustomGNN" path (reference :326-336, :375-387, GraphNetBlock :528-566)."""
-        packs = self._packed()
+    def _forward_cuda_eagnn(self, x, edge_index, edge_attr, batch, node_level=False, width=512):
+        """EA-GNN / "CustomGNN" path (reference :326-336, :375-387, GraphNetBlock :528-566).  `width` 128: a
+        hidden_channels = 128 model on the 128-wide kernels (graph-level head only)."""
+        packs = self._packed() if width == 512 else self._packed128()
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         if not edge_attr.is_cuda:
@@ -509,17 +533,17 @@ class BuckGNN(nn.Module):
         n = x.shape[0]
         # GraphNetBlock aggregates on row = edge_index[0] (:553,561) -> CSR keyed by row 0
         pending = engine.begin_graph_index(edge_index, batch, n, key_row=0)
-        cur = Activation(n, 512, prec, x.device)
+        cur = Activation(n, width, prec, x.device)
         flag = self._new_nonfinite_flag(x.device)
         engine.encoder_forward(x, packs["enc"], packs["enc_w3"], prec, cur, cg, nonfinite=flag)  # :323
         idx = pending.finish()
         ne = idx.n_edges
         ex = engine.edge_extras(idx, prec)
-        e = Activation(max(ne, 1), 512, prec, x.device)
+        e = Activation(max(ne, 1), width, prec, x.device)
         if ne > 0:                                   # edge_encoder on edge_attr in CSR order (:327, :376)
             engine.encoder_forward(edge_attr, packs["edge_enc"], packs["edge_enc_w3"], prec, e, cg,
                                    row_gather=idx.perm[:ne], nonfinite=flag)
-        buf = engine.GNBlockBuffers(n, ne, prec, x.device)
+        buf = engine.GNBlockBuffers(n, ne, prec, x.device, width)
         L = self.num_layers
         for i, w in enumerate(packs["gn"]):
             cur, e_next = engine.gnblock_layer(cur, e, buf, idx, ex, w, skip=(0 < i < L - 1),

@@ -223,10 +223,22 @@ int bg_sage_fused512(const bg_gemm_segment* segments_host, int32_t n_segments, i
  *    out[m, 0:128] = epilogue( sum_s A_s[m, :] . B_s[:, :]^T ),   B_s [128, k_s] (nn.Linear weight layout)
  * Same arguments, operand formats, K rules and epilogue order as bg_gemm512, with 128 for 512 throughout: the
  * epilogue's host vectors are [128], residual / out rows are [M,128] (ld >= 128), pool_block_sums is [ceil(M/32), 128].
- * Not built at this width (BG_ERR_UNSUPPORTED): gathered addends and b_groups > 1. */
+ * Not built at this width (BG_ERR_UNSUPPORTED): gathered addends (see bg_gemm128_gathered) and b_groups > 1. */
 int bg_gemm128(const bg_gemm_segment* segments_host, int32_t n_segments, int64_t m,
                int a_dtype, int b_dtype, const bg_epilogue* epilogue_host,
                void* out, int out_dtype, int64_t ldo, int cta_group, void* stream);
+
+/* bg_gemm128 with gathered pre-activation addends (the edge GEMMs of a hidden_channels = 128 EA-GNN layer, GraphNetBlock
+ * Models/BuckGNN.py:528-566):
+ *    out[m, :] = relu( sum_s A_s[m, :] . B_s^T + bias + gather[0][gather_idx[0][m], :] + gather[1][gather_idx[1][m], :] )
+ * summed in fp32 and rounded once to out_dtype.  gather[k] are DEVICE [*, 128] row-major matrices of out_dtype with
+ * leading dimension gather_ld >= 128 (rows 16-byte aligned), gather_idx[k] DEVICE [M] int32 row indices; gather[1] may
+ * be NULL.  BG_ERR_INVALID for a missing index, gather[1] without gather[0] or a misaligned matrix;
+ * BG_ERR_UNSUPPORTED for gathered addends together with normalize, residual or the pool-fused epilogue (as bg_gemm512).
+ * Without gathered addends the call is bg_gemm128.  Every argument is checked before the first CUDA call. */
+int bg_gemm128_gathered(const bg_gemm_segment* segments_host, int32_t n_segments, int64_t m,
+                        int a_dtype, int b_dtype, const bg_epilogue* epilogue_host,
+                        void* out, int out_dtype, int64_t ldo, int cta_group, void* stream);
 
 /* Aggregates of the hub rows only, compact: hub_out[b, :] = reduce over the neighbours of node big_rows[b] (mean / sum,
  * 16-bit rows).  workspace: bg_aggregate_workspace_bytes(n_big). */
