@@ -41,6 +41,7 @@ EXPORTED_SYMBOLS = (
     "bg_sag_pool_backward", "bg_max_aggregate_backward", "bg_max_bwd_workspace_bytes",
     "bg_bn_batch_stats128", "bg_bn_act_forward128", "bg_sage_backward_rows128", "bg_pool_backward128",
     "bg_max_aggregate_backward128", "bg_wgrad128",
+    "bg_dropout_residual128", "bg_grad_mask128", "bg_segment_expand128", "bg_wgrad128_ld",
 )
 
 
@@ -155,6 +156,10 @@ _SIGNATURES = {
     "bg_max_aggregate_backward128": (C.c_int, [_P, _P, _P, C.c_int, _I64, _P, _P, _P, _I32, _P, _P, _P, _I32, _P, _P, _P,
                                                C.c_size_t, _P]),
     "bg_wgrad128": (C.c_int, [_P, _P, _P, C.c_int, _I64, _I32, _I64, _P, _P, _P, C.c_int, _P]),
+    "bg_dropout_residual128": (C.c_int, [_P, _P, _P, C.c_int, _I64, C.c_float, C.c_uint64, _P]),
+    "bg_grad_mask128": (C.c_int, [_P, _P, _P, _P, C.c_int, _I64, C.c_float, C.c_uint64, _P]),
+    "bg_segment_expand128": (C.c_int, [_P, _P, _I64, C.c_int, _P, C.c_int, _P]),
+    "bg_wgrad128_ld": (C.c_int, [_P, _P, _P, C.c_int, _I64, _I32, _I64, _P, _P, _I64, _P, _I64, C.c_int, _P]),
 }
 
 
@@ -477,16 +482,26 @@ def wgrad128(dz, agg, x, dtype, n_rows, n_chunks, chunk_k, partial, dwl, dwr, ac
                               stream), "bg_wgrad128")
 
 
-def dropout_residual(x, x_prev, y, dtype, n_rows, dropout_p, seed, stream):
-    _check(load().bg_dropout_residual(x, x_prev, y, dtype, n_rows, dropout_p, seed, stream), "bg_dropout_residual")
+def wgrad128_ld(dz, a0, a1, dtype, n_rows, n_chunks, chunk_k, partial, dw0, ld0, dw1, ld1, accumulate, stream):
+    """bg_wgrad128_ld: dw0[o*ld0 + i] (+)= (dz^T a0)[o, i] and, when a1 is given, dw1[o*ld1 + i] (+)= (dz^T a1)[o, i]
+    for [n_rows, 128] rows; partial [n_chunks * 256, 128] f32."""
+    _check(load().bg_wgrad128_ld(dz, a0, a1, dtype, n_rows, n_chunks, chunk_k, partial, dw0, ld0, dw1, ld1,
+                                 int(bool(accumulate)), stream), "bg_wgrad128_ld")
 
 
-def grad_mask(dy, dy2, act, out, dtype, n_rows, dropout_p, seed, stream):
-    _check(load().bg_grad_mask(dy, dy2, act, out, dtype, n_rows, dropout_p, seed, stream), "bg_grad_mask")
+def dropout_residual(x, x_prev, y, dtype, n_rows, dropout_p, seed, stream, width=512):
+    fn = _w("bg_dropout_residual", width)
+    _check(getattr(load(), fn)(x, x_prev, y, dtype, n_rows, dropout_p, seed, stream), fn)
 
 
-def segment_expand(src, rowptr, n_rows, mean, out, dtype, stream):
-    _check(load().bg_segment_expand(src, rowptr, n_rows, int(bool(mean)), out, dtype, stream), "bg_segment_expand")
+def grad_mask(dy, dy2, act, out, dtype, n_rows, dropout_p, seed, stream, width=512):
+    fn = _w("bg_grad_mask", width)
+    _check(getattr(load(), fn)(dy, dy2, act, out, dtype, n_rows, dropout_p, seed, stream), fn)
+
+
+def segment_expand(src, rowptr, n_rows, mean, out, dtype, stream, width=512):
+    fn = _w("bg_segment_expand", width)
+    _check(getattr(load(), fn)(src, rowptr, n_rows, int(bool(mean)), out, dtype, stream), fn)
 
 
 # ----------------------------------------------------------------------------- SAGPooling

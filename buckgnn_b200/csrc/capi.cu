@@ -825,25 +825,27 @@ int bg_wgrad512(const void* dz, int64_t ld_dz, const void* act, int32_t act_cols
   return launch_gemm512<2, float, kAddNone, false>(p, stream);
 }
 
-int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64_t n_rows, int32_t n_chunks, int64_t chunk_k,
-                float* partial, float* dwl, float* dwr, int accumulate, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  // every argument is checked before the first CUDA call
+// The weight-gradient GEMM of both 128-wide entry points: per node chunk one M = 256 pair tile [a0^T ; a1^T]·dz into
+// partial.  `a1` null (a single product): the rank-1 CTA re-reads a0 (its rows arrive from L2 with rank 0's) and that
+// half of the tile is discarded by the reduction.  Checks every argument it takes before any CUDA call; the callers
+// check theirs before calling it.
+static int wgrad128_gemm(const char* fn, const void* dz, const void* a0, const void* a1, int dtype, int64_t n_rows,
+                         int32_t n_chunks, int64_t chunk_k, float* partial, cudaStream_t stream) {
   const int fmt = umma_format_of(dtype);
-  if (fmt < 0) return fail(BG_ERR_INVALID, "bg_wgrad128: bad dtype");
+  if (fmt < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");
   const int esz = fmt == 2 ? 4 : 2;
   const int kblk = kStageKBytes / esz;                     // nodes per pipeline stage: 64 (16-bit) / 32 (tf32)
   if (n_rows <= 0 || n_chunks <= 0 || chunk_k <= 0 || chunk_k % kblk != 0 || (int64_t)n_chunks * chunk_k < n_rows ||
       (int64_t)n_chunks * chunk_k >= 0x7fffffffLL)
-    return fail(BG_ERR_INVALID, "bg_wgrad128: chunk_k must be a multiple of 64 (16-bit) / 32 (tf32) and n_chunks*chunk_k >= n_rows");
-  if (!dz || !agg || !x || !partial || !dwl || !dwr || !aligned16(dz) || !aligned16(agg) || !aligned16(x) || !aligned16(partial))
-    return fail(BG_ERR_INVALID, "bg_wgrad128: null or misaligned pointer");
+    return fail_in(BG_ERR_INVALID, fn, "chunk_k must be a multiple of 64 (16-bit) / 32 (tf32) and n_chunks*chunk_k >= n_rows");
+  if (!dz || !a0 || !partial || !aligned16(dz) || !aligned16(a0) || (a1 && !aligned16(a1)) || !aligned16(partial))
+    return fail_in(BG_ERR_INVALID, fn, "null or misaligned pointer");
   Gemm128Params p;
   memset(&p, 0, sizeof(p));
-  int rc = make_mn_operand_map(&p.seg[0].a, agg, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
-  if (rc == BG_OK) rc = make_mn_operand_map(&p.seg[1].a, x, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
+  int rc = make_mn_operand_map(&p.seg[0].a, a0, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
+  if (rc == BG_OK) rc = make_mn_operand_map(&p.seg[1].a, a1 ? a1 : a0, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
   if (rc == BG_OK) rc = make_mn_operand_map(&p.seg[0].b, dz, n_rows, kW128, kW128, (uint32_t)fmt, kblk);
-  if (rc != BG_OK) return fail(rc, "bg_wgrad128: cuTensorMapEncodeTiled failed");
+  if (rc != BG_OK) return fail_in(rc, fn, "cuTensorMapEncodeTiled failed");
   p.n_seg = 1;                                             // the MMA warp walks segment 0's K blocks; rank 1 reads seg[1].a
   p.kblocks[0] = (int32_t)(chunk_k / kblk);
   p.k_elems_per_block = kblk;
@@ -853,9 +855,29 @@ int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64
   p.m = (int64_t)n_chunks * 2 * kW128;
   for (int i = 0; i < kW128; ++i) { p.bias[i] = 0.f; p.scale[i] = 1.f; p.shift[i] = 0.f; }
   p.out = partial; p.ldo = kW128;
-  rc = launch_gemm128<float, false, false, true>(p, stream);
+  return launch_gemm128<float, false, false, true>(p, stream);
+}
+
+int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64_t n_rows, int32_t n_chunks, int64_t chunk_k,
+                float* partial, float* dwl, float* dwr, int accumulate, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (!agg || !x || !dwl || !dwr) return fail(BG_ERR_INVALID, "bg_wgrad128: null or misaligned pointer");
+  const int rc = wgrad128_gemm("bg_wgrad128", dz, agg, x, dtype, n_rows, n_chunks, chunk_k, partial, stream);
   if (rc != BG_OK) return rc;
   k_reduce_wgrad128<<<grid_for(2 * kW128 * kW128, 256, sm_count() * 4), 256, 0, stream>>>(partial, n_chunks, dwl, dwr, accumulate);
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+
+int bg_wgrad128_ld(const void* dz, const void* a0, const void* a1, int dtype, int64_t n_rows, int32_t n_chunks, int64_t chunk_k,
+                   float* partial, float* dw0, int64_t ld0, float* dw1, int64_t ld1, int accumulate, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (!dw0 || ld0 < kW128 || (a1 && (!dw1 || ld1 < kW128)) || (!a1 && dw1))
+    return fail(BG_ERR_INVALID, "bg_wgrad128_ld: dw0 (and dw1 exactly when a1 is given) non-null with ld >= 128");
+  const int rc = wgrad128_gemm("bg_wgrad128_ld", dz, a0, a1, dtype, n_rows, n_chunks, chunk_k, partial, stream);
+  if (rc != BG_OK) return rc;
+  k_reduce_wgrad128_ld<<<grid_for((a1 ? 2 : 1) * kW128 * kW128, 256, sm_count() * 4), 256, 0, stream>>>(
+      partial, n_chunks, dw0, ld0, a1 ? dw1 : nullptr, ld1, accumulate);
   BG_LAUNCH_OK();
   return BG_OK;
 }
@@ -1486,42 +1508,81 @@ int bg_sgemm(const void* a, int a_dtype, int64_t sam, int64_t sak, const void* b
   return BG_OK;
 }
 
-int bg_dropout_residual(const void* x, const void* x_prev, void* y, int dtype, int64_t N, float dropout_p, uint64_t seed, void* stream_) {
+extern "C++" {
+template <int kW>
+static int dropout_residual_impl(const char* fn, const void* x, const void* x_prev, void* y, int dtype, int64_t N,
+                                 float dropout_p, uint64_t seed, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail(BG_ERR_INVALID, "bg_dropout_residual: bad size / dropout_p");
+  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail_in(BG_ERR_INVALID, fn, "bad size / dropout_p");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
   if (N == 0) return BG_OK;
-  if (!x || !y || !aligned16(x) || !aligned16(y) || (x_prev && !aligned16(x_prev))) return fail(BG_ERR_INVALID, "bg_dropout_residual: bad pointer");
+  if (!x || !y || !aligned16(x) || !aligned16(y) || (x_prev && !aligned16(x_prev))) return fail_in(BG_ERR_INVALID, fn, "bad pointer");
   const DropArgs d = drop_args(dropout_p, seed);
   const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_dropout_residual<T><<<grid, 256, 0, stream>>>(static_cast<const T*>(x), static_cast<const T*>(x_prev), static_cast<T*>(y), N, d)))
+  BG_BY_DTYPE(dtype, (k_dropout_residual<T, kW><<<grid, 256, 0, stream>>>(static_cast<const T*>(x), static_cast<const T*>(x_prev),
+                                                                          static_cast<T*>(y), N, d)))
   BG_LAUNCH_OK();
   return BG_OK;
+}
+
+template <int kW>
+static int grad_mask_impl(const char* fn, const void* dy, const void* dy2, const void* act, void* out, int dtype, int64_t N,
+                          float dropout_p, uint64_t seed, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail_in(BG_ERR_INVALID, fn, "bad size / dropout_p");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  if (N == 0) return BG_OK;
+  if (!dy || !out || !aligned16(dy) || !aligned16(out) || (dy2 && !aligned16(dy2)) || (act && !aligned16(act)))
+    return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  const DropArgs d = drop_args(dropout_p, seed);
+  const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
+  BG_BY_DTYPE(dtype, (k_grad_mask<T, kW><<<grid, 256, 0, stream>>>(static_cast<const T*>(dy), static_cast<const T*>(dy2),
+                                                                   static_cast<const T*>(act), static_cast<T*>(out), N, d)))
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+
+template <int kW>
+static int segment_expand_impl(const char* fn, const void* src, const int32_t* rowptr, int64_t n_rows, int mean, void* out,
+                               int dtype, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (n_rows < 0) return fail_in(BG_ERR_INVALID, fn, "bad size");
+  if (kW != kHidden && umma_format_of(dtype) < 0) return fail_in(BG_ERR_INVALID, fn, "bad dtype");   // (512: BG_BY_DTYPE)
+  if (n_rows == 0) return BG_OK;
+  if (!src || !rowptr || !out || !aligned16(src) || !aligned16(out)) return fail_in(BG_ERR_INVALID, fn, "bad pointer");
+  const unsigned grid = grid_for(n_rows * 32, 256, sm_count() * 8);
+  BG_BY_DTYPE(dtype, (k_segment_expand<T, kW><<<grid, 256, 0, stream>>>(static_cast<const T*>(src), rowptr, n_rows, mean,
+                                                                        static_cast<T*>(out))))
+  BG_LAUNCH_OK();
+  return BG_OK;
+}
+}  // extern "C++"
+
+int bg_dropout_residual(const void* x, const void* x_prev, void* y, int dtype, int64_t N, float dropout_p, uint64_t seed, void* stream_) {
+  return dropout_residual_impl<kHidden>("bg_dropout_residual", x, x_prev, y, dtype, N, dropout_p, seed, stream_);
+}
+
+int bg_dropout_residual128(const void* x, const void* x_prev, void* y, int dtype, int64_t N, float dropout_p, uint64_t seed,
+                           void* stream_) {
+  return dropout_residual_impl<kW128>("bg_dropout_residual128", x, x_prev, y, dtype, N, dropout_p, seed, stream_);
 }
 
 int bg_grad_mask(const void* dy, const void* dy2, const void* act, void* out, int dtype, int64_t N, float dropout_p,
                  uint64_t seed, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || !(dropout_p >= 0.f && dropout_p < 1.f)) return fail(BG_ERR_INVALID, "bg_grad_mask: bad size / dropout_p");
-  if (N == 0) return BG_OK;
-  if (!dy || !out || !aligned16(dy) || !aligned16(out) || (dy2 && !aligned16(dy2)) || (act && !aligned16(act)))
-    return fail(BG_ERR_INVALID, "bg_grad_mask: bad pointer");
-  const DropArgs d = drop_args(dropout_p, seed);
-  const unsigned grid = grid_for(N * 32, 256, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_grad_mask<T><<<grid, 256, 0, stream>>>(static_cast<const T*>(dy), static_cast<const T*>(dy2), static_cast<const T*>(act),
-                                                               static_cast<T*>(out), N, d)))
-  BG_LAUNCH_OK();
-  return BG_OK;
+  return grad_mask_impl<kHidden>("bg_grad_mask", dy, dy2, act, out, dtype, N, dropout_p, seed, stream_);
+}
+
+int bg_grad_mask128(const void* dy, const void* dy2, const void* act, void* out, int dtype, int64_t N, float dropout_p,
+                    uint64_t seed, void* stream_) {
+  return grad_mask_impl<kW128>("bg_grad_mask128", dy, dy2, act, out, dtype, N, dropout_p, seed, stream_);
 }
 
 int bg_segment_expand(const void* src, const int32_t* rowptr, int64_t n_rows, int mean, void* out, int dtype, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (n_rows < 0) return fail(BG_ERR_INVALID, "bg_segment_expand: bad size");
-  if (n_rows == 0) return BG_OK;
-  if (!src || !rowptr || !out || !aligned16(src) || !aligned16(out)) return fail(BG_ERR_INVALID, "bg_segment_expand: bad pointer");
-  const unsigned grid = grid_for(n_rows * 32, 256, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_segment_expand<T><<<grid, 256, 0, stream>>>(static_cast<const T*>(src), rowptr, n_rows, mean, static_cast<T*>(out))))
-  BG_LAUNCH_OK();
-  return BG_OK;
+  return segment_expand_impl<kHidden>("bg_segment_expand", src, rowptr, n_rows, mean, out, dtype, stream_);
+}
+
+int bg_segment_expand128(const void* src, const int32_t* rowptr, int64_t n_rows, int mean, void* out, int dtype, void* stream_) {
+  return segment_expand_impl<kW128>("bg_segment_expand128", src, rowptr, n_rows, mean, out, dtype, stream_);
 }
 
 int bg_collate_ptr(const int64_t* sel, int64_t G, const int64_t* node_ptr, const int64_t* edge_ptr,

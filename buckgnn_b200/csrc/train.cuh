@@ -380,6 +380,20 @@ k_reduce_wgrad128(const float* __restrict__ partial, int n_chunks, float* __rest
     *out = accumulate ? *out + v : v;
   }
 }
+// bg_wgrad128_ld: the same sum into column slices of wider weights, dw_k[o * ld_k + i] (+)= sum_s partial[s][128 k + i][o];
+// dw1 null: the second half of every pair tile is discarded (a single product).
+__global__ void __launch_bounds__(256)
+k_reduce_wgrad128_ld(const float* __restrict__ partial, int n_chunks, float* __restrict__ dw0, int64_t ld0,
+                     float* __restrict__ dw1, int64_t ld1, int accumulate) {
+  const int64_t n = (dw1 ? 2 : 1) * 128 * 128, stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const int which = (int)(t >> 14), i = (int)(t >> 7) & 127, o = (int)t & 127;
+    float v = 0.f;
+    for (int s = 0; s < n_chunks; ++s) v += partial[((size_t)s * 256 + which * 128 + i) * 128 + o];
+    float* out = which ? dw1 + (size_t)o * ld1 + i : dw0 + (size_t)o * ld0 + i;
+    *out = accumulate ? *out + v : v;
+  }
+}
 
 // ------------------------------------------------------------------ generic loads by run-time dtype
 BG_DEVINL float load_as_float(const void* p, int dtype, size_t i) {
@@ -536,65 +550,72 @@ __global__ void k_sgemm_epilogue(const SgemmEpilogue p) {
 
 // ------------------------------------------------------------------ elementwise pieces of the EA-GNN training step
 // (Models/BuckGNN.py:375-387 wrapper and GraphNetBlock :552-566 in train mode)
+// (templates on the row width kW like the SAGE row kernels above: 128 for a hidden_channels = 128 model, bg_*128)
 // y = dropout(x + x_prev)   -- the wrapper's skip + Dropout on node and edge tensors (no activation in between)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_dropout_residual(const T* __restrict__ x, const T* __restrict__ x_prev, T* __restrict__ y, int64_t N, const DropArgs drop) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += n_warps) {
-    float v[16];
-    row_load<T>(x + (size_t)r * kHidden, lane, v);
+    float v[kPer];
+    IO::load(x + (size_t)r * kW, lane, v);
     if (x_prev) {
-      float t[16];
-      row_load<T>(x_prev + (size_t)r * kHidden, lane, t);
+      float t[kPer];
+      IO::load(x_prev + (size_t)r * kW, lane, t);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] += t[i];
+      for (int i = 0; i < kPer; ++i) v[i] += t[i];
     }
     if (drop.thr) {
 #pragma unroll
-      for (int i = 0; i < 16; ++i)
-        v[i] = dropout_keep(drop.seed, r, RowFrag<T>::col_of(lane, i), drop.thr) ? v[i] * drop.inv_keep : 0.f;
+      for (int i = 0; i < kPer; ++i)
+        v[i] = dropout_keep(drop.seed, r, IO::col_of(lane, i), drop.thr) ? v[i] * drop.inv_keep : 0.f;
     }
-    RowFrag<T>::store(y + (size_t)r * kHidden, lane, v);
+    IO::store(y + (size_t)r * kW, lane, v);
   }
 }
 // out = dropout'(dy + dy2) [act > 0]   (either part optional: thr = 0 -> no dropout, act = null -> no ReLU mask)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_grad_mask(const T* __restrict__ dy, const T* __restrict__ dy2, const T* __restrict__ act, T* __restrict__ out, int64_t N,
             const DropArgs drop) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < N; r += n_warps) {
-    float g[16];
-    load_upstream<T>(dy, dy2, r, lane, drop, g);
+    float g[kPer];
+    load_upstream<T, kW>(dy, dy2, r, lane, drop, g);
     if (act) {
-      float a[16];
-      row_load<T>(act + (size_t)r * kHidden, lane, a);
+      float a[kPer];
+      IO::load(act + (size_t)r * kW, lane, a);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) g[i] = a[i] > 0.f ? g[i] : 0.f;
+      for (int i = 0; i < kPer; ++i) g[i] = a[i] > 0.f ? g[i] : 0.f;
     }
-    RowFrag<T>::store(out + (size_t)r * kHidden, lane, g);
+    IO::store(out + (size_t)r * kW, lane, g);
   }
 }
 // scatter_mean backward: every CSR slot of row r receives src[r] / max(count_r, 1)  (count = 1 without `mean`)
-template <typename T>
+template <typename T, int kW = kHidden>
 __global__ void __launch_bounds__(256)
 k_segment_expand(const T* __restrict__ src, const int32_t* __restrict__ rowptr, int64_t n_rows, int mean, T* __restrict__ out) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n_rows; r += n_warps) {
     const int32_t b = rowptr[r], e = rowptr[r + 1];
     if (e == b) continue;
-    float v[16];
-    row_load<T>(src + (size_t)r * kHidden, lane, v);
+    float v[kPer];
+    IO::load(src + (size_t)r * kW, lane, v);
     if (mean) {
       const float w = 1.f / (float)(e - b);
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] *= w;
+      for (int i = 0; i < kPer; ++i) v[i] *= w;
     }
-    for (int32_t s = b; s < e; ++s) RowFrag<T>::store(out + (size_t)s * kHidden, lane, v);
+    for (int32_t s = b; s < e; ++s) IO::store(out + (size_t)s * kW, lane, v);
   }
 }
 

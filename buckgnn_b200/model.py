@@ -21,7 +21,9 @@ A hidden_channels = 128 GraphSAGE model (the reference's default width) evaluate
 trains on them too when `model.native128_train` is set (a module attribute, default from BUCKGNN_NATIVE128_TRAIN=1 in
 the environment); otherwise, and for what the 128-wide step does not cover, training runs as the zero-padded 512-wide
 twin (narrow.py).  A 128-wide EA_GNN / EA_GNN_Shared model evaluates on the 128-wide kernels when
-`model.native128_eagnn` is set (default from BUCKGNN_NATIVE128_EAGNN=1); it always trains as the twin.
+`model.native128_eagnn` is set (default from BUCKGNN_NATIVE128_EAGNN=1), and trains on them when
+`model.native128_eagnn_train` is set (default from BUCKGNN_NATIVE128_EAGNN_TRAIN=1; train_eagnn.py at width 128);
+otherwise it trains as the twin.
 
 Extra, non-reference keywords: `train_precision` in {"tf32", "bf16", "fp16"} (storage of the training
 step's activations and activation gradients; default tf32 = fp32 storage), and `precision` in {"auto", "fp16", "bf16", "tf32", "fp32"}
@@ -58,6 +60,10 @@ NATIVE128_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_TRAIN", "0") not in 
 # `model.native128_eagnn = True`.
 _NATIVE128_EAGNN_MODELS = ("EA_GNN", "EA_GNN_Shared")
 NATIVE128_EAGNN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN", "0") not in ("", "0")
+# train-mode forwards of the same EA-GNN models at hidden_channels == 128 on the 128-wide kernels (train_eagnn.py at
+# width 128) instead of the twin.  Opt-in: BUCKGNN_NATIVE128_EAGNN_TRAIN=1 in the environment, or
+# `model.native128_eagnn_train = True`.
+NATIVE128_EAGNN_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN_TRAIN", "0") not in ("", "0")
 
 
 class SAGEConv(nn.Module):
@@ -167,6 +173,7 @@ class BuckGNN(nn.Module):
         self.fuse_aggregate = engine.FUSE_AGGREGATE_DEFAULT    # the aggregate operand gathered inside the update GEMM (opt-in)
         self.native128_train = NATIVE128_TRAIN_DEFAULT         # hidden_channels 128: train on the 128-wide kernels (opt-in)
         self.native128_eagnn = NATIVE128_EAGNN_DEFAULT         # hidden_channels 128: EA-GNN eval on the 128-wide kernels (opt-in)
+        self.native128_eagnn_train = NATIVE128_EAGNN_TRAIN_DEFAULT   # hidden_channels 128: EA-GNN training on them (opt-in)
         self.output_dim = output_dim = _output_dim(prediction_type, use_z_coord, use_rotations)
         h = hidden_channels
         cat_dec = pooling_layer == "supernode_with_pooling" and prediction_type == "buckling"
@@ -390,6 +397,14 @@ class BuckGNN(nn.Module):
                 and self.model_name in _NATIVE128_MODELS and self.prediction_type == "buckling"
                 and self.pooling_layer in _POOLINGS)
 
+    def _trains_native128_eagnn(self) -> bool:
+        """With `native128_eagnn_train` on, train-mode forwards of EA_GNN / EA_GNN_Shared at hidden_channels == 128 with a
+        graph-level head run the EA-GNN training step at width 128 on the module's own parameters (train_eagnn.py);
+        `native128_train` and `native128_eagnn` leave them on the twin."""
+        return (self.hidden_channels == 128 and self.training and bool(self.native128_eagnn_train)
+                and self.model_name in _NATIVE128_EAGNN_MODELS and self.prediction_type == "buckling"
+                and self.pooling_layer in _POOLINGS)
+
     def forward(self, x, edge_index, edge_attr, batch=None, mask=None):
         self._check_supported(x)
         self._ran_native128 = False
@@ -401,7 +416,7 @@ class BuckGNN(nn.Module):
                     pred = self._forward_cuda(x, edge_index, batch, width=128)
             self._ran_native128 = True
             return pred.squeeze(), batch
-        if self._trains_native128():
+        if self._trains_native128() or self._trains_native128_eagnn():
             from . import train
             pred = train.forward_train(self, x, edge_index, batch, edge_attr=edge_attr)
             self._pack_sig = None                # BatchNorm statistics changed: the next native eval forward repacks
@@ -475,10 +490,11 @@ class BuckGNN(nn.Module):
         """Multi-GPU training (BASELINE.json configs[3]): all-reduce (mean) the gradients of this model's trainable
         parameters over `group`, bucketed per layer and overlapped with the backward pass (dist.GradSync).  Call once
         after `.to(device)`, on every rank; `loss.backward()` then leaves the REDUCED gradients in `.grad`."""
-        if self.hidden_channels != 512 and not (self.hidden_channels == 128 and self.native128_train):
+        native128 = self.native128_train or (self.native128_eagnn_train and self.model_name in _NATIVE128_EAGNN_MODELS)
+        if self.hidden_channels != 512 and not (self.hidden_channels == 128 and native128):
             raise NotImplementedError("buckgnn_b200: overlapped gradient sync is built for hidden_channels=512, and for "
-                                      "128 with native128_train on; use dist.allreduce_gradients(model.parameters()) "
-                                      "after backward() instead")
+                                      "128 with native128_train (EA_GNN / EA_GNN_Shared: native128_eagnn_train) on; use "
+                                      "dist.allreduce_gradients(model.parameters()) after backward() instead")
         from . import train
         from .dist import GradSync
         self._grad_sync = GradSync(train.trainable_parameters(self), next(self.parameters()).device, group)

@@ -499,6 +499,24 @@ int bg_max_aggregate_backward128(const void* x, const void* agg, const void* dag
 int bg_wgrad128(const void* dz, const void* agg, const void* x, int dtype, int64_t n_rows, int32_t n_chunks,
                 int64_t chunk_k, float* partial, float* dwl, float* dwr, int accumulate, void* stream);
 
+/* The EA-GNN training step at width 128 (BuckGNN.native128_eagnn_train), on [N, 128] rows:
+ *   bg_dropout_residual128, bg_grad_mask128, bg_segment_expand128: the arguments and rules of bg_dropout_residual,
+ *     bg_grad_mask and bg_segment_expand with 128 for 512.  The dropout element index stays r*512 + c, so the mask is
+ *     the first 128 columns of the 512-wide one (bg_dropout_mask).
+ *   bg_wgrad128_ld: the weight gradients of EA-GNN's concatenated Linears, written in place into column slices,
+ *       dw0[o * ld0 + i] (+)= sum_n dz[n, o] a0[n, i],   dw1[o * ld1 + i] (+)= sum_n dz[n, o] a1[n, i]    (o, i < 128)
+ *     e.g. dw0 = dW + 128 with ld0 = 384 for the middle slice of a [128, 384] weight.  a1 is nullable (a single
+ *     product; dw1 must then be null too), ld0 / ld1 >= 128.  dz, a0, a1, partial, n_chunks, chunk_k and accumulate as
+ *     bg_wgrad128 (a single product still fills the 256 x 128 pair tile of partial: its second half is discarded). */
+int bg_dropout_residual128(const void* x, const void* x_prev, void* y, int dtype, int64_t n_rows, float dropout_p,
+                           uint64_t seed, void* stream);
+int bg_grad_mask128(const void* dy, const void* dy2, const void* act, void* out, int dtype, int64_t n_rows, float dropout_p,
+                    uint64_t seed, void* stream);
+int bg_segment_expand128(const void* src, const int32_t* rowptr, int64_t n_rows, int mean, void* out, int dtype, void* stream);
+int bg_wgrad128_ld(const void* dz, const void* a0, const void* a1, int dtype, int64_t n_rows, int32_t n_chunks,
+                   int64_t chunk_k, float* partial, float* dw0, int64_t ld0, float* dw1, int64_t ld1, int accumulate,
+                   void* stream);
+
 /* Device-side collate (SURVEY.md section 8 row f1): PyG `DataLoader` / `Batch.from_data_list` for a dataset kept in HBM in
  * concatenated form -- x_all [sum n, F], ei_all [2, E_all] with node ids LOCAL to their graph (as
  * GraphCreate.py:417-432 emits them), ea_all [E_all, Fe], y_all [G_all], node_ptr / edge_ptr [G_all+1] int64.
