@@ -585,6 +585,7 @@ static int gemm512_impl(const bg_gemm_segment* segs, int32_t n_seg, int64_t m, i
       memcpy(p.shift, epi->bn_shift_host, sizeof(float) * kHidden);
     }
     p.normalize = epi->normalize; p.relu = epi->relu;
+    if (!epi->gather[0] && epi->gather[1]) return fail(BG_ERR_INVALID, "bg_gemm512: gather[1] without gather[0]");
     for (int k = 0; k < 2; ++k) {
       if (!epi->gather[k]) break;
       if (!epi->gather_idx[k] || !aligned16(epi->gather[k]) || (epi->gather_ld * osz) % 16 != 0 || epi->gather_ld < kHidden)

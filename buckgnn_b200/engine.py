@@ -378,9 +378,13 @@ class FoldedLayer0Pack:
     bias_all_gated: Optional[torch.Tensor] = None   # HOST f32 [512]: bias + W_l b3, valid when every row's gate is 1
 
 
-def pack_folded_layer0(enc_last: torch.nn.Linear, conv, bn, aggr: str, precision: str, width: int = 512) -> FoldedLayer0Pack:
+def pack_folded_layer0(enc_last: torch.nn.Linear, conv, bn, aggr: str, precision: str,
+                       width: int = 512) -> Optional[FoldedLayer0Pack]:
     """`width`: the layer's output width (512, or 128 for a hidden_channels = 128 model, whose encoder's last Linear
-    reads the 64-wide hidden layer stored 128 wide: W3 is zero-padded to 128 columns)."""
+    reads the 64-wide hidden layer stored 128 wide: W3 is zero-padded to 128 columns).
+    None when a folded weight does not fit its operand format (fp16 with sum / add aggregation: the degree digits'
+    gate columns carry W_l b3 x 65536, inf once |W_l b3| > ~1, and the MMA would make every row 0 x inf = NaN); the
+    caller then runs layer 0 unfolded."""
     dev = conv.lin_l.weight.device
     d64 = lambda t: t.detach().to(torch.float64).cpu()
     W3, b3 = d64(enc_last.weight), d64(enc_last.bias)
@@ -393,8 +397,11 @@ def pack_folded_layer0(enc_last: torch.nn.Linear, conv, bn, aggr: str, precision
         # (thousands) is not exact in 8 / 11 significant bits, its digits are
         gate[:, 1] = gate[:, 0] * 256.0
         gate[:, 2] = gate[:, 0] * 65536.0
+    wl3, wr3, wgate = lp(Wl @ W3), lp(Wr @ W3), lp(gate)
+    if not all(bool(torch.isfinite(t).all()) for pk in (wl3, wr3, wgate) for t in pk.parts):
+        return None
     scale, shift = fold_batchnorm(bn) if bn is not None else (None, None)
-    return FoldedLayer0Pack(lp(Wl @ W3), lp(Wr @ W3), lp(gate), (Wr @ b3 + bl).to(torch.float32).contiguous(),
+    return FoldedLayer0Pack(wl3, wr3, wgate, (Wr @ b3 + bl).to(torch.float32).contiguous(),
                             scale, shift, aggr in ("sum", "add"),
                             bias_all_gated=(Wr @ b3 + bl + Wl @ b3).to(torch.float32).contiguous())
 

@@ -283,7 +283,7 @@ class BuckGNN(nn.Module):
             sl = []                                   # num_layers == 1: the pooling runs on the encoder output itself
         if self.fold_encoder and sl and sl[0][0].aggr != "max":
             conv0, bn0 = sl[0]
-            packs["layer0_folded"] = engine.pack_folded_layer0(enc[4], conv0, bn0, conv0.aggr, prec)
+            packs["layer0_folded"] = engine.pack_folded_layer0(enc[4], conv0, bn0, conv0.aggr, prec)  # None: unfolded
         if self.model_name in ("EA_GNN", "EA_GNN_Shared"):
             ee = self.edge_encoder
             packs["edge_enc"] = {"w1": f32(ee[0].weight), "b1": f32(ee[0].bias), "w2": f32(ee[2].weight),
@@ -345,11 +345,7 @@ class BuckGNN(nn.Module):
         sl = self._sage_layers()
         if self.fold_encoder and sl and sl[0][0].aggr != "max":
             conv0, bn0 = sl[0]
-            folded = engine.pack_folded_layer0(enc[2], conv0, bn0, conv0.aggr, prec, width=128)
-            # a folded weight its storage format cannot hold (fp16, sum / add: the degree digits' gate columns carry
-            # W_l b3 x 65536) would turn every prediction into NaN: run layer 0 unfolded instead
-            if not all(bool(torch.isfinite(t).all()) for pk in (folded.wl3, folded.wr3, folded.wgate) for t in pk.parts):
-                folded = None
+            folded = engine.pack_folded_layer0(enc[2], conv0, bn0, conv0.aggr, prec, width=128)   # None: unfolded
         packs["layer0_folded"] = folded
         if self.model_name in _NATIVE128_EAGNN_MODELS:      # the edge encoder by the same [I; 0] embedding
             ee = self.edge_encoder

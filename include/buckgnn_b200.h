@@ -154,7 +154,11 @@ int bg_sage_aggregate(const void* x, void* out, int dtype, int64_t n_nodes, int3
  * The gathered addends serve the EA-GNN block (Models/BuckGNN.py:556-560), where
  * cat[x[row], x[col], e] W^T is evaluated as (x W_a^T)[row] + (x W_b^T)[col] + e W_c^T: the two
  * node-level products are gathered per edge inside the epilogue of the edge-level GEMM.
- * normalize cannot be combined with gathered addends, nor gathered addends with residual.
+ * normalize cannot be combined with gathered addends, nor gathered addends with residual; gather[1] needs gather[0].
+ * Rounding of the gathered addends with a 16-bit out_dtype (unlike bg_gemm128_gathered, which rounds once):
+ * acc + bias is rounded to out_dtype first; two gathered rows are summed in out_dtype (one rounding) before they
+ * join; without BatchNorm vectors the join is itself an out_dtype add (rounded again), with them it is an fp32 add
+ * and the result is rounded once more at the store.  An fp32 out_dtype adds everything in fp32.
  * Operand formats: a_dtype == b_dtype in {BG_BF16, BG_F16} (tcgen05 kind::f16, k_s % 64 == 0;
  * the hardware rejects bf16 x fp16 mixes) or both BG_F32 (read as
  * tf32, kind::tf32; k_s % 32 == 0 -- with hi/lo split operands from bg_split_tf32 this

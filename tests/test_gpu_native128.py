@@ -7,109 +7,21 @@ the oracle and against the twin, the routing, the fold guard, the finite check a
 import pytest
 import torch
 
-from buckgnn_b200 import capi, engine
+from buckgnn_b200 import capi
 from buckgnn_b200.model import BuckGNN
 from buckgnn_b200.narrow import WideTwin
 from buckgnn_b200.synth import collate, config_batch, make_batch, make_plate_graph
 from oracle.buckgnn_oracle import OracleBuckGNN, randomize_bn_stats
+from tests.gemm_harness import Spec, run_case
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-CANARY = 1234.0
 
 
 # ----------------------------------------------------------------------------- bg_gemm128 against fp64 torch
-def _as_operand(t, prec):
-    """the values the tensor core multiplies: 16-bit rounding, tf32 truncation (tcgen05 kind::tf32), or fp32 itself
-    (3xTF32 carries ~fp32 precision)"""
-    if prec == "fp16":
-        return t.half().double()
-    if prec == "bf16":
-        return t.bfloat16().double()
-    if prec == "tf32":
-        return (t.float().contiguous().view(torch.int32) & ~0x1FFF).view(torch.float32).double()
-    return t.double()
-
-
-def _gemm_case(prec, m, ks, *, normalize=False, bn=False, relu=False, residual=False, pool=False, inv_norm=False,
-               zero_rows=0, seed=0):
-    g = torch.Generator().manual_seed(seed * 1000 + m + sum(ks))
-    pad = 37
-    acts, packs, a_host, w_host = [], [], [], []
-    # 3xTF32 with three K segments: the third operand is tf32-exact (like the folded layer 0's degree digits), so its
-    # lo part is 0 and two of its three products suffice -- 3 + 3 + 2 = BG_MAX_GEMM_SEGMENTS
-    exact_last = prec == "fp32" and len(ks) == 3
-    for i, k in enumerate(ks):
-        a = torch.randn(m, k, generator=g)
-        a[:zero_rows] = 0
-        if exact_last and i == 2:
-            a = _as_operand(a, "tf32").float()
-        w = torch.randn(128, k, generator=g) / k ** 0.5
-        act = engine.Activation(m, k, prec, DEV)
-        act.data.copy_(a.to(act.dtype))
-        act.refresh_split()
-        acts.append(act)
-        packs.append(engine.pack_linear(w.to(DEV), prec))
-        a_host.append(a)
-        w_host.append(w)
-    bias = torch.zeros(128) if zero_rows else torch.randn(128, generator=g) * 0.1
-    scale = torch.rand(128, generator=g) + 0.5
-    shift = torch.randn(128, generator=g) * 0.1
-    out = engine.Activation(m + pad, 128, prec, DEV)
-    out.data.fill_(CANARY)
-    epi = dict(bias=bias.data_ptr(), normalize=normalize, relu=relu)
-    if bn:
-        epi.update(bn_scale=scale.data_ptr(), bn_shift=shift.data_ptr())
-    res = None
-    if residual:
-        res = torch.randn(m, 128, generator=g).to(out.dtype).to(DEV)
-        epi.update(residual=res.data_ptr(), ldr=128)
-    inv = torch.full((m,), -1.0, device=DEV) if inv_norm else None
-    if inv is not None:
-        epi.update(inv_norm_out=inv.data_ptr())
-    nb = (m + 31) // 32
-    keep = sums = None
-    if pool:
-        keep = (torch.rand(nb, generator=g) < 0.3).to(torch.uint8).to(DEV)
-        sums = torch.full((nb, 128), CANARY, device=DEV)
-        epi.update(pool_block_sums=sums.data_ptr(), pool_block_keep=keep.data_ptr())
-    segs = []
-    for i, (act, pk) in enumerate(zip(acts, packs)):
-        segs += engine._segments(act, pk)[:2] if exact_last and i == 2 else engine._segments(act, pk)
-    engine.gemm(segs, m, prec, out, **epi)
-    torch.cuda.synchronize()
-
-    acc = sum(_as_operand(a, prec) @ _as_operand(w, prec).T for a, w in zip(a_host, w_host)) + bias.double()
-    if normalize:
-        acc = acc / acc.norm(dim=1, keepdim=True).clamp_min(1e-12)
-    if bn:
-        acc = acc * scale.double() + shift.double()
-    if relu:
-        acc = acc.clamp_min(0)
-    if residual:
-        acc = acc + res.cpu().double()
-    got = out.data.cpu().double()
-    tol = {"fp16": 2e-3, "bf16": 1.6e-2, "tf32": 1e-5, "fp32": 1e-5}[prec]
-    scale_ref = acc.abs().max().item() + 1e-30
-    canary = torch.tensor(CANARY).to(out.dtype).double()
-    assert (got[m:] == canary).all(), "rows >= M were written"
-    rows = torch.ones(m, dtype=torch.bool)
-    if pool:
-        rows = keep.cpu().bool().repeat_interleave(32)[:m]
-        assert (got[:m][~rows] == canary).all(), "rows of a block that is not flagged were stored"
-        ref_sums = torch.zeros(nb * 32, 128, dtype=torch.float64)
-        ref_sums[:m] = acc.to(out.dtype).double()
-        ref_sums = ref_sums.view(nb, 32, 128).sum(1)
-        err = (sums.cpu().double() - ref_sums).abs().max().item()
-        assert err <= 32 * tol * scale_ref, f"pool sums: {err}"
-    err = (got[:m][rows] - acc[rows]).abs().max().item() / scale_ref if rows.any() else 0.0
-    assert err < tol, f"{prec} m={m} ks={ks}: max err {err:.3e} (rel. to max |out|)"
-    if zero_rows:
-        assert (got[:zero_rows] == 0).all()
-    if inv_norm:                                            # all-zero rows: 1 / eps
-        ref_inv = 1.0 / (sum(_as_operand(a, prec) @ _as_operand(w, prec).T for a, w in zip(a_host, w_host))
-                         + bias.double()).norm(dim=1).clamp_min(1e-12)
-        assert torch.allclose(inv.cpu().double(), ref_inv, rtol=10 * tol + 1e-6)
+def _gemm_case(prec, m, ks, *, seed=0, **epi):
+    """the shared harness (tests/gemm_harness.py) at width 128: per-row fp64 comparison, canary rows past M"""
+    run_case(128, prec, m, Spec(list(ks), **epi), seed=seed)
 
 
 @pytest.mark.parametrize("prec", ["fp16", "bf16", "tf32", "fp32"])

@@ -7,12 +7,11 @@ finite check and the flag-off fallback."""
 import pytest
 import torch
 
-from buckgnn_b200 import engine
 from buckgnn_b200.model import BuckGNN
 from buckgnn_b200.narrow import WideTwin
 from buckgnn_b200.synth import config_batch, make_batch
 from oracle.buckgnn_oracle import OracleBuckGNN, randomize_bn_stats
-from tests.test_gpu_native128 import CANARY, _as_operand
+from tests.gemm_harness import Spec, run_case
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -20,44 +19,9 @@ DEV = "cuda:0"
 
 # ----------------------------------------------------------------------------- bg_gemm128_gathered against fp64 torch
 def _gathered_case(prec, m, n_gather, idx_kind, *, gather_ld=128, relu=True, seed=0):
-    g = torch.Generator().manual_seed(seed * 1000 + m + 10 * n_gather + gather_ld)
-    k = 128
-    a = torch.randn(m, k, generator=g)
-    w = torch.randn(128, k, generator=g) / k ** 0.5
-    act = engine.Activation(m, k, prec, DEV)
-    act.data.copy_(a.to(act.dtype))
-    act.refresh_split()
-    pack = engine.pack_linear(w.to(DEV), prec)
-    bias = torch.randn(128, generator=g) * 0.1
-    out = engine.Activation(m + 37, 128, prec, DEV)
-    out.data.fill_(CANARY)
-    n_src = max(m // 3, 5)                                     # fewer source rows than outputs: every index repeats
-    mats, idxs, gather = [], [], []
-    for _ in range(n_gather):
-        src = torch.randn(n_src, gather_ld, generator=g).to(out.dtype)
-        if idx_kind == "sorted":                               # row_of: the key node of each CSR slot
-            idx = torch.sort(torch.randint(0, n_src, (m,), generator=g)).values
-        else:                                                  # col: any node, in any order
-            idx = torch.randint(0, n_src, (m,), generator=g)
-        src_d, idx_d = src.to(DEV), idx.to(torch.int32).to(DEV)
-        mats.append(src_d)
-        idxs.append(idx_d)
-        gather.append((src_d.data_ptr(), idx_d.data_ptr()))
-    engine.gemm(engine._segments(act, pack), m, prec, out, bias=bias.data_ptr(), relu=relu, gather=gather,
-                gather_ld=gather_ld)
-    torch.cuda.synchronize()
-
-    acc = _as_operand(a, prec) @ _as_operand(w, prec).T + bias.double()
-    for src, idx in zip(mats, idxs):
-        acc = acc + src.cpu().double()[idx.cpu().long(), :128]
-    if relu:
-        acc = acc.clamp_min(0)
-    got = out.data.cpu().double()
-    assert (got[m:] == torch.tensor(CANARY).to(out.dtype).double()).all(), "rows >= M were written"
-    # fp32 sum, one rounding: within one rounding of the output format of the exact value (plus operand rounding)
-    tol = {"fp16": 2e-3, "bf16": 1.6e-2, "tf32": 1e-5, "fp32": 1e-5}[prec]
-    err = (got[:m] - acc).abs().max().item() / (acc.abs().max().item() + 1e-30)
-    assert err < tol, f"{prec} m={m} n_gather={n_gather} {idx_kind}: max err {err:.3e}"
+    """the shared harness (tests/gemm_harness.py) at width 128: fp32 sum, one rounding, compared row by row"""
+    run_case(128, prec, m, Spec([128], relu=relu, n_gather=n_gather, idx_kind=idx_kind, wide_ld=gather_ld - 128),
+             seed=seed)
 
 
 @pytest.mark.parametrize("prec", ["fp16", "bf16", "tf32", "fp32"])
