@@ -270,51 +270,38 @@ def sage_aggregate(x, out, dtype, n_nodes, rowptr, col, big_rows, n_big, aggr, w
                                     hub_lo, hub_of_row, hub_max_degree, ws, ws_bytes, stream), "bg_sage_aggregate")
 
 
-def gemm512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
-            bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
-            gather=(), gather_ld=512, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+def _gemm(entry, segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
+          bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
+          gather=(), gather_ld, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+    n = len(segments)
+    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
+    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
+    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
+    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
+                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
+    _check(getattr(load(), entry)(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group, stream),
+           entry)
+
+
+def gemm512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, gather_ld=512, **epi):
     """segments: list of (a_ptr, lda, b_ptr, ldb, k); bias / bn_scale / bn_shift are HOST pointers;
     gather: up to two (matrix_ptr, index_ptr) pairs of gathered pre-activation addends;
     pool_block_sums / pool_block_keep: the pool-fused epilogue of the last layer (see the header)."""
-    n = len(segments)
-    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
-    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
-    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
-    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
-                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
-    _check(load().bg_gemm512(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group, stream),
-           "bg_gemm512")
+    _gemm("bg_gemm512", segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, gather_ld=gather_ld, **epi)
 
 
-def gemm128(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
-            bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
-            gather=(), gather_ld=128, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+def gemm128(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, gather_ld=128, **epi):
     """bg_gemm128: gemm512 with 128-wide output rows (B [128, k], epilogue vectors [128]).  `gather` and `b_groups`
     are accepted only so that the library can reject them (BG_ERR_UNSUPPORTED)."""
-    n = len(segments)
-    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
-    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
-    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
-    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
-                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
-    _check(load().bg_gemm128(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group, stream),
-           "bg_gemm128")
+    _gemm("bg_gemm128", segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, gather_ld=gather_ld, **epi)
 
 
-def gemm128_gathered(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, bias=None, bn_scale=None,
-                     bn_shift=None, residual=None, ldr=0, normalize=False, relu=False, cta_group=2,
-                     gather=(), gather_ld=128, inv_norm_out=None, b_groups=0, pool_block_sums=None, pool_block_keep=None):
+def gemm128_gathered(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, gather_ld=128, **epi):
     """bg_gemm128_gathered: gemm128 plus up to two (matrix_ptr, index_ptr) pairs of gathered pre-activation addends,
     [*, 128] rows of the output dtype with leading dimension gather_ld.  The library rejects them together with
     normalize, residual or pool fusion."""
-    n = len(segments)
-    arr = (GemmSegment * n)(*[GemmSegment(a, lda, b, ldb, k, b_groups) for (a, lda, b, ldb, k) in segments])
-    gm = (C.c_void_p * 2)(*([g[0] for g in gather] + [None] * (2 - len(gather))))
-    gi = (C.c_void_p * 2)(*([g[1] for g in gather] + [None] * (2 - len(gather))))
-    epi = Epilogue(bias, bn_scale, bn_shift, residual, ldr, int(bool(normalize)), int(bool(relu)),
-                   gm, gi, gather_ld, inv_norm_out, pool_block_sums, pool_block_keep)
-    _check(load().bg_gemm128_gathered(arr, n, m, a_dtype, b_dtype, C.byref(epi), out, out_dtype, ldo, cta_group,
-                                      stream), "bg_gemm128_gathered")
+    _gemm("bg_gemm128_gathered", segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, gather_ld=gather_ld,
+          **epi)
 
 
 def sage_fused512(segments, m, a_dtype, b_dtype, out, out_dtype, ldo, stream, *, x, ldx, rowptr, col, aggr, hub_agg=None,

@@ -427,6 +427,22 @@ def sage_layer0_folded(h: "Activation", out: "Activation", idx: GraphIndex, w: F
              bn_shift=_p(w.bn_shift), normalize=normalize, relu=relu)
 
 
+def pack_encoder(enc, precision: str, width: int = 512) -> Tuple[Dict[str, torch.Tensor], LinearPack]:
+    """(enc_w, w3) of `encoder_forward` for a node / edge encoder.  `width` 128: the 2-layer encoder Linear(F,64) ReLU
+    Linear(64,128) of h <= 128 (Models/BuckGNN.py:41-48) runs on the same kernels by exact embedding: [I; 0] as the
+    second Linear (the 64-wide hidden layer stored 128 wide), then Linear(64,128) with W zero-padded to [128, 128]."""
+    f32 = lambda t: t.detach().float().contiguous()
+    enc_w = {"w1": f32(enc[0].weight), "b1": f32(enc[0].bias)}
+    if width == 512:
+        enc_w.update(w2=f32(enc[2].weight), b2=f32(enc[2].bias), b3_host=host_vector(enc[4].bias))
+        return enc_w, pack_linear(enc[4].weight, precision)
+    dev = enc[0].weight.device
+    w2 = torch.zeros((128, 64), dtype=torch.float32, device=dev)
+    w2[:64] = torch.eye(64, device=dev)
+    enc_w.update(w2=w2, b2=torch.zeros(128, dtype=torch.float32, device=dev), b3_host=host_vector(enc[2].bias))
+    return enc_w, pack_linear(torch.nn.functional.pad(f32(enc[2].weight), (0, 64)), precision)
+
+
 def encoder_forward(x: torch.Tensor, enc_w: Dict[str, torch.Tensor], w3: LinearPack, precision: str,
                     out: Activation, cta_group: int, row_gather: Optional[torch.Tensor] = None,
                     nonfinite: Optional[torch.Tensor] = None) -> None:
@@ -512,6 +528,24 @@ def sage_layer(x: Activation, agg: Activation, out: Activation, idx: GraphIndex,
                 bias=layer.bias.data_ptr(), bn_scale=_p(layer.bn_scale), bn_shift=_p(layer.bn_shift),
                 residual=x.data.data_ptr() if residual else None, ldr=x.data.shape[1],
                 normalize=normalize, relu=relu, **pool)
+
+
+def pack_decoder(dec, width: int = 512) -> Dict[str, torch.Tensor]:
+    """The fp32 decoder weights w1, b1, w2, b2, w3, b3 of `pool_head`.  `width` 128: the 2-layer decoder
+    Linear(in,64) ReLU Linear(64,out) of h <= 128 (Models/BuckGNN.py:41-65) in the 3-layer form bg_pool_head128
+    takes (include/buckgnn_b200.h): w1 = [W1; 0], w2 = [I64 | 0], w3 = W2."""
+    f32 = lambda t: t.detach().float().contiguous()
+    if width == 512:
+        return {"w1": f32(dec[0].weight), "b1": f32(dec[0].bias), "w2": f32(dec[2].weight),
+                "b2": f32(dec[2].bias), "w3": f32(dec[4].weight), "b3": f32(dec[4].bias)}
+    dev = dec[0].weight.device
+    w1 = torch.zeros((128, dec[0].in_features), dtype=torch.float32, device=dev)
+    b1 = torch.zeros(128, dtype=torch.float32, device=dev)
+    w1[:64], b1[:64] = f32(dec[0].weight), f32(dec[0].bias)
+    w2 = torch.zeros((64, 128), dtype=torch.float32, device=dev)
+    w2[:, :64] = torch.eye(64, device=dev)
+    return {"w1": w1, "b1": b1, "w2": w2, "b2": torch.zeros(64, dtype=torch.float32, device=dev),
+            "w3": f32(dec[2].weight), "b3": f32(dec[2].bias)}
 
 
 def pool_head(x: Activation, idx: GraphIndex, dec: Dict[str, torch.Tensor], out_dim: int,

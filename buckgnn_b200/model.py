@@ -250,22 +250,21 @@ class BuckGNN(nn.Module):
             return list(zip(self.sage_layers_1, self.batch_norms_1)) + list(zip(self.sage_layers_2, self.batch_norms_2))
         return []
 
-    def _packed(self):
-        """Operand-format copies of the weights, rebuilt when any parameter/buffer changes."""
-        sig = self._signature()
+    def _packed(self, width: int = 512):
+        """Operand-format copies of the weights for the kernels of `width` (512, or 128: a hidden_channels = 128 model
+        in eval on the 128-wide kernels), rebuilt when any parameter/buffer changes.  Only the encoders and the decoder
+        pack differently at 128 (engine.pack_encoder / pack_decoder)."""
+        sig = (width,) + self._signature()
         if self._pack_sig == sig:
             return self._packs
         prec = self.precision
         f32 = lambda t: t.detach().float().contiguous()
         enc = self.node_encoder
-        packs = {"enc": {"w1": f32(enc[0].weight), "b1": f32(enc[0].bias), "w2": f32(enc[2].weight),
-                         "b2": f32(enc[2].bias), "b3_host": engine.host_vector(enc[4].bias)},
-                 "enc_w3": engine.pack_linear(enc[4].weight, prec)}
-        dec = self.decoder
-        packs["dec"] = {"w1": f32(dec[0].weight), "b1": f32(dec[0].bias), "w2": f32(dec[2].weight),
-                        "b2": f32(dec[2].bias), "w3": f32(dec[4].weight), "b3": f32(dec[4].bias)}
+        packs = {}
+        packs["enc"], packs["enc_w3"] = engine.pack_encoder(enc, prec, width)
+        packs["dec"] = engine.pack_decoder(self.decoder, width)
         if self.prediction_type != "buckling" and self.hidden_channels >= 256:
-            packs["node_head"] = engine.pack_node_head(dec, prec)
+            packs["node_head"] = engine.pack_node_head(self.decoder, prec)
         mpl = self.pooling_mpl.mlp[0]
         packs["pool_mlp"] = {"w": f32(mpl.weight), "b": f32(mpl.bias)}
         layers, seen = [], {}
@@ -283,79 +282,19 @@ class BuckGNN(nn.Module):
             sl = []                                   # num_layers == 1: the pooling runs on the encoder output itself
         if self.fold_encoder and sl and sl[0][0].aggr != "max":
             conv0, bn0 = sl[0]
-            packs["layer0_folded"] = engine.pack_folded_layer0(enc[4], conv0, bn0, conv0.aggr, prec)  # None: unfolded
-        if self.model_name in ("EA_GNN", "EA_GNN_Shared"):
-            ee = self.edge_encoder
-            packs["edge_enc"] = {"w1": f32(ee[0].weight), "b1": f32(ee[0].bias), "w2": f32(ee[2].weight),
-                                 "b2": f32(ee[2].bias), "b3_host": engine.host_vector(ee[4].bias)}
-            packs["edge_enc_w3"] = engine.pack_linear(ee[4].weight, prec)
-            if self.model_name == "EA_GNN_Shared":
-                shared = engine.pack_gnblock(self.shared_gn_block, prec)
-                packs["gn"] = [shared] * self.num_layers
-            else:
-                packs["gn"] = [engine.pack_gnblock(b, prec) for b in self.gn_blocks]
+            packs["layer0_folded"] = engine.pack_folded_layer0(enc[-1], conv0, bn0, conv0.aggr, prec,
+                                                               width=width)                       # None: unfolded
+        if self.model_name in ("EA_GNN", "EA_GNN_Shared", "EAGNN_SAG"):
+            packs["edge_enc"], packs["edge_enc_w3"] = engine.pack_encoder(self.edge_encoder, prec, width)
+        if self.model_name == "EA_GNN_Shared":
+            packs["gn"] = [engine.pack_gnblock(self.shared_gn_block, prec, width=width)] * self.num_layers
+        elif self.model_name == "EA_GNN":
+            packs["gn"] = [engine.pack_gnblock(b, prec, width=width) for b in self.gn_blocks]
         if self.model_name in ("GraphSAGE_SAG", "EAGNN_SAG"):
             packs["sag_pool"] = engine.pack_sag_pool(self.pool)
         if self.model_name == "EAGNN_SAG":
-            ee = self.edge_encoder
-            packs["edge_enc"] = {"w1": f32(ee[0].weight), "b1": f32(ee[0].bias), "w2": f32(ee[2].weight),
-                                 "b2": f32(ee[2].bias), "b3_host": engine.host_vector(ee[4].bias)}
-            packs["edge_enc_w3"] = engine.pack_linear(ee[4].weight, prec)
             packs["gn1"] = [engine.pack_gnblock(b, prec) for b in self.gnn_layers_1]
             packs["gn2"] = [engine.pack_gnblock(b, prec) for b in self.gnn_layers_2]
-        self._packs, self._pack_sig = packs, sig
-        return packs
-
-    def _packed128(self):
-        """Operand-format copies for the 128-wide kernels (hidden_channels == 128, eval), rebuilt when any parameter /
-        buffer changes.  The 2-layer encoder / decoder of h <= 128 (Models/BuckGNN.py:41-65) run on the 3-layer
-        kernels by exact embedding: encoder Linear(F,64) ReLU [I; 0] ReLU (the 64-wide hidden layer stored 128 wide),
-        then its Linear(64,128) padded to [128,128]; decoder [W1; 0] ReLU [I64 | 0] ReLU W2."""
-        sig = self._signature()
-        if self._pack_sig == sig:
-            return self._packs
-        prec = self.precision
-        f32 = lambda t: t.detach().float().contiguous()
-        enc, dec = self.node_encoder, self.decoder
-        dev = enc[0].weight.device
-        eye = torch.eye(64, device=dev)
-        zeros = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=dev)
-        w2 = zeros(128, 64)
-        w2[:64] = eye
-        packs = {"enc": {"w1": f32(enc[0].weight), "b1": f32(enc[0].bias), "w2": w2, "b2": zeros(128),
-                         "b3_host": engine.host_vector(enc[2].bias)},
-                 "enc_w3": engine.pack_linear(torch.nn.functional.pad(f32(enc[2].weight), (0, 64)), prec)}
-        w1, b1 = zeros(128, dec[0].in_features), zeros(128)
-        w1[:64], b1[:64] = f32(dec[0].weight), f32(dec[0].bias)
-        i64 = zeros(64, 128)
-        i64[:, :64] = eye
-        packs["dec"] = {"w1": w1, "b1": b1, "w2": i64, "b2": zeros(64), "w3": f32(dec[2].weight), "b3": f32(dec[2].bias)}
-        mpl = self.pooling_mpl.mlp[0]
-        packs["pool_mlp"] = {"w": f32(mpl.weight), "b": f32(mpl.bias)}
-        layers, seen = [], {}
-        for conv, bn in self._sage_layers():
-            if id(conv) not in seen:
-                scale, shift = engine.fold_batchnorm(bn) if bn is not None else (None, None)
-                seen[id(conv)] = SageLayerPack(engine.pack_linear(conv.lin_l.weight, prec),
-                                               engine.pack_linear(conv.lin_r.weight, prec),
-                                               engine.host_vector(conv.lin_l.bias), scale, shift)
-            layers.append(seen[id(conv)])
-        packs["layers"] = layers
-        folded = None
-        sl = self._sage_layers()
-        if self.fold_encoder and sl and sl[0][0].aggr != "max":
-            conv0, bn0 = sl[0]
-            folded = engine.pack_folded_layer0(enc[2], conv0, bn0, conv0.aggr, prec, width=128)   # None: unfolded
-        packs["layer0_folded"] = folded
-        if self.model_name in _NATIVE128_EAGNN_MODELS:      # the edge encoder by the same [I; 0] embedding
-            ee = self.edge_encoder
-            packs["edge_enc"] = {"w1": f32(ee[0].weight), "b1": f32(ee[0].bias), "w2": w2, "b2": zeros(128),
-                                 "b3_host": engine.host_vector(ee[2].bias)}
-            packs["edge_enc_w3"] = engine.pack_linear(torch.nn.functional.pad(f32(ee[2].weight), (0, 64)), prec)
-            if self.model_name == "EA_GNN_Shared":
-                packs["gn"] = [engine.pack_gnblock(self.shared_gn_block, prec, width=128)] * self.num_layers
-            else:
-                packs["gn"] = [engine.pack_gnblock(b, prec, width=128) for b in self.gn_blocks]
         self._packs, self._pack_sig = packs, sig
         return packs
 
@@ -536,7 +475,7 @@ class BuckGNN(nn.Module):
     def _forward_cuda_eagnn(self, x, edge_index, edge_attr, batch, node_level=False, width=512):
         """EA-GNN / "CustomGNN" path (reference :326-336, :375-387, GraphNetBlock :528-566).  `width` 128: a
         hidden_channels = 128 model on the 128-wide kernels (graph-level head only)."""
-        packs = self._packed() if width == 512 else self._packed128()
+        packs = self._packed(width)
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         if not edge_attr.is_cuda:
@@ -571,7 +510,7 @@ class BuckGNN(nn.Module):
 
     def _forward_cuda(self, x, edge_index, batch, node_level=False, width=512):
         """`width` 128: a hidden_channels = 128 model on the 128-wide kernels (bg_gemm128, bg_pool_head128)."""
-        packs = self._packed() if width == 512 else self._packed128()
+        packs = self._packed(width)
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         n = x.shape[0]

@@ -204,231 +204,141 @@ class GradStore:
 
 
 # ----------------------------------------------------------------------------- shared pieces: encoders and head
+def _mat(t):
+    """(tensor, format code) of an fp32 matrix or of an Activation in its storage format."""
+    return (t.data, t.code) if isinstance(t, Activation) else (t, capi.BG_F32)
+
+
+def _linears(seq):
+    """[(nn.Linear, whether an nn.ReLU follows it)] of an nn.Sequential."""
+    mods = list(seq)
+    return [(m, isinstance(nxt, torch.nn.ReLU)) for m, nxt in zip(mods, mods[1:] + [None])
+            if isinstance(m, torch.nn.Linear)]
+
+
+def chain_forward(chain, x, out: Optional[Activation] = None):
+    """y = L_k(..relu(L_1(x))..) for chain = [(nn.Linear, relu after)], one bg_sgemm per Linear.  `x` is fp32 or an
+    Activation; every intermediate is fp32, and so is y unless `out` (an Activation) is given.  Returns (y, the input
+    of every Linear): the operands of `chain_backward`."""
+    F32 = capi.BG_F32
+    m = _mat(x)[0].shape[0]
+    xs = []
+    for i, (lin, relu) in enumerate(chain):
+        w, b = lin.weight.detach().float().contiguous(), lin.bias.detach().float().contiguous()
+        n_out, k = w.shape
+        y = out if out is not None and i == len(chain) - 1 else _f32((m, n_out), w.device)
+        (xd, xc), (yd, yc) = _mat(x), _mat(y)
+        sgemm(xd, xc, k, 1, w, F32, 1, k, m, n_out, k, yd, yc, n_out, bias=b, relu=relu)
+        xs.append(x)
+        x = y
+    if out is not None:
+        out.refresh_split()
+    return x, xs
+
+
+def chain_backward(chain, xs, dy, grads: GradStore, dx=None):
+    """Backward of `chain_forward` given dy = d(y) (fp32 or an Activation), last Linear first: dW = dy^T x,
+    db = colsum(dy), then d(x) = dy W, masked by x > 0 where x is the output of a ReLU of the chain.  The gradient of
+    the chain's input goes to `dx` (fp32 or an Activation) and is not computed without one; the others are fp32."""
+    F32 = capi.BG_F32
+    m = _mat(xs[0])[0].shape[0]
+    for i in range(len(chain) - 1, -1, -1):
+        lin = chain[i][0]
+        w = lin.weight.detach().float().contiguous()
+        n_out, k = w.shape
+        (dyd, dyc), (xd, xc) = _mat(dy), _mat(xs[i])
+        dw, _ = grads.get(lin.weight); db, _ = grads.get(lin.bias)
+        sgemm(dyd, dyc, 1, n_out, xd, xc, k, 1, n_out, k, m, dw, F32, k)
+        colsum(dyd, dyc, m, n_out, n_out, db)
+        if i == 0 and dx is None:
+            break
+        dxi = dx if i == 0 else _f32((m, k), w.device)
+        mask = xd if i > 0 and chain[i - 1][1] else None
+        dxd, dxc = _mat(dxi)
+        sgemm(dyd, dyc, n_out, 1, w, F32, k, 1, m, k, n_out, dxd, dxc, k, mask=mask,
+              mask_ld=0 if mask is None else k)
+        dy = dxi
+    if isinstance(dx, Activation):
+        dx.refresh_split()
+    return dx
+
+
 def encoder_forward_train(enc, inp: torch.Tensor, prec: str, bias3_host: torch.Tensor, width: int = 512):
     """node_encoder / edge_encoder (Models/BuckGNN.py:68-82): the two narrow Linears on bg_sgemm (fp32), the
     128 -> 512 one on the tensor cores.  Returns (h1 [n,64] f32, h2 [n,128], out [n,512]).
     width 128: the 2-layer encoder Linear(F,64) ReLU Linear(64,128) (:41-48), both on bg_sgemm; returns
     (h1 [n,64] f32, None, out [n,128])."""
-    dev, n, f = inp.device, inp.shape[0], inp.shape[1]
-    code = engine.PRECISION_FORMATS[prec][0]
-    F32 = capi.BG_F32
-    w1, b1 = enc[0].weight.detach().float().contiguous(), enc[0].bias.detach().float().contiguous()
-    w2, b2 = enc[2].weight.detach().float().contiguous(), enc[2].bias.detach().float().contiguous()
-    if width == 128:
-        with engine.TIMERS.span("train_encoder"):
-            h1 = _f32((n, 64), dev)
-            sgemm(inp, F32, f, 1, w1, F32, 1, f, n, 64, f, h1, F32, 64, bias=b1, relu=True)
-            out = Activation(n, 128, prec, dev)
-            sgemm(h1, F32, 64, 1, w2, F32, 1, 64, n, 128, 64, out.data, code, 128, bias=b2)
-            out.refresh_split()
-        return h1, None, out
+    dev, n = inp.device, inp.shape[0]
     with engine.TIMERS.span("train_encoder"):
-        h1 = _f32((n, 64), dev)
-        sgemm(inp, F32, f, 1, w1, F32, 1, f, n, 64, f, h1, F32, 64, bias=b1, relu=True)
-        h2 = Activation(n, 128, prec, dev)
-        sgemm(h1, F32, 64, 1, w2, F32, 1, 64, n, 128, 64, h2.data, code, 128, bias=b2, relu=True)
-        h2.refresh_split()
+        h = Activation(n, 128, prec, dev)                    # h2, or the output at width 128
+        _, (_, h1) = chain_forward(_linears(enc)[:2], inp, out=h)
+        if width == 128:
+            return h1, None, h
         out = Activation(n, 512, prec, dev)
-        engine.gemm512(engine._segments(h2, engine.pack_linear(enc[4].weight, prec)), n, prec, out,
+        engine.gemm512(engine._segments(h, engine.pack_linear(enc[4].weight, prec)), n, prec, out,
                        bias=bias3_host.data_ptr())
-    return h1, h2, out
+    return h1, h, out
 
 
 def encoder_backward(enc, inp: torch.Tensor, h1: torch.Tensor, h2: Optional[Activation], dout: Activation, prec: str,
                      grads: GradStore) -> None:
-    """Gradients of the three encoder Linears given d(out) [n, 512] (of the two given d(out) [n, 128] at width 128)."""
-    dev, n, f = inp.device, inp.shape[0], inp.shape[1]
+    """Gradients of the three encoder Linears given d(out) [n, 512] (of the two given d(out) [n, 128] at width 128,
+    where h2 is None)."""
+    dev, n = inp.device, inp.shape[0]
     code = engine.PRECISION_FORMATS[prec][0]
-    F32 = capi.BG_F32
     s = _stream()
-    dx0 = dout.data
-    if dx0.shape[1] == 128:
-        with engine.TIMERS.span("train_encoder_bwd"):
-            w2 = enc[2].weight.detach().float().contiguous()          # [128, 64]
-            dw2e, _ = grads.get(enc[2].weight); db2e, _ = grads.get(enc[2].bias)
-            sgemm(dx0, code, 1, 128, h1, F32, 64, 1, 128, 64, n, dw2e, F32, 64)
-            colsum(dx0, code, n, 128, 128, db2e)
-            dh1 = _f32((n, 64), dev)
-            sgemm(dx0, code, 128, 1, w2, F32, 64, 1, n, 64, 128, dh1, F32, 64, mask=h1, mask_ld=64)
-            dw1e, _ = grads.get(enc[0].weight); db1e, _ = grads.get(enc[0].bias)
-            sgemm(dh1, F32, 1, 64, inp, F32, f, 1, 64, f, n, dw1e, F32, f)
-            colsum(dh1, F32, n, 64, 64, db1e)
-        return
     with engine.TIMERS.span("train_encoder_bwd"):
-        w3 = enc[4].weight.detach().float().contiguous()          # [512, 128]
-        w2 = enc[2].weight.detach().float().contiguous()
-        dw3e, _ = grads.get(enc[4].weight); db3e, _ = grads.get(enc[4].bias)
-        tmp = _f32((512, 512), dev)
-        weight_grad_mn(dx0, h2.data, code, n, tmp, False)             # dW3 = dx0^T h2; columns >= 128 of tmp come out 0
-        dw3e.copy_(tmp[:, :128])
-        colsum(dx0, code, n, 512, 512, db3e)
-        # dh2 = (dx0 W3) [h2 > 0]: W3^T zero-padded to 512 output rows on the tensor cores, then mask + narrow
-        w3t_pad = torch.zeros((512, 512), dtype=torch.float32, device=dev)
-        capi.transpose_chunks(w3.data_ptr(), F32, 512, 128, 128, 1, 512, w3t_pad.data_ptr(), s)
-        full = Activation(n, 512, prec, dev)
-        engine.gemm512(engine._segments(dout, engine.pack_linear(w3t_pad, prec)), n, prec, full)
-        dh2 = _f32((n, 128), dev)
-        capi.mask_narrow(full.data.data_ptr(), code, 512, h2.data.data_ptr(), code, 128, n, 128, dh2.data_ptr(), s)
-        dw2e, _ = grads.get(enc[2].weight); db2e, _ = grads.get(enc[2].bias)
-        sgemm(dh2, F32, 1, 128, h1, F32, 64, 1, 128, 64, n, dw2e, F32, 64)
-        colsum(dh2, F32, n, 128, 128, db2e)
-        dh1 = _f32((n, 64), dev)
-        sgemm(dh2, F32, 128, 1, w2, F32, 64, 1, n, 64, 128, dh1, F32, 64, mask=h1, mask_ld=64)
-        dw1e, _ = grads.get(enc[0].weight); db1e, _ = grads.get(enc[0].bias)
-        sgemm(dh1, F32, 1, 64, inp, F32, f, 1, 64, f, n, dw1e, F32, f)
-        colsum(dh1, F32, n, 64, 64, db1e)
+        dh = dout                                                 # d(output of the bg_sgemm Linears)
+        if h2 is not None:
+            w3 = enc[4].weight.detach().float().contiguous()      # [512, 128]
+            dw3e, _ = grads.get(enc[4].weight); db3e, _ = grads.get(enc[4].bias)
+            tmp = _f32((512, 512), dev)
+            weight_grad_mn(dout.data, h2.data, code, n, tmp, False)    # dW3 = dout^T h2; columns >= 128 of tmp come out 0
+            dw3e.copy_(tmp[:, :128])
+            colsum(dout.data, code, n, 512, 512, db3e)
+            # dh2 = (dout W3) [h2 > 0]: W3^T zero-padded to 512 output rows on the tensor cores, then mask + narrow
+            w3t_pad = torch.zeros((512, 512), dtype=torch.float32, device=dev)
+            capi.transpose_chunks(w3.data_ptr(), capi.BG_F32, 512, 128, 128, 1, 512, w3t_pad.data_ptr(), s)
+            full = Activation(n, 512, prec, dev)
+            engine.gemm512(engine._segments(dout, engine.pack_linear(w3t_pad, prec)), n, prec, full)
+            dh = _f32((n, 128), dev)
+            capi.mask_narrow(full.data.data_ptr(), code, 512, h2.data.data_ptr(), code, 128, n, 128, dh.data_ptr(), s)
+        chain_backward(_linears(enc)[:2], [inp, h1], dh, grads)
 
 
-def _decoder128_embedded(dec) -> dict:
-    """The 2-layer decoder Linear(in,64) ReLU Linear(64,out) of a hidden_channels = 128 model in the 3-layer form
-    bg_pool_head128 takes (include/buckgnn_b200.h): w1 = [W1; 0], w2 = [I64 | 0], w3 = W2."""
-    f32 = lambda t: t.detach().float().contiguous()
-    dev = dec[0].weight.device
-    w1 = torch.zeros((128, dec[0].in_features), dtype=torch.float32, device=dev)
-    b1 = torch.zeros(128, dtype=torch.float32, device=dev)
-    w1[:64], b1[:64] = f32(dec[0].weight), f32(dec[0].bias)
-    w2 = torch.zeros((64, 128), dtype=torch.float32, device=dev)
-    w2[:, :64] = torch.eye(64, device=dev)
-    return {"w1": w1, "b1": b1, "w2": w2, "b2": torch.zeros(64, dtype=torch.float32, device=dev),
-            "w3": f32(dec[2].weight), "b3": f32(dec[2].bias)}
-
-
-def _head_forward_train128(model, cur: Activation, idx, sv) -> torch.Tensor:
-    """head_forward_train at width 128: bg_pool_head128's pooled feature, MLPPooling Linear(128,128) and the 2-layer
-    decoder Linear(128 | 256, 64) ReLU Linear(64, out) on bg_sgemm.  sv.h1d is the decoder's hidden layer [G, 64];
-    there is no second one (sv.h2d = None)."""
-    dev = cur.data.device
-    dec = model.decoder
-    F32 = capi.BG_F32
-    with engine.TIMERS.span("pool_head"):
-        _, raw = engine.pool_head(cur, idx, _decoder128_embedded(dec), model.output_dim, want_pooled=True,
-                                  pooling=model.pooling_layer)
-        g_count, in_dim = raw.shape
-        sv.mlp = None
-        dec_in = raw
-        if model.pooling_layer in ("mlp", "mlp_no_super"):                     # MLPPooling (:568-581)
-            lin = model.pooling_mpl.mlp[0]
-            wp, bp = lin.weight.detach().float().contiguous(), lin.bias.detach().float().contiguous()
-            dec_in = _f32((g_count, 128), dev)
-            sgemm(raw, F32, 128, 1, wp, F32, 1, 128, g_count, 128, 128, dec_in, F32, 128, bias=bp, relu=True)
-            sv.mlp = (lin, wp)
-        decw = {"w1": dec[0].weight.detach().float().contiguous(), "b1": dec[0].bias.detach().float().contiguous(),
-                "w2": dec[2].weight.detach().float().contiguous(), "b2": dec[2].bias.detach().float().contiguous()}
-        out_dim = model.output_dim
-        h1d, pred = _f32((g_count, 64), dev), _f32((g_count, out_dim), dev)
-        sgemm(dec_in, F32, in_dim, 1, decw["w1"], F32, 1, in_dim, g_count, 64, in_dim, h1d, F32, 64, bias=decw["b1"], relu=True)
-        sgemm(h1d, F32, 64, 1, decw["w2"], F32, 1, 64, g_count, out_dim, 64, pred, F32, out_dim, bias=decw["b2"])
-    sv.decw, sv.raw, sv.dec_in, sv.h1d, sv.h2d = decw, raw, dec_in, h1d, None
-    return pred
-
-
-def _head_backward128(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
-    """head_backward at width 128: returns d(last layer output) [n, 128]."""
-    dev = dpred.device
-    code = engine.PRECISION_FORMATS[prec][0]
-    F32 = capi.BG_F32
-    g_count, out_dim = sv.raw.shape[0], model.output_dim
-    in_dim = sv.dec_in.shape[1]
-    d, dec = sv.decw, model.decoder
-    h1d, dec_in = sv.h1d, sv.dec_in
-    with engine.TIMERS.span("train_head_bwd"):
-        dw2, _ = grads.get(dec[2].weight); db2, _ = grads.get(dec[2].bias)
-        sgemm(dpred, F32, 1, out_dim, h1d, F32, 64, 1, out_dim, 64, g_count, dw2, F32, 64)
-        colsum(dpred, F32, g_count, out_dim, out_dim, db2)
-        dh1d = _f32((g_count, 64), dev)
-        sgemm(dpred, F32, out_dim, 1, d["w2"], F32, 64, 1, g_count, 64, out_dim, dh1d, F32, 64, mask=h1d, mask_ld=64)
-        dw1, _ = grads.get(dec[0].weight); db1, _ = grads.get(dec[0].bias)
-        sgemm(dh1d, F32, 1, 64, dec_in, F32, in_dim, 1, 64, in_dim, g_count, dw1, F32, in_dim)
-        colsum(dh1d, F32, g_count, 64, 64, db1)
-        dpooled = _f32((g_count, in_dim), dev)
-        if sv.mlp is None:
-            sgemm(dh1d, F32, 64, 1, d["w1"], F32, in_dim, 1, g_count, in_dim, 64, dpooled, F32, in_dim)
-        else:                                                   # through relu(Linear(128, 128)) of MLPPooling
-            lin, wp = sv.mlp
-            dpm = _f32((g_count, 128), dev)
-            sgemm(dh1d, F32, 64, 1, d["w1"], F32, 128, 1, g_count, 128, 64, dpm, F32, 128, mask=dec_in, mask_ld=128)
-            dwp, _ = grads.get(lin.weight); dbp, _ = grads.get(lin.bias)
-            sgemm(dpm, F32, 1, 128, sv.raw, F32, 128, 1, 128, 128, g_count, dwp, F32, 128)
-            colsum(dpm, F32, g_count, 128, 128, dbp)
-            sgemm(dpm, F32, 128, 1, wp, F32, 128, 1, g_count, 128, 128, dpooled, F32, 128)
-        dcur = Activation(n, 128, prec, dev)
-        capi.pool_backward(dpooled.data_ptr(), in_dim, sv.idx.graph_ptr.data_ptr(), g_count,
-                           capi.POOL_MODES[model.pooling_layer], n, dcur.data.data_ptr(), code, _stream(), width=128)
-    return dcur
+def _keep_head(sv, chain, xs, mlp: bool) -> None:
+    """The head's chain and the input of each of its Linears for the backward pass.  The decoder's input and hidden
+    layers are also kept by name: dec_in, h1d and h2d (None for the 2-layer decoder of h <= 128); `mlp` is MLPPooling's
+    Linear, or None."""
+    sv.head, sv.head_in = chain, xs
+    sv.mlp = chain[0][0] if mlp else None
+    sv.dec_in, sv.h1d, *h2d = xs[int(mlp):]
+    sv.h2d = h2d[0] if h2d else None
 
 
 def head_forward_train(model, cur: Activation, idx, sv) -> torch.Tensor:
     """get_pooling_layer + decoder (Models/BuckGNN.py:246-307, 515-516): the pooled feature comes from bg_pool_head
-    (its own decoder output is not used here); MLPPooling and the decoder run on bg_sgemm so that their hidden
-    layers are kept for the backward pass."""
-    if cur.data.shape[1] == 128:
-        return _head_forward_train128(model, cur, idx, sv)
-    dev = cur.data.device
-    dec = model.decoder
-    decw = {"w1": dec[0].weight.detach(), "b1": dec[0].bias.detach(), "w2": dec[2].weight.detach(),
-            "b2": dec[2].bias.detach(), "w3": dec[4].weight.detach(), "b3": dec[4].bias.detach()}
-    decw = {k: v.float().contiguous() for k, v in decw.items()}
-    F32 = capi.BG_F32
+    (its own decoder output is not used here); MLPPooling (:568-581) and the decoder run on bg_sgemm so that their
+    hidden layers are kept for the backward pass."""
+    mlp = model.pooling_layer in ("mlp", "mlp_no_super")
+    chain = (_linears(model.pooling_mpl.mlp) if mlp else []) + _linears(model.decoder)
     with engine.TIMERS.span("pool_head"):
-        _, raw = engine.pool_head(cur, idx, decw, model.output_dim, want_pooled=True, pooling=model.pooling_layer)
-        g_count, in_dim = raw.shape
-        sv.mlp = None
-        dec_in = raw
-        if model.pooling_layer in ("mlp", "mlp_no_super"):                     # MLPPooling (:568-581)
-            lin = model.pooling_mpl.mlp[0]
-            wp, bp = lin.weight.detach().float().contiguous(), lin.bias.detach().float().contiguous()
-            dec_in = _f32((g_count, 512), dev)
-            sgemm(raw, F32, 512, 1, wp, F32, 1, 512, g_count, 512, 512, dec_in, F32, 512, bias=bp, relu=True)
-            sv.mlp = (lin, wp)
-        h1d, h2d = _f32((g_count, 128), dev), _f32((g_count, 64), dev)
-        out_dim = model.output_dim
-        pred = _f32((g_count, out_dim), dev)
-        sgemm(dec_in, F32, in_dim, 1, decw["w1"], F32, 1, in_dim, g_count, 128, in_dim, h1d, F32, 128, bias=decw["b1"], relu=True)
-        sgemm(h1d, F32, 128, 1, decw["w2"], F32, 1, 128, g_count, 64, 128, h2d, F32, 64, bias=decw["b2"], relu=True)
-        sgemm(h2d, F32, 64, 1, decw["w3"], F32, 1, 64, g_count, out_dim, 64, pred, F32, out_dim, bias=decw["b3"])
-    sv.decw, sv.raw, sv.dec_in, sv.h1d, sv.h2d = decw, raw, dec_in, h1d, h2d
+        _, raw = engine.pool_head(cur, idx, engine.pack_decoder(model.decoder, cur.data.shape[1]), model.output_dim,
+                                  want_pooled=True, pooling=model.pooling_layer)
+        pred, xs = chain_forward(chain, raw)
+    _keep_head(sv, chain, xs, mlp)
     return pred
 
 
 def head_backward(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
-    """Decoder (+ MLPPooling) and pooling backward: returns d(last layer output) [n, 512] ([n, 128] at width 128)."""
-    if sv.h2d is None:
-        return _head_backward128(model, sv, dpred, n, prec, grads)
-    dev = dpred.device
-    code = engine.PRECISION_FORMATS[prec][0]
-    F32 = capi.BG_F32
-    g_count, out_dim = sv.raw.shape[0], model.output_dim
-    in_dim = sv.dec_in.shape[1]
-    d, dec = sv.decw, model.decoder
-    h1d, h2d, dec_in = sv.h1d, sv.h2d, sv.dec_in
+    """Decoder (+ MLPPooling) and pooling backward: returns d(last layer output) [n, hidden_channels]."""
+    dev, W = dpred.device, model.hidden_channels
+    g_count, in_dim = sv.head_in[0].shape
     with engine.TIMERS.span("train_head_bwd"):
-        dw3, _ = grads.get(dec[4].weight); db3, _ = grads.get(dec[4].bias)
-        sgemm(dpred, F32, 1, out_dim, h2d, F32, 64, 1, out_dim, 64, g_count, dw3, F32, 64)
-        colsum(dpred, F32, g_count, out_dim, out_dim, db3)
-        dh2d = _f32((g_count, 64), dev)
-        sgemm(dpred, F32, out_dim, 1, d["w3"], F32, 64, 1, g_count, 64, out_dim, dh2d, F32, 64, mask=h2d, mask_ld=64)
-        dw2, _ = grads.get(dec[2].weight); db2, _ = grads.get(dec[2].bias)
-        sgemm(dh2d, F32, 1, 64, h1d, F32, 128, 1, 64, 128, g_count, dw2, F32, 128)
-        colsum(dh2d, F32, g_count, 64, 64, db2)
-        dh1d = _f32((g_count, 128), dev)
-        sgemm(dh2d, F32, 64, 1, d["w2"], F32, 128, 1, g_count, 128, 64, dh1d, F32, 128, mask=h1d, mask_ld=128)
-        dw1, _ = grads.get(dec[0].weight); db1, _ = grads.get(dec[0].bias)
-        sgemm(dh1d, F32, 1, 128, dec_in, F32, in_dim, 1, 128, in_dim, g_count, dw1, F32, in_dim)
-        colsum(dh1d, F32, g_count, 128, 128, db1)
-        dpooled = _f32((g_count, in_dim), dev)
-        if sv.mlp is None:
-            sgemm(dh1d, F32, 128, 1, d["w1"], F32, in_dim, 1, g_count, in_dim, 128, dpooled, F32, in_dim)
-        else:                                                   # through relu(Linear(512, 512)) of MLPPooling
-            lin, wp = sv.mlp
-            dpm = _f32((g_count, 512), dev)
-            sgemm(dh1d, F32, 128, 1, d["w1"], F32, 512, 1, g_count, 512, 128, dpm, F32, 512, mask=dec_in, mask_ld=512)
-            dwp, _ = grads.get(lin.weight); dbp, _ = grads.get(lin.bias)
-            sgemm(dpm, F32, 1, 512, sv.raw, F32, 512, 1, 512, 512, g_count, dwp, F32, 512)
-            colsum(dpm, F32, g_count, 512, 512, dbp)
-            sgemm(dpm, F32, 512, 1, wp, F32, 512, 1, g_count, 512, 512, dpooled, F32, 512)
-        dcur = Activation(n, 512, prec, dev)
+        dpooled = chain_backward(sv.head, sv.head_in, dpred, grads, dx=_f32((g_count, in_dim), dev))
+        dcur = Activation(n, W, prec, dev)
         capi.pool_backward(dpooled.data_ptr(), in_dim, sv.idx.graph_ptr.data_ptr(), g_count,
-                           capi.POOL_MODES[model.pooling_layer], n, dcur.data.data_ptr(), code, _stream())
+                           capi.POOL_MODES[model.pooling_layer], n, dcur.data.data_ptr(), dcur.code, _stream(), width=W)
     return dcur
 
 
@@ -438,51 +348,21 @@ def is_node_level(model) -> bool:
 
 def node_head_forward_train(model, cur: Activation, sv) -> torch.Tensor:
     """Node-level heads (`static_disp`, `static_stress`, `mode_shape`): `decoder(x)` on every node
-    (Models/BuckGNN.py:518-524; the caller drops the super-node rows).  Three `bg_sgemm` calls whose hidden layers
-    are kept for the backward pass."""
-    dev, n = cur.data.device, cur.data.shape[0]
-    dec = model.decoder
-    if len(dec) != 5:
+    (Models/BuckGNN.py:518-524; the caller drops the super-node rows) on bg_sgemm, its hidden layers kept for the
+    backward pass."""
+    if len(model.decoder) != 5:
         raise NotImplementedError("buckgnn_b200: node-level training needs the 3-layer decoder (hidden_channels >= 256)")
-    decw = {"w1": dec[0].weight.detach(), "b1": dec[0].bias.detach(), "w2": dec[2].weight.detach(),
-            "b2": dec[2].bias.detach(), "w3": dec[4].weight.detach(), "b3": dec[4].bias.detach()}
-    decw = {k: v.float().contiguous() for k, v in decw.items()}
-    F32 = capi.BG_F32
-    out_dim = model.output_dim
+    chain = _linears(model.decoder)
     with engine.TIMERS.span("node_head"):
-        h1d, h2d, pred = _f32((n, 128), dev), _f32((n, 64), dev), _f32((n, out_dim), dev)
-        sgemm(cur.data, cur.code, 512, 1, decw["w1"], F32, 1, 512, n, 128, 512, h1d, F32, 128, bias=decw["b1"], relu=True)
-        sgemm(h1d, F32, 128, 1, decw["w2"], F32, 1, 128, n, 64, 128, h2d, F32, 64, bias=decw["b2"], relu=True)
-        sgemm(h2d, F32, 64, 1, decw["w3"], F32, 1, 64, n, out_dim, 64, pred, F32, out_dim, bias=decw["b3"])
-    sv.decw, sv.dec_in, sv.h1d, sv.h2d, sv.mlp, sv.raw = decw, cur, h1d, h2d, None, None
+        pred, xs = chain_forward(chain, cur)
+    _keep_head(sv, chain, xs, False)
     return pred
 
 
 def node_head_backward(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
     """Backward of `decoder(x)` over all n nodes: returns d(last layer output) [n, 512]."""
-    dev = dpred.device
-    F32 = capi.BG_F32
-    out_dim = model.output_dim
-    d, dec = sv.decw, model.decoder
-    h1d, h2d, x = sv.h1d, sv.h2d, sv.dec_in
     with engine.TIMERS.span("train_head_bwd"):
-        dw3, _ = grads.get(dec[4].weight); db3, _ = grads.get(dec[4].bias)
-        sgemm(dpred, F32, 1, out_dim, h2d, F32, 64, 1, out_dim, 64, n, dw3, F32, 64)
-        colsum(dpred, F32, n, out_dim, out_dim, db3)
-        dh2d = _f32((n, 64), dev)
-        sgemm(dpred, F32, out_dim, 1, d["w3"], F32, 64, 1, n, 64, out_dim, dh2d, F32, 64, mask=h2d, mask_ld=64)
-        dw2, _ = grads.get(dec[2].weight); db2, _ = grads.get(dec[2].bias)
-        sgemm(dh2d, F32, 1, 64, h1d, F32, 128, 1, 64, 128, n, dw2, F32, 128)
-        colsum(dh2d, F32, n, 64, 64, db2)
-        dh1d = _f32((n, 128), dev)
-        sgemm(dh2d, F32, 64, 1, d["w2"], F32, 128, 1, n, 128, 64, dh1d, F32, 128, mask=h1d, mask_ld=128)
-        dw1, _ = grads.get(dec[0].weight); db1, _ = grads.get(dec[0].bias)
-        sgemm(dh1d, F32, 1, 128, x.data, x.code, 512, 1, 128, 512, n, dw1, F32, 512)
-        colsum(dh1d, F32, n, 128, 128, db1)
-        dcur = Activation(n, 512, prec, dev)
-        sgemm(dh1d, F32, 128, 1, d["w1"], F32, 512, 1, n, 512, 128, dcur.data, dcur.code, 512)
-        dcur.refresh_split()
-    return dcur
+        return chain_backward(sv.head, sv.head_in, dpred, grads, dx=Activation(n, 512, prec, dpred.device))
 
 
 # ----------------------------------------------------------------------------- GraphSAGE
