@@ -41,7 +41,7 @@ EXPORTED_SYMBOLS = (
     "bg_sag_pool_backward", "bg_max_aggregate_backward", "bg_max_bwd_workspace_bytes",
     "bg_bn_batch_stats128", "bg_bn_act_forward128", "bg_sage_backward_rows128", "bg_pool_backward128",
     "bg_max_aggregate_backward128", "bg_wgrad128",
-    "bg_dropout_residual128", "bg_grad_mask128", "bg_segment_expand128", "bg_wgrad128_ld",
+    "bg_dropout_residual128", "bg_grad_mask128", "bg_segment_expand128", "bg_wgrad128_ld", "bg_node_head128",
 )
 
 
@@ -160,6 +160,7 @@ _SIGNATURES = {
     "bg_grad_mask128": (C.c_int, [_P, _P, _P, _P, C.c_int, _I64, C.c_float, C.c_uint64, _P]),
     "bg_segment_expand128": (C.c_int, [_P, _P, _I64, C.c_int, _P, C.c_int, _P]),
     "bg_wgrad128_ld": (C.c_int, [_P, _P, _P, C.c_int, _I64, _I32, _I64, _P, _P, _I64, _P, _I64, C.c_int, _P]),
+    "bg_node_head128": (C.c_int, [_P, C.c_int, _I64, _P, _P, _P, _P, _I32, _P, _P]),
 }
 
 
@@ -338,6 +339,12 @@ def pool_head128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b
                  pred, pooled_out, ws, ws_bytes, stream, nonfinite=None):
     _check(load().bg_pool_head128(x, dtype, n_nodes, graph_ptr, n_graphs, pool_mode, pre_w, pre_b, w1, b1, w2, b2,
                                   w3, b3, out_dim, pred, pooled_out, ws, ws_bytes, nonfinite, stream), "bg_pool_head128")
+
+
+def node_head128(x, dtype, n_rows, w1, b1, w2, b2, out_dim, out, stream):
+    """bg_node_head128: out [n_rows, out_dim] f32 = W2 relu(W1 x + b1) + b2 for x [n_rows, 128] of `dtype`, w1 [64, 128]
+    in the operand format of dtype, b1 / w2 / b2 f32."""
+    _check(load().bg_node_head128(x, dtype, n_rows, w1, b1, w2, b2, out_dim, out, stream), "bg_node_head128")
 
 
 def pool_block_flags(graph_ptr, n_graphs, n_nodes, keep, stream):

@@ -14,6 +14,7 @@
 #include "train.cuh"
 #include "sag_pool.cuh"
 #include "max_bwd.cuh"
+#include "node_head.cuh"
 
 namespace bg {
 
@@ -64,6 +65,7 @@ PFN_tensorMapEncodeTiled get_tensor_map_encoder() {
 }
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+static inline bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; }
 
 template <typename T>
 __global__ void k_cast_f32_16(const float* __restrict__ src, T* __restrict__ dst, int64_t n) {
@@ -999,6 +1001,39 @@ int bg_pool_head_blocks128(const void* x, int dtype, int64_t N, const int32_t* g
   return pool_head_blocks_impl("bg_pool_head_blocks128", kW128, x, dtype, N, graph_ptr, G, pool_mode, pre_w, pre_b, w1, b1,
                                w2, b2, w3, b3, out_dim, pred, pooled_out, block_sums, keep, workspace, workspace_bytes,
                                nonfinite_flag, stream_);
+}
+
+// ------------------------------------------------------------------ node-level head, hidden_channels = 128
+int bg_node_head128(const void* x, int dtype, int64_t n_rows, const void* w1, const float* b1, const float* w2,
+                    const float* b2, int32_t out_dim, float* out, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (dtype != BG_BF16 && dtype != BG_F16 && dtype != BG_F32) return fail(BG_ERR_INVALID, "bg_node_head128: bad dtype");
+  if (n_rows < 0) return fail(BG_ERR_INVALID, "bg_node_head128: n_rows < 0");
+  if (out_dim < 1 || out_dim > kNhMaxOut) return fail(BG_ERR_INVALID, "bg_node_head128: out_dim must be in 1..8");
+  if (!w1 || !b1 || !w2 || !b2 || !aligned16(w1) || !aligned4(b1) || !aligned4(w2) || !aligned4(b2))
+    return fail(BG_ERR_INVALID, "bg_node_head128: bad weight pointer (null, or w1 not 16-byte / b1, w2, b2 not 4-byte aligned)");
+  // x and out may be null only when there are no rows (an empty tensor has no storage)
+  if ((n_rows > 0 && (!x || !out)) || !aligned16(x) || !aligned4(out))
+    return fail(BG_ERR_INVALID, "bg_node_head128: bad x / out pointer (null, or x not 16-byte / out not 4-byte aligned)");
+  if (n_rows == 0) return BG_OK;
+  if (dtype == BG_F32) {
+    const int smem = (int)sizeof(NodeHeadSmem32);
+    static bool set = false;
+    if (!set) { BG_CUDA_OK(cudaFuncSetAttribute(k_node_head128_f32, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); set = true; }
+    const unsigned grid = (unsigned)min64(ceil_div64(n_rows, kNhRows32), (int64_t)sm_count() * 2);
+    k_node_head128_f32<<<grid, 256, smem, stream>>>(static_cast<const float*>(x), n_rows, static_cast<const float*>(w1),
+                                                    b1, w2, b2, out_dim, out);
+  } else {
+    const unsigned grid = (unsigned)min64(ceil_div64(n_rows, 16 * kNhWarps), (int64_t)sm_count() * 2);
+    if (dtype == BG_BF16)
+      k_node_head128_mma<__nv_bfloat16><<<grid, kNhWarps * 32, 0, stream>>>(
+          static_cast<const __nv_bfloat16*>(x), n_rows, static_cast<const __nv_bfloat16*>(w1), b1, w2, b2, out_dim, out);
+    else
+      k_node_head128_mma<__half><<<grid, kNhWarps * 32, 0, stream>>>(
+          static_cast<const __half*>(x), n_rows, static_cast<const __half*>(w1), b1, w2, b2, out_dim, out);
+  }
+  BG_LAUNCH_OK();
+  return BG_OK;
 }
 
 // ------------------------------------------------------------------ EA-GNN helpers

@@ -595,10 +595,28 @@ def pack_node_head(decoder, precision: str) -> Dict[str, object]:
             "w2": f32(decoder[2].weight), "b2": f32(decoder[2].bias), "w3": f32(decoder[4].weight), "b3": f32(decoder[4].bias)}
 
 
+def pack_node_head128(decoder, precision: str) -> Dict[str, torch.Tensor]:
+    """The 2-layer decoder Linear(128,64) ReLU Linear(64,out) of h <= 128 (Models/BuckGNN.py:41-65) for
+    bg_node_head128: W1 in the operand format of the model's storage format (fp16 / bf16; the exact fp32 weight for the
+    fp32-storage modes, whose kernel uses fp32 FMAs), b1, W2 and b2 in fp32."""
+    f32 = lambda t: t.detach().float().contiguous()
+    w1 = decoder[0].weight
+    code = PRECISION_FORMATS[precision][0]
+    return {"w1": f32(w1) if code == capi.BG_F32 else pack_linear(w1, precision).parts[0],
+            "b1": f32(decoder[0].bias), "w2": f32(decoder[2].weight), "b2": f32(decoder[2].bias)}
+
+
 def node_head(x: Activation, n: int, head: Dict[str, object], out_dim: int, cta_group: int = 2) -> torch.Tensor:
-    """decoder(x) for all n nodes -> [n, out_dim] f32."""
+    """decoder(x) for all n nodes -> [n, out_dim] f32.  128-wide rows (a hidden_channels = 128 model) run on
+    bg_node_head128 with `pack_node_head128`'s weights, 512-wide ones on the tensor-core GEMM and bg_sgemm."""
     dev = x.data.device
     s = _stream()
+    if x.data.shape[1] == 128:
+        out = torch.empty((n, out_dim), dtype=torch.float32, device=dev)
+        with TIMERS.span("node_head"):
+            capi.node_head128(x.data.data_ptr(), x.code, n, head["w1"].data_ptr(), head["b1"].data_ptr(),
+                              head["w2"].data_ptr(), head["b2"].data_ptr(), out_dim, out.data_ptr(), s)
+        return out
     h1 = Activation(n, 512, x.precision, dev)
     with TIMERS.span("node_head"):
         gemm512(_segments(x, head["w1"]), n, x.precision, h1, cta_group=cta_group, bias=head["b1_host"].data_ptr(), relu=True)

@@ -23,7 +23,10 @@ the environment); otherwise, and for what the 128-wide step does not cover, trai
 twin (narrow.py).  A 128-wide EA_GNN / EA_GNN_Shared model evaluates on the 128-wide kernels when
 `model.native128_eagnn` is set (default from BUCKGNN_NATIVE128_EAGNN=1), and trains on them when
 `model.native128_eagnn_train` is set (default from BUCKGNN_NATIVE128_EAGNN_TRAIN=1; train_eagnn.py at width 128);
-otherwise it trains as the twin.
+otherwise it trains as the twin.  Those flags cover graph-level heads.  Node-level heads (static_disp, static_stress,
+mode_shape) of the same eight models at 128 evaluate and train on the 128-wide kernels when `model.native128_node_head`
+is set (default from BUCKGNN_NATIVE128_NODE_HEAD=1; bg_node_head128 in eval), and otherwise run as the twin.  The
+SAGPooling variants and widths 64 / 256 always run as the twin.
 
 Extra, non-reference keywords: `train_precision` in {"tf32", "bf16", "fp16"} (storage of the training
 step's activations and activation gradients; default tf32 = fp32 storage), and `precision` in {"auto", "fp16", "bf16", "tf32", "fp32"}
@@ -64,6 +67,10 @@ NATIVE128_EAGNN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN", "0") not in 
 # width 128) instead of the twin.  Opt-in: BUCKGNN_NATIVE128_EAGNN_TRAIN=1 in the environment, or
 # `model.native128_eagnn_train = True`.
 NATIVE128_EAGNN_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN_TRAIN", "0") not in ("", "0")
+# node-level heads (static_disp, static_stress, mode_shape) of the models above at hidden_channels == 128: eval forward
+# and training step on the 128-wide kernels (bg_node_head128 in eval, bg_sgemm in training) instead of the twin.
+# Opt-in: BUCKGNN_NATIVE128_NODE_HEAD=1 in the environment, or `model.native128_node_head = True`.
+NATIVE128_NODE_HEAD_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_NODE_HEAD", "0") not in ("", "0")
 
 
 class SAGEConv(nn.Module):
@@ -174,6 +181,7 @@ class BuckGNN(nn.Module):
         self.native128_train = NATIVE128_TRAIN_DEFAULT         # hidden_channels 128: train on the 128-wide kernels (opt-in)
         self.native128_eagnn = NATIVE128_EAGNN_DEFAULT         # hidden_channels 128: EA-GNN eval on the 128-wide kernels (opt-in)
         self.native128_eagnn_train = NATIVE128_EAGNN_TRAIN_DEFAULT   # hidden_channels 128: EA-GNN training on them (opt-in)
+        self.native128_node_head = NATIVE128_NODE_HEAD_DEFAULT       # hidden_channels 128: node-level heads on them (opt-in)
         self.output_dim = output_dim = _output_dim(prediction_type, use_z_coord, use_rotations)
         h = hidden_channels
         cat_dec = pooling_layer == "supernode_with_pooling" and prediction_type == "buckling"
@@ -265,6 +273,8 @@ class BuckGNN(nn.Module):
         packs["dec"] = engine.pack_decoder(self.decoder, width)
         if self.prediction_type != "buckling" and self.hidden_channels >= 256:
             packs["node_head"] = engine.pack_node_head(self.decoder, prec)
+        elif self.prediction_type != "buckling" and width == 128:
+            packs["node_head"] = engine.pack_node_head128(self.decoder, prec)
         mpl = self.pooling_mpl.mlp[0]
         packs["pool_mlp"] = {"w": f32(mpl.weight), "b": f32(mpl.bias)}
         layers, seen = [], {}
@@ -340,9 +350,38 @@ class BuckGNN(nn.Module):
                 and self.model_name in _NATIVE128_EAGNN_MODELS and self.prediction_type == "buckling"
                 and self.pooling_layer in _POOLINGS)
 
+    def _runs_native128_node_head(self, training: Optional[bool] = None) -> bool:
+        """With `native128_node_head` on, eval and train-mode forwards of the GraphSAGE models `_runs_native128` covers
+        and of EA_GNN / EA_GNN_Shared at hidden_channels == 128 with a node-level head (static_disp, static_stress,
+        mode_shape) run on the 128-wide kernels; the other three flags leave them on the twin.  GraphSAGE eval needs
+        `fuse_aggregate` off, as in `_runs_native128`.  `training` overrides the module's mode."""
+        training = self.training if training is None else training
+        if (self.hidden_channels != 128 or not self.native128_node_head
+                or not ("static" in self.prediction_type or "mode_shape" in self.prediction_type)):
+            return False
+        if self.model_name in _NATIVE128_EAGNN_MODELS:
+            return True
+        return self.model_name in _NATIVE128_MODELS and (training or not self.fuse_aggregate)
+
     def forward(self, x, edge_index, edge_attr, batch=None, mask=None):
         self._check_supported(x)
         self._ran_native128 = False
+        if self._runs_native128_node_head():
+            if self.training:
+                from . import train
+                pred = train.forward_train(self, x, edge_index, batch, edge_attr=edge_attr)
+                self._pack_sig = None            # BatchNorm statistics changed: the next native eval forward repacks
+            else:
+                with torch.no_grad():
+                    if self.model_name in _NATIVE128_EAGNN_MODELS:
+                        pred = self._forward_cuda_eagnn(x, edge_index, edge_attr, batch, node_level=True, width=128)
+                    else:
+                        pred = self._forward_cuda(x, edge_index, batch, node_level=True, width=128)
+                self._ran_native128 = True
+            if "super" in self.pooling_layer:                # reference :518-524, as the twin returns it
+                is_real_node = x[:, -1] == 0
+                return pred[is_real_node], (batch[is_real_node] if batch is not None else None)
+            return pred, batch
         if self._runs_native128():
             with torch.no_grad():
                 if self.model_name in _NATIVE128_EAGNN_MODELS:
@@ -425,10 +464,12 @@ class BuckGNN(nn.Module):
         """Multi-GPU training (BASELINE.json configs[3]): all-reduce (mean) the gradients of this model's trainable
         parameters over `group`, bucketed per layer and overlapped with the backward pass (dist.GradSync).  Call once
         after `.to(device)`, on every rank; `loss.backward()` then leaves the REDUCED gradients in `.grad`."""
-        native128 = self.native128_train or (self.native128_eagnn_train and self.model_name in _NATIVE128_EAGNN_MODELS)
+        native128 = (self.native128_train or (self.native128_eagnn_train and self.model_name in _NATIVE128_EAGNN_MODELS)
+                     or self._runs_native128_node_head(training=True))
         if self.hidden_channels != 512 and not (self.hidden_channels == 128 and native128):
             raise NotImplementedError("buckgnn_b200: overlapped gradient sync is built for hidden_channels=512, and for "
-                                      "128 with native128_train (EA_GNN / EA_GNN_Shared: native128_eagnn_train) on; use "
+                                      "128 with native128_train (EA_GNN / EA_GNN_Shared: native128_eagnn_train; "
+                                      "node-level heads: native128_node_head) on; use "
                                       "dist.allreduce_gradients(model.parameters()) after backward() instead")
         from . import train
         from .dist import GradSync
@@ -474,7 +515,7 @@ class BuckGNN(nn.Module):
 
     def _forward_cuda_eagnn(self, x, edge_index, edge_attr, batch, node_level=False, width=512):
         """EA-GNN / "CustomGNN" path (reference :326-336, :375-387, GraphNetBlock :528-566).  `width` 128: a
-        hidden_channels = 128 model on the 128-wide kernels (graph-level head only)."""
+        hidden_channels = 128 model on the 128-wide kernels."""
         packs = self._packed(width)
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()

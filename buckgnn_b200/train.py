@@ -20,7 +20,7 @@ The encoder's first two Linears, the decoder and their gradients run on `bg_sgem
 Width: the step runs at the model's hidden_channels, 512 or 128 (`BuckGNN.native128_train`: a hidden_channels = 128
 model trains on its own 128-wide kernels -- bg_gemm128, bg_wgrad128 and the `*128` row kernels -- instead of the
 zero-padded 512-wide twin of narrow.py).  At 128 the encoder and decoder are the reference's 2-layer MLPs
-(Models/BuckGNN.py:41-65), all on bg_sgemm.
+(Models/BuckGNN.py:41-65), all on bg_sgemm.  Node-level heads train at 128 when `BuckGNN.native128_node_head` is on.
 
 Precision: `train_precision` in {"tf32" (default; fp32 storage), "bf16", "fp16"}: activations, saved tensors and
 gradients of activations are stored in that format, weight gradients and all reductions are fp32.
@@ -350,8 +350,9 @@ def node_head_forward_train(model, cur: Activation, sv) -> torch.Tensor:
     """Node-level heads (`static_disp`, `static_stress`, `mode_shape`): `decoder(x)` on every node
     (Models/BuckGNN.py:518-524; the caller drops the super-node rows) on bg_sgemm, its hidden layers kept for the
     backward pass."""
-    if len(model.decoder) != 5:
-        raise NotImplementedError("buckgnn_b200: node-level training needs the 3-layer decoder (hidden_channels >= 256)")
+    if len(model.decoder) != 5 and not model._runs_native128_node_head():
+        raise NotImplementedError("buckgnn_b200: node-level training needs the 3-layer decoder (hidden_channels >= 256), "
+                                  "or hidden_channels = 128 with native128_node_head on")
     chain = _linears(model.decoder)
     with engine.TIMERS.span("node_head"):
         pred, xs = chain_forward(chain, cur)
@@ -360,9 +361,10 @@ def node_head_forward_train(model, cur: Activation, sv) -> torch.Tensor:
 
 
 def node_head_backward(model, sv, dpred: torch.Tensor, n: int, prec: str, grads: GradStore) -> Activation:
-    """Backward of `decoder(x)` over all n nodes: returns d(last layer output) [n, 512]."""
+    """Backward of `decoder(x)` over all n nodes: returns d(last layer output) [n, hidden_channels]."""
     with engine.TIMERS.span("train_head_bwd"):
-        return chain_backward(sv.head, sv.head_in, dpred, grads, dx=Activation(n, 512, prec, dpred.device))
+        return chain_backward(sv.head, sv.head_in, dpred, grads,
+                              dx=Activation(n, model.hidden_channels, prec, dpred.device))
 
 
 # ----------------------------------------------------------------------------- GraphSAGE
@@ -380,8 +382,9 @@ class SageTrainFunction(torch.autograd.Function):
         W = model.hidden_channels                          # 512, or 128 (BuckGNN.native128_train)
         if W not in (512, 128):
             raise NotImplementedError(f"buckgnn_b200: the training step runs at width 512 or 128, not {W}")
-        if W == 128 and is_node_level(model):
-            raise NotImplementedError("buckgnn_b200: the 128-wide training step has graph-level heads only")
+        if W == 128 and is_node_level(model) and not model._runs_native128_node_head():
+            raise NotImplementedError("buckgnn_b200: the 128-wide training step has node-level heads only with "
+                                      "native128_node_head on")
         convs = model._sage_layers()
         L = len(convs)
         aggr = convs[0][0].aggr if convs else "mean"      # no layers: the default model_name (encoder -> pool -> decoder)

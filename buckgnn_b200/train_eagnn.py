@@ -283,8 +283,9 @@ class EAGNNTrainFunction(torch.autograd.Function):
         W = model.hidden_channels                          # 512, or 128 (BuckGNN.native128_eagnn_train)
         if W not in (512, 128):
             raise NotImplementedError(f"buckgnn_b200: the EA-GNN training step runs at width 512 or 128, not {W}")
-        if W == 128 and is_node_level(model):
-            raise NotImplementedError("buckgnn_b200: the 128-wide EA-GNN training step has graph-level heads only")
+        if W == 128 and is_node_level(model) and not model._runs_native128_node_head():
+            raise NotImplementedError("buckgnn_b200: the 128-wide EA-GNN training step has node-level heads only with "
+                                      "native128_node_head on")
         p_drop = float(model.dropout.p)
         pending = engine.begin_graph_index(edge_index, batch, n, key_row=0)       # GraphNetBlock aggregates on row (:553,561)
         blocks = _blocks(model)

@@ -314,6 +314,16 @@ int bg_pool_head_blocks128(const void* x, int dtype, int64_t n_nodes, const int3
                            float* pred, float* pooled_out, const float* block_sums, const uint8_t* keep,
                            void* workspace, size_t workspace_bytes, const int32_t* nonfinite_flag, void* stream);
 
+/* Node-level decoder of a hidden_channels = 128 model (Models/BuckGNN.py:518-524, h <= 128 decoder :41-65):
+ *   out[r] = W2 relu(W1 x[r] + b1) + b2      x [n_rows,128] of `dtype`, out [n_rows,out_dim] f32 row-major
+ * w1 [64,128] in the operand format of dtype (fp16 / bf16 for 16-bit x, f32 for f32 x), b1 [64] f32,
+ * w2 [out_dim,64] f32, b2 [out_dim] f32, 1 <= out_dim <= 8.  Rows are independent; no workspace, no atomics.
+ * 16-bit x: mma.sync with fp32 accumulation, the hidden layer kept in fp32 (not rounded); f32 x: fp32 FMAs.
+ * x and w1 16-byte aligned, b1 / w2 / b2 / out 4-byte aligned.  n_rows == 0 launches nothing (x and out may then be
+ * NULL).  The result is the same bit for bit from run to run. */
+int bg_node_head128(const void* x, int dtype, int64_t n_rows, const void* w1, const float* b1,
+                    const float* w2, const float* b2, int32_t out_dim, float* out, void* stream);
+
 /* ------------------------------------------------------------------ EA-GNN helpers
  * bg_expand_rowptr: row_of[i] = r with rowptr[r] <= i < rowptr[r+1], iota[i] = i   (i < E)
  *   (row ids of the CSR slots, and the identity "col" that turns bg_sage_aggregate into the
