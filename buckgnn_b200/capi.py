@@ -42,6 +42,7 @@ EXPORTED_SYMBOLS = (
     "bg_bn_batch_stats128", "bg_bn_act_forward128", "bg_sage_backward_rows128", "bg_pool_backward128",
     "bg_max_aggregate_backward128", "bg_wgrad128",
     "bg_dropout_residual128", "bg_grad_mask128", "bg_segment_expand128", "bg_wgrad128_ld", "bg_node_head128",
+    "bg_sag_select128", "bg_gather_rows128", "bg_sag_pool_backward128",
 )
 
 
@@ -162,6 +163,8 @@ _SIGNATURES = {
     "bg_wgrad128_ld": (C.c_int, [_P, _P, _P, C.c_int, _I64, _I32, _I64, _P, _P, _I64, _P, _I64, C.c_int, _P]),
     "bg_node_head128": (C.c_int, [_P, C.c_int, _I64, _P, _P, _P, _P, _I32, _P, _P]),
 }
+for _name in ("bg_sag_select", "bg_gather_rows", "bg_sag_pool_backward"):    # the 128-wide twins take the same arguments
+    _SIGNATURES[_name + "128"] = _SIGNATURES[_name]
 
 
 def library_path() -> str:
@@ -503,11 +506,27 @@ def sag_workspace_bytes(n_nodes: int, n_edges: int, n_graphs: int) -> int:
     return _query("bg_sag_workspace_bytes", n_nodes, n_edges, n_graphs)
 
 
+def _sag_select(fn, x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr, n_graphs, ratio,
+                edge_index, n_edges, score, new_id, perm, batch_out, score_out, new_graph_ptr, info, ws, ws_bytes, stream):
+    _check(getattr(load(), fn)(x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr,
+                               n_graphs, ratio, edge_index, n_edges, score, new_id, perm, batch_out, score_out,
+                               new_graph_ptr, info, ws, ws_bytes, stream), fn)
+
+
 def sag_select(x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr, n_graphs, ratio,
                edge_index, n_edges, score, new_id, perm, batch_out, score_out, new_graph_ptr, info, ws, ws_bytes, stream):
-    _check(load().bg_sag_select(x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr,
-                                n_graphs, ratio, edge_index, n_edges, score, new_id, perm, batch_out, score_out,
-                                new_graph_ptr, info, ws, ws_bytes, stream), "bg_sag_select")
+    _sag_select("bg_sag_select", x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr,
+                n_graphs, ratio, edge_index, n_edges, score, new_id, perm, batch_out, score_out, new_graph_ptr, info, ws,
+                ws_bytes, stream)
+
+
+def sag_select128(x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr, n_graphs, ratio,
+                  edge_index, n_edges, score, new_id, perm, batch_out, score_out, new_graph_ptr, info, ws, ws_bytes,
+                  stream):
+    """bg_sag_select128: sag_select for x [N, 128] and w_l / w_r [128]."""
+    _sag_select("bg_sag_select128", x, dtype, n_nodes, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign, graph_ptr,
+                n_graphs, ratio, edge_index, n_edges, score, new_id, perm, batch_out, score_out, new_graph_ptr, info, ws,
+                ws_bytes, stream)
 
 
 def sag_connect(edge_index, n_edges, n_nodes, new_id, n_edges_out, edge_index_out, kept_edge, ws, ws_bytes, stream):
@@ -519,6 +538,12 @@ def gather_rows(x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, strea
     _check(load().bg_gather_rows(x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, stream), "bg_gather_rows")
 
 
+def gather_rows128(x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, stream):
+    """bg_gather_rows128: out[r, 0:128] = x[row_index[r], 0:128] * row_scale[row_index[r]] (row_scale nullable)."""
+    _check(load().bg_gather_rows128(x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, stream),
+           "bg_gather_rows128")
+
+
 def index_invert(perm, n, out, stream):
     _check(load().bg_index_invert(perm, n, out, stream), "bg_index_invert")
 
@@ -527,11 +552,23 @@ def index_gather(table, idx, n, out, stream):
     _check(load().bg_index_gather(table, idx, n, out, stream), "bg_index_gather")
 
 
+def _sag_pool_backward(fn, dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign, rowptr_src, col_src,
+                       big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream):
+    _check(getattr(load(), fn)(dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign, rowptr_src,
+                               col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream), fn)
+
+
 def sag_pool_backward(dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign, rowptr_src, col_src,
                       big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream):
-    _check(load().bg_sag_pool_backward(dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign, rowptr_src,
-                                       col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream),
-           "bg_sag_pool_backward")
+    _sag_pool_backward("bg_sag_pool_backward", dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign,
+                       rowptr_src, col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream)
+
+
+def sag_pool_backward128(dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign, rowptr_src, col_src,
+                         big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream):
+    """bg_sag_pool_backward128: sag_pool_backward for dx_pooled / x / dx [*, 128] and w_l / w_r [128]."""
+    _sag_pool_backward("bg_sag_pool_backward128", dx_pooled, x, dtype, n_nodes, n_nodes_out, perm, new_id, score, sign,
+                       rowptr_src, col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream)
 
 
 def max_bwd_workspace_bytes(n_big_tgt: int, n_big_src: int) -> int:

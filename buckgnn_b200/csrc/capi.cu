@@ -1087,26 +1087,34 @@ int bg_sag_workspace_bytes(int64_t N, int64_t E, int64_t G, size_t* bytes_host) 
   return BG_OK;
 }
 
-int bg_sag_select(const void* x, int dtype, int64_t N, const int32_t* rowptr, const int32_t* col,
-                  const int32_t* big_rows, int32_t n_big, const float* w_l, const float* w_r, float bias, float sign,
-                  const int32_t* graph_ptr, int64_t G, float ratio, const int64_t* edge_index, int64_t E,
-                  float* score, int32_t* new_id, int32_t* perm, int64_t* batch_out, float* score_out,
-                  int32_t* new_graph_ptr, int32_t* info, void* workspace, size_t workspace_bytes, void* stream_) {
+// The 512- and 128-wide entry points share everything but the dot pass over x (k_sag_dots<T, width>)
+static int sag_select_impl(const char* fn, int width, const void* x, int dtype, int64_t N, const int32_t* rowptr,
+                           const int32_t* col, const int32_t* big_rows, int32_t n_big, const float* w_l, const float* w_r,
+                           float bias, float sign, const int32_t* graph_ptr, int64_t G, float ratio,
+                           const int64_t* edge_index, int64_t E, float* score, int32_t* new_id, int32_t* perm,
+                           int64_t* batch_out, float* score_out, int32_t* new_graph_ptr, int32_t* info, void* workspace,
+                           size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (N < 0 || E < 0 || G < 0 || N >= 0x7fffffffLL || E >= 0x7fffffffLL || G >= 0x7fffffffLL || n_big < 0)
-    return fail(BG_ERR_INVALID, "bg_sag_select: sizes out of range");
-  if (!(ratio > 0.f) || ratio > 1.f) return fail(BG_ERR_INVALID, "bg_sag_select: ratio must be in (0, 1]");
-  if (!info || !new_graph_ptr || !graph_ptr || !workspace) return fail(BG_ERR_INVALID, "bg_sag_select: null pointer");
+    return fail_in(BG_ERR_INVALID, fn, "sizes out of range");
+  if (!(ratio > 0.f) || ratio > 1.f) return fail_in(BG_ERR_INVALID, fn, "ratio must be in (0, 1]");
+  if (!info || !new_graph_ptr || !graph_ptr || !workspace) return fail_in(BG_ERR_INVALID, fn, "null pointer");
   if (N > 0 && (!x || !aligned16(x) || !rowptr || !w_l || !w_r || !score || !new_id || !perm || !batch_out || !score_out))
-    return fail(BG_ERR_INVALID, "bg_sag_select: null or misaligned pointer");
-  if ((E > 0 && (!edge_index || !col)) || (n_big > 0 && !big_rows)) return fail(BG_ERR_INVALID, "bg_sag_select: null pointer");
+    return fail_in(BG_ERR_INVALID, fn, "null or misaligned pointer");
+  if ((E > 0 && (!edge_index || !col)) || (n_big > 0 && !big_rows)) return fail_in(BG_ERR_INVALID, fn, "null pointer");
   SagWorkspace w = sag_workspace_layout(workspace, N, E, G);
-  if (workspace_bytes < w.bytes) return fail(BG_ERR_WORKSPACE, "bg_sag_select: workspace too small");
+  if (workspace_bytes < w.bytes) return fail_in(BG_ERR_WORKSPACE, fn, "workspace too small");
+  if (width != kHidden && dtype != BG_BF16 && dtype != BG_F16 && dtype != BG_F32)
+    return fail_in(BG_ERR_INVALID, fn, "bad dtype");                                    // (512: BG_BY_DTYPE)
   const int sms = sm_count();
   BG_CUDA_OK(cudaMemsetAsync(info, 0, sizeof(int32_t) * 2, stream));
   if (N > 0) {
     const unsigned grid = grid_for(N * 32, kSagWarps * 32, sms * 8);
-    BG_BY_DTYPE(dtype, (k_sag_dots<T><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(x), N, w_l, w_r, w.p, w.q)));
+    if (width == kHidden) {
+      BG_BY_DTYPE(dtype, (k_sag_dots<T, kHidden><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(x), N, w_l, w_r, w.p, w.q)));
+    } else {
+      BG_BY_DTYPE(dtype, (k_sag_dots<T, kW128><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(x), N, w_l, w_r, w.p, w.q)));
+    }
     BG_LAUNCH_OK();
     k_sag_score<true><<<grid_for(N * 8, 256, sms * 8), 256, 0, stream>>>(rowptr, col, w.p, w.q, bias, sign, N, score);
     BG_LAUNCH_OK();
@@ -1141,6 +1149,26 @@ int bg_sag_select(const void* x, int dtype, int64_t N, const int32_t* rowptr, co
   return BG_OK;
 }
 
+int bg_sag_select(const void* x, int dtype, int64_t N, const int32_t* rowptr, const int32_t* col,
+                  const int32_t* big_rows, int32_t n_big, const float* w_l, const float* w_r, float bias, float sign,
+                  const int32_t* graph_ptr, int64_t G, float ratio, const int64_t* edge_index, int64_t E,
+                  float* score, int32_t* new_id, int32_t* perm, int64_t* batch_out, float* score_out,
+                  int32_t* new_graph_ptr, int32_t* info, void* workspace, size_t workspace_bytes, void* stream_) {
+  return sag_select_impl("bg_sag_select", kHidden, x, dtype, N, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign,
+                         graph_ptr, G, ratio, edge_index, E, score, new_id, perm, batch_out, score_out, new_graph_ptr, info,
+                         workspace, workspace_bytes, stream_);
+}
+
+int bg_sag_select128(const void* x, int dtype, int64_t N, const int32_t* rowptr, const int32_t* col,
+                     const int32_t* big_rows, int32_t n_big, const float* w_l, const float* w_r, float bias, float sign,
+                     const int32_t* graph_ptr, int64_t G, float ratio, const int64_t* edge_index, int64_t E,
+                     float* score, int32_t* new_id, int32_t* perm, int64_t* batch_out, float* score_out,
+                     int32_t* new_graph_ptr, int32_t* info, void* workspace, size_t workspace_bytes, void* stream_) {
+  return sag_select_impl("bg_sag_select128", kW128, x, dtype, N, rowptr, col, big_rows, n_big, w_l, w_r, bias, sign,
+                         graph_ptr, G, ratio, edge_index, E, score, new_id, perm, batch_out, score_out, new_graph_ptr, info,
+                         workspace, workspace_bytes, stream_);
+}
+
 int bg_sag_connect(const int64_t* edge_index, int64_t E, int64_t N, const int32_t* new_id, int64_t E_out,
                    int64_t* edge_index_out, int32_t* kept_edge, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -1155,22 +1183,30 @@ int bg_sag_connect(const int64_t* edge_index, int64_t E, int64_t N, const int32_
   return BG_OK;
 }
 
-int bg_sag_pool_backward(const void* dx_pooled, const void* x, int dtype, int64_t N, int64_t N_out, const int32_t* perm,
-                         const int32_t* new_id, const float* score, float sign, const int32_t* rowptr_src,
-                         const int32_t* col_src, const int32_t* big_rows_src, int32_t n_big_src, const float* w_l,
-                         const float* w_r, void* dx, float* t, float* dpre, void* stream_) {
+static int sag_pool_backward_impl(const char* fn, int width, const void* dx_pooled, const void* x, int dtype, int64_t N,
+                                  int64_t N_out, const int32_t* perm, const int32_t* new_id, const float* score, float sign,
+                                  const int32_t* rowptr_src, const int32_t* col_src, const int32_t* big_rows_src,
+                                  int32_t n_big_src, const float* w_l, const float* w_r, void* dx, float* t, float* dpre,
+                                  void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (N < 0 || N_out < 0 || N_out > N || n_big_src < 0) return fail(BG_ERR_INVALID, "bg_sag_pool_backward: bad size");
+  if (N < 0 || N_out < 0 || N_out > N || n_big_src < 0) return fail_in(BG_ERR_INVALID, fn, "bad size");
   if (N == 0) return BG_OK;
   if (!x || !new_id || !score || !rowptr_src || !w_l || !w_r || !dx || !t || !dpre || !aligned16(x) || !aligned16(dx) ||
       (N_out > 0 && (!dx_pooled || !perm || !aligned16(dx_pooled))) || (n_big_src > 0 && !big_rows_src))
-    return fail(BG_ERR_INVALID, "bg_sag_pool_backward: null or misaligned pointer");
+    return fail_in(BG_ERR_INVALID, fn, "null or misaligned pointer");
+  if (width != kHidden && dtype != BG_BF16 && dtype != BG_F16 && dtype != BG_F32)
+    return fail_in(BG_ERR_INVALID, fn, "bad dtype");                                    // (512: BG_BY_DTYPE)
   const int sms = sm_count();
   BG_CUDA_OK(cudaMemsetAsync(dpre, 0, sizeof(float) * (size_t)N, stream));
   if (N_out > 0) {
     const unsigned grid = grid_for(N_out * 32, kSagWarps * 32, sms * 8);
-    BG_BY_DTYPE(dtype, (k_sag_bwd_rowdot<T><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(dx_pooled), static_cast<const T*>(x),
-                                                                               perm, score, sign, N_out, dpre)));
+    if (width == kHidden) {
+      BG_BY_DTYPE(dtype, (k_sag_bwd_rowdot<T, kHidden><<<grid, kSagWarps * 32, 0, stream>>>(
+                             static_cast<const T*>(dx_pooled), static_cast<const T*>(x), perm, score, sign, N_out, dpre)));
+    } else {
+      BG_BY_DTYPE(dtype, (k_sag_bwd_rowdot<T, kW128><<<grid, kSagWarps * 32, 0, stream>>>(
+                             static_cast<const T*>(dx_pooled), static_cast<const T*>(x), perm, score, sign, N_out, dpre)));
+    }
     BG_LAUNCH_OK();
   }
   k_sag_score<false><<<grid_for(N * 8, 256, sms * 8), 256, 0, stream>>>(rowptr_src, col_src, dpre, nullptr, 0.f, 1.f, N, t);
@@ -1180,10 +1216,31 @@ int bg_sag_pool_backward(const void* dx_pooled, const void* x, int dtype, int64_
     BG_LAUNCH_OK();
   }
   const unsigned grid = grid_for(N * 32, kSagWarps * 32, sms * 8);
-  BG_BY_DTYPE(dtype, (k_sag_bwd_dx<T><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(dx_pooled), new_id, score, t, dpre, w_l, w_r,
-                                                                         N, static_cast<T*>(dx))));
+  if (width == kHidden) {
+    BG_BY_DTYPE(dtype, (k_sag_bwd_dx<T, kHidden><<<grid, kSagWarps * 32, 0, stream>>>(
+                           static_cast<const T*>(dx_pooled), new_id, score, t, dpre, w_l, w_r, N, static_cast<T*>(dx))));
+  } else {
+    BG_BY_DTYPE(dtype, (k_sag_bwd_dx<T, kW128><<<grid, kSagWarps * 32, 0, stream>>>(
+                           static_cast<const T*>(dx_pooled), new_id, score, t, dpre, w_l, w_r, N, static_cast<T*>(dx))));
+  }
   BG_LAUNCH_OK();
   return BG_OK;
+}
+
+int bg_sag_pool_backward(const void* dx_pooled, const void* x, int dtype, int64_t N, int64_t N_out, const int32_t* perm,
+                         const int32_t* new_id, const float* score, float sign, const int32_t* rowptr_src,
+                         const int32_t* col_src, const int32_t* big_rows_src, int32_t n_big_src, const float* w_l,
+                         const float* w_r, void* dx, float* t, float* dpre, void* stream_) {
+  return sag_pool_backward_impl("bg_sag_pool_backward", kHidden, dx_pooled, x, dtype, N, N_out, perm, new_id, score, sign,
+                                rowptr_src, col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream_);
+}
+
+int bg_sag_pool_backward128(const void* dx_pooled, const void* x, int dtype, int64_t N, int64_t N_out, const int32_t* perm,
+                            const int32_t* new_id, const float* score, float sign, const int32_t* rowptr_src,
+                            const int32_t* col_src, const int32_t* big_rows_src, int32_t n_big_src, const float* w_l,
+                            const float* w_r, void* dx, float* t, float* dpre, void* stream_) {
+  return sag_pool_backward_impl("bg_sag_pool_backward128", kW128, dx_pooled, x, dtype, N, N_out, perm, new_id, score, sign,
+                                rowptr_src, col_src, big_rows_src, n_big_src, w_l, w_r, dx, t, dpre, stream_);
 }
 
 int bg_max_bwd_workspace_bytes(int32_t n_big_tgt, int32_t n_big_src, size_t* bytes_host) {
@@ -1239,19 +1296,36 @@ int bg_max_aggregate_backward128(const void* x, const void* agg, const void* dag
                                      workspace_bytes, stream_);
 }
 
-int bg_gather_rows(const void* x, int dtype, int64_t ldx, const int32_t* row_index, const float* row_scale,
-                   int64_t n_rows_out, void* out, int64_t ldo, void* stream_) {
+static int gather_rows_impl(const char* fn, int width, const void* x, int dtype, int64_t ldx, const int32_t* row_index,
+                            const float* row_scale, int64_t n_rows_out, void* out, int64_t ldo, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (n_rows_out < 0 || ldx < kHidden || ldo < kHidden) return fail(BG_ERR_INVALID, "bg_gather_rows: bad size");
+  if (n_rows_out < 0 || ldx < width || ldo < width) return fail_in(BG_ERR_INVALID, fn, "bad size");
   if (n_rows_out == 0) return BG_OK;
-  if (!x || !out || !row_index || !aligned16(x) || !aligned16(out)) return fail(BG_ERR_INVALID, "bg_gather_rows: null or misaligned pointer");
+  if (!x || !out || !row_index || !aligned16(x) || !aligned16(out)) return fail_in(BG_ERR_INVALID, fn, "null or misaligned pointer");
   const int esz = (dtype == BG_F32) ? 4 : 2;
-  if ((ldx * esz) % 16 != 0 || (ldo * esz) % 16 != 0) return fail(BG_ERR_INVALID, "bg_gather_rows: rows must be 16-byte aligned");
+  if ((ldx * esz) % 16 != 0 || (ldo * esz) % 16 != 0) return fail_in(BG_ERR_INVALID, fn, "rows must be 16-byte aligned");
+  if (width != kHidden && dtype != BG_BF16 && dtype != BG_F16 && dtype != BG_F32)
+    return fail_in(BG_ERR_INVALID, fn, "bad dtype");                                    // (512: BG_BY_DTYPE)
   const unsigned grid = grid_for(n_rows_out * 32, kSagWarps * 32, sm_count() * 8);
-  BG_BY_DTYPE(dtype, (k_gather_rows<T><<<grid, kSagWarps * 32, 0, stream>>>(static_cast<const T*>(x), ldx, row_index, row_scale,
-                                                                          n_rows_out, static_cast<T*>(out), ldo)));
+  if (width == kHidden) {
+    BG_BY_DTYPE(dtype, (k_gather_rows<T, kHidden><<<grid, kSagWarps * 32, 0, stream>>>(
+                           static_cast<const T*>(x), ldx, row_index, row_scale, n_rows_out, static_cast<T*>(out), ldo)));
+  } else {
+    BG_BY_DTYPE(dtype, (k_gather_rows<T, kW128><<<grid, kSagWarps * 32, 0, stream>>>(
+                           static_cast<const T*>(x), ldx, row_index, row_scale, n_rows_out, static_cast<T*>(out), ldo)));
+  }
   BG_LAUNCH_OK();
   return BG_OK;
+}
+
+int bg_gather_rows(const void* x, int dtype, int64_t ldx, const int32_t* row_index, const float* row_scale,
+                   int64_t n_rows_out, void* out, int64_t ldo, void* stream_) {
+  return gather_rows_impl("bg_gather_rows", kHidden, x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, stream_);
+}
+
+int bg_gather_rows128(const void* x, int dtype, int64_t ldx, const int32_t* row_index, const float* row_scale,
+                      int64_t n_rows_out, void* out, int64_t ldo, void* stream_) {
+  return gather_rows_impl("bg_gather_rows128", kW128, x, dtype, ldx, row_index, row_scale, n_rows_out, out, ldo, stream_);
 }
 
 int bg_index_invert(const int32_t* perm, int64_t n, int32_t* out, void* stream_) {

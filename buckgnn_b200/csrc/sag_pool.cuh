@@ -10,7 +10,8 @@
 // Kernels (all deterministic, no floating-point atomics):
 //   k_sag_dots        p = x . w_l, q = x . w_r  -- the 512 -> 1 SAGEConv is linear, so
 //                     w_l . (sum_j x_j) = sum_j (w_l . x_j): ONE pass over x [N,512] (HBM bound)
-//                     and a scalar neighbourhood sum instead of a 512-wide aggregation
+//                     and a scalar neighbourhood sum instead of a 512-wide aggregation (x [N,128] for a
+//                     hidden_channels = 128 model: the row kernels are templates on the row width)
 //   k_sag_score(_big) score_i = tanh(sign * (sum_{j -> i} p_j + b + q_i)) over the CSR keyed by target
 //   k_sag_plan        k_g = ceil(ratio * n_g); exclusive scans -> new graph offsets, rank-tile offsets
 //   k_sag_sort        graphs of up to 16384 nodes: one CTA per graph sorts 64-bit keys (order-preserving score
@@ -40,35 +41,32 @@ constexpr int kRankTileJ = 2048;                            // scores staged in 
 constexpr int kEdgeItemsPerBlock = 4096;                    // 1024 threads x 4 consecutive edges
 constexpr int kSagSortMax = 16384;                          // graphs up to this size sort in shared memory (128 KB of keys)
 
-template <typename T> BG_DEVINL void row_values(const T* row, int lane, float (&v)[16]) {
-  RowFrag<T> f;
-  f.load(row, lane);
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = 0.f;
-  f.template accumulate<BG_AGGR_SUM>(v);          // 0 + value: exact
-}
-
-template <typename T>
+// The four row kernels (k_sag_dots, k_gather_rows, k_sag_bwd_rowdot, k_sag_bwd_dx) are templates on the row width kW:
+// 512, or 128 for a hidden_channels = 128 model (the `bg_*128` entry points).  A warp owns a row, each lane
+// RowIO<T, kW>::kPer of its columns (train.cuh): 16 interleaved ones at 512, 4 consecutive ones at 128.
+template <typename T, int kW>
 __global__ void __launch_bounds__(kSagWarps * 32)
 k_sag_dots(const T* __restrict__ x, int64_t N, const float* __restrict__ w_l, const float* __restrict__ w_r,
            float* __restrict__ p, float* __restrict__ q) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
-  float wl[16], wr[16];
+  float wl[kPer], wr[kPer];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int c = RowFrag<T>::col_of(lane, i);
+  for (int i = 0; i < kPer; ++i) {
+    const int c = IO::col_of(lane, i);
     wl[i] = w_l[c];
     wr[i] = w_r[c];
   }
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   for (; r + n_warps < N; r += 2 * n_warps) {                 // two rows in flight per warp
-    float v0[16], v1[16];
-    row_values(x + (size_t)r * kHidden, lane, v0);
-    row_values(x + (size_t)(r + n_warps) * kHidden, lane, v1);
+    float v0[kPer], v1[kPer];
+    IO::load(x + (size_t)r * kW, lane, v0);
+    IO::load(x + (size_t)(r + n_warps) * kW, lane, v1);
     float a0 = 0.f, b0 = 0.f, a1 = 0.f, b1 = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < kPer; ++i) {
       a0 = fmaf(v0[i], wl[i], a0); b0 = fmaf(v0[i], wr[i], b0);
       a1 = fmaf(v1[i], wl[i], a1); b1 = fmaf(v1[i], wr[i], b1);
     }
@@ -76,11 +74,11 @@ k_sag_dots(const T* __restrict__ x, int64_t N, const float* __restrict__ w_l, co
     if (lane == 0) { p[r] = a0; q[r] = b0; p[r + n_warps] = a1; q[r + n_warps] = b1; }
   }
   for (; r < N; r += n_warps) {
-    float v0[16];
-    row_values(x + (size_t)r * kHidden, lane, v0);
+    float v0[kPer];
+    IO::load(x + (size_t)r * kW, lane, v0);
     float a0 = 0.f, b0 = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) { a0 = fmaf(v0[i], wl[i], a0); b0 = fmaf(v0[i], wr[i], b0); }
+    for (int i = 0; i < kPer; ++i) { a0 = fmaf(v0[i], wl[i], a0); b0 = fmaf(v0[i], wr[i], b0); }
     a0 = warp_sum(a0); b0 = warp_sum(b0);
     if (lane == 0) { p[r] = a0; q[r] = b0; }
   }
@@ -375,52 +373,56 @@ k_sag_edge_write(const int64_t* __restrict__ ei, int64_t E, int64_t N, const int
   }
 }
 
-// out[r, :] = x[idx[r], :] * scale[idx[r]]   (warp per row; scale nullable; idx[r] < 0 gives a zero row)
-template <typename T>
+// out[r, 0:kW] = x[idx[r], 0:kW] * scale[idx[r]]   (warp per row; scale nullable; idx[r] < 0 gives a zero row)
+template <typename T, int kW>
 __global__ void __launch_bounds__(kSagWarps * 32)
 k_gather_rows(const T* __restrict__ x, int64_t ldx, const int32_t* __restrict__ idx, const float* __restrict__ scale,
               int64_t n_out, T* __restrict__ out, int64_t ldo) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n_out; r += n_warps) {
     const int32_t src = idx[r];
-    float v[16];
+    float v[kPer];
     if (src < 0) {                                   // no source row: zeros (the gradient of a dropped edge)
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = 0.f;
+      for (int i = 0; i < kPer; ++i) v[i] = 0.f;
     } else {
-      row_values(x + (size_t)src * ldx, lane, v);
+      IO::load(x + (size_t)src * ldx, lane, v);
       if (scale) {
         const float s = scale[src];
 #pragma unroll
-        for (int i = 0; i < 16; ++i) v[i] *= s;
+        for (int i = 0; i < kPer; ++i) v[i] *= s;
       }
     }
-    RowFrag<T>::store(out + (size_t)r * ldo, lane, v);
+    IO::store(out + (size_t)r * ldo, lane, v);
   }
 }
 
 // ------------------------------------------------------------------ SAGPooling backward (training step)
 // Forward: s = tanh(sign * pre), pre_i = sum_{j -> i} w_l . x_j + b + w_r . x_i;  x'_r = x[perm[r]] * s[perm[r]].
-// Given dx' [N', 512]:
+// Given dx' [N', kW]:
 //   k_sag_bwd_rowdot   ds_r = dx'_r . x[perm[r]];  dpre[perm[r]] = sign * (1 - s^2) * ds_r   (dpre zero elsewhere)
 //   k_sag_score<false> t_j = sum_{i: j -> i} dpre_i  over the CSR keyed by SOURCE
 //   k_sag_bwd_dx       dx_j = [j kept] s_j dx'_{new_id[j]} + w_l t_j + w_r dpre_j
 // and on the host side dw_l = sum_j t_j x_j, dw_r = sum_j dpre_j x_j (bg_sgemm with M = 1), db = sum_j dpre_j (bg_colsum).
-template <typename T>
+template <typename T, int kW>
 __global__ void __launch_bounds__(kSagWarps * 32)
 k_sag_bwd_rowdot(const T* __restrict__ dxp, const T* __restrict__ x, const int32_t* __restrict__ perm,
                  const float* __restrict__ score, float sign, int64_t n_out, float* __restrict__ dpre) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n_out; r += n_warps) {
     const int32_t j = perm[r];
-    float a[16], b[16];
-    row_values(dxp + (size_t)r * kHidden, lane, a);
-    row_values(x + (size_t)j * kHidden, lane, b);
+    float a[kPer], b[kPer];
+    IO::load(dxp + (size_t)r * kW, lane, a);
+    IO::load(x + (size_t)j * kW, lane, b);
     float d = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) d = fmaf(a[i], b[i], d);
+    for (int i = 0; i < kPer; ++i) d = fmaf(a[i], b[i], d);
     d = warp_sum(d);
     if (lane == 0) {
       const float sj = score[j];
@@ -429,36 +431,38 @@ k_sag_bwd_rowdot(const T* __restrict__ dxp, const T* __restrict__ x, const int32
   }
 }
 
-template <typename T>
+template <typename T, int kW>
 __global__ void __launch_bounds__(kSagWarps * 32)
 k_sag_bwd_dx(const T* __restrict__ dxp, const int32_t* __restrict__ new_id, const float* __restrict__ score,
              const float* __restrict__ t, const float* __restrict__ dpre, const float* __restrict__ w_l,
              const float* __restrict__ w_r, int64_t N, T* __restrict__ dx) {
+  using IO = RowIO<T, kW>;
+  constexpr int kPer = IO::kPer;
   const int lane = threadIdx.x & 31;
-  float wl[16], wr[16];
+  float wl[kPer], wr[kPer];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int c = RowFrag<T>::col_of(lane, i);
+  for (int i = 0; i < kPer; ++i) {
+    const int c = IO::col_of(lane, i);
     wl[i] = w_l[c];
     wr[i] = w_r[c];
   }
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < N; j += n_warps) {
     const int32_t nid = new_id[j];
-    float v[16];
+    float v[kPer];
     if (nid >= 0) {
-      row_values(dxp + (size_t)nid * kHidden, lane, v);
+      IO::load(dxp + (size_t)nid * kW, lane, v);
       const float sj = score[j];
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] *= sj;
+      for (int i = 0; i < kPer; ++i) v[i] *= sj;
     } else {
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = 0.f;
+      for (int i = 0; i < kPer; ++i) v[i] = 0.f;
     }
     const float tj = t[j], dj = dpre[j];
 #pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = fmaf(wl[i], tj, fmaf(wr[i], dj, v[i]));
-    RowFrag<T>::store(dx + (size_t)j * kHidden, lane, v);
+    for (int i = 0; i < kPer; ++i) v[i] = fmaf(wl[i], tj, fmaf(wr[i], dj, v[i]));
+    IO::store(dx + (size_t)j * kW, lane, v);
   }
 }
 

@@ -772,7 +772,7 @@ def gnblock_layer(x: Activation, e: Activation, buf: GNBlockBuffers, idx: GraphI
 @dataclass
 class SagPoolResult:
     """What PyG `SAGPooling.forward` returns (Models/BuckGNN.py:365-367, 502-504), plus the index maps."""
-    x: Optional[Activation]       # [N', 512] = x[perm] * score[perm]
+    x: Optional[Activation]       # [N', width] = x[perm] * score[perm]   (width 512, or 128: bg_*128)
     edge_index: torch.Tensor      # [2, E'] int64, relabelled, original edge order
     batch: torch.Tensor           # [N'] int64
     perm: torch.Tensor            # [N'] int32: old node id of each kept row
@@ -803,8 +803,10 @@ def sag_pool(x: Activation, csr_by_target: GraphIndex, graph_ptr: torch.Tensor, 
              edge_index: torch.Tensor, w: Dict[str, object], sign: float = 1.0, want_kept_edges: bool = False) -> SagPoolResult:
     """SAGPooling on the device: score GNN + per-graph top-k + row gather + edge filter.  Two result words
     (N', E') come back to the host through pinned memory -- PyG syncs at the same place (`num_nodes.max().item()`
-    inside `topk`)."""
+    inside `topk`).  The row width of `x` picks the kernels: 512, or 128 (bg_sag_select128 / bg_gather_rows128)."""
     dev = x.data.device
+    width = x.data.shape[1]
+    select, gather = (capi.sag_select128, capi.gather_rows128) if width == 128 else (capi.sag_select, capi.gather_rows)
     n, g = csr_by_target.n_nodes, int(n_graphs)
     edge_index = edge_index.contiguous()
     e = edge_index.shape[1]
@@ -820,23 +822,22 @@ def sag_pool(x: Activation, csr_by_target: GraphIndex, graph_ptr: torch.Tensor, 
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     idx = csr_by_target
     with TIMERS.span("sag_select"):
-        capi.sag_select(x.data.data_ptr(), x.code, n, idx.rowptr.data_ptr(), idx.col.data_ptr(), idx.big_rows.data_ptr(),
-                        idx.n_big, w["w_l"].data_ptr(), w["w_r"].data_ptr(), w["bias"], float(sign),
-                        graph_ptr.data_ptr(), g, w["ratio"], edge_index.data_ptr(), e,
-                        score.data_ptr(), new_id.data_ptr(), perm.data_ptr(), batch_out.data_ptr(), score_sel.data_ptr(),
-                        new_ptr.data_ptr(), info.data_ptr(), ws.data_ptr(), ws_bytes, s)
+        select(x.data.data_ptr(), x.code, n, idx.rowptr.data_ptr(), idx.col.data_ptr(), idx.big_rows.data_ptr(),
+               idx.n_big, w["w_l"].data_ptr(), w["w_r"].data_ptr(), w["bias"], float(sign),
+               graph_ptr.data_ptr(), g, w["ratio"], edge_index.data_ptr(), e,
+               score.data_ptr(), new_id.data_ptr(), perm.data_ptr(), batch_out.data_ptr(), score_sel.data_ptr(),
+               new_ptr.data_ptr(), info.data_ptr(), ws.data_ptr(), ws_bytes, s)
     host = torch.zeros(2, dtype=torch.int32).pin_memory()
     capi.publish_words(info.data_ptr(), host.data_ptr(), 2, s)
     done = torch.cuda.Event()
     done.record()
     done.synchronize()
     n2, e2 = host.tolist()
-    x_new = Activation(n2, 512, x.precision, dev)
+    x_new = Activation(n2, width, x.precision, dev)
     ei_new = torch.empty((2, e2), dtype=torch.int64, device=dev)
     kept = torch.empty(max(e2, 1), **i32) if want_kept_edges else None
     with TIMERS.span("sag_connect"):
-        capi.gather_rows(x.data.data_ptr(), x.code, x.data.shape[1], perm.data_ptr(), score.data_ptr(), n2,
-                         x_new.data.data_ptr(), 512, s)
+        gather(x.data.data_ptr(), x.code, width, perm.data_ptr(), score.data_ptr(), n2, x_new.data.data_ptr(), width, s)
         x_new.refresh_split()
         capi.sag_connect(edge_index.data_ptr(), e, n, new_id.data_ptr(), e2, ei_new.data_ptr(), _p(kept),
                          ws.data_ptr(), ws_bytes, s)
@@ -861,12 +862,14 @@ def edge_slot_map(idx_old: GraphIndex, idx_new: GraphIndex, kept_edge: torch.Ten
 
 def regather_edge_rows(e: Activation, idx_old: GraphIndex, idx_new: GraphIndex, kept_edge: torch.Tensor) -> Activation:
     """Edge features of the kept edges, moved from the old CSR slot order to the new one (EAGNN_SAG:
-    `edge_attr[mask]` of PyG filter_adj, for edge tensors that live in CSR order)."""
+    `edge_attr[mask]` of PyG filter_adj, for edge tensors that live in CSR order), at the row width of `e`."""
     e_new = idx_new.n_edges
-    out = Activation(max(e_new, 1), 512, e.precision, e.data.device)
+    width = e.data.shape[1]
+    out = Activation(max(e_new, 1), width, e.precision, e.data.device)
     if e_new == 0:
         return out
     slot = edge_slot_map(idx_old, idx_new, kept_edge)
-    capi.gather_rows(e.data.data_ptr(), e.code, e.data.shape[1], slot.data_ptr(), None, e_new, out.data.data_ptr(), 512, _stream())
+    gather = capi.gather_rows128 if width == 128 else capi.gather_rows
+    gather(e.data.data_ptr(), e.code, width, slot.data_ptr(), None, e_new, out.data.data_ptr(), width, _stream())
     out.refresh_split()
     return out

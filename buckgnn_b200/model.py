@@ -26,7 +26,9 @@ twin (narrow.py).  A 128-wide EA_GNN / EA_GNN_Shared model evaluates on the 128-
 otherwise it trains as the twin.  Those flags cover graph-level heads.  Node-level heads (static_disp, static_stress,
 mode_shape) of the same eight models at 128 evaluate and train on the 128-wide kernels when `model.native128_node_head`
 is set (default from BUCKGNN_NATIVE128_NODE_HEAD=1; bg_node_head128 in eval), and otherwise run as the twin.  The
-SAGPooling variants and widths 64 / 256 always run as the twin.
+SAGPooling variants GraphSAGE_SAG / EAGNN_SAG at 128 evaluate (every head the 512-wide path has) and train (the
+eigenvalue head) on the 128-wide kernels when `model.native128_sag` is set (default from BUCKGNN_NATIVE128_SAG=1), and
+otherwise run as the twin.  Widths 64 / 256 always run as the twin.
 
 Extra, non-reference keywords: `train_precision` in {"tf32", "bf16", "fp16"} (storage of the training
 step's activations and activation gradients; default tf32 = fp32 storage), and `precision` in {"auto", "fp16", "bf16", "tf32", "fp32"}
@@ -71,6 +73,11 @@ NATIVE128_EAGNN_TRAIN_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_EAGNN_TRAIN", 
 # and training step on the 128-wide kernels (bg_node_head128 in eval, bg_sgemm in training) instead of the twin.
 # Opt-in: BUCKGNN_NATIVE128_NODE_HEAD=1 in the environment, or `model.native128_node_head = True`.
 NATIVE128_NODE_HEAD_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_NODE_HEAD", "0") not in ("", "0")
+# the SAGPooling variants at hidden_channels == 128: eval forward (graph- and node-level heads) and the eigenvalue-head
+# training step on the 128-wide kernels (bg_sag_select128 and friends) instead of the twin.
+# Opt-in: BUCKGNN_NATIVE128_SAG=1 in the environment, or `model.native128_sag = True`.
+_SAG_MODELS = ("GraphSAGE_SAG", "EAGNN_SAG")
+NATIVE128_SAG_DEFAULT = os.environ.get("BUCKGNN_NATIVE128_SAG", "0") not in ("", "0")
 
 
 class SAGEConv(nn.Module):
@@ -182,6 +189,7 @@ class BuckGNN(nn.Module):
         self.native128_eagnn = NATIVE128_EAGNN_DEFAULT         # hidden_channels 128: EA-GNN eval on the 128-wide kernels (opt-in)
         self.native128_eagnn_train = NATIVE128_EAGNN_TRAIN_DEFAULT   # hidden_channels 128: EA-GNN training on them (opt-in)
         self.native128_node_head = NATIVE128_NODE_HEAD_DEFAULT       # hidden_channels 128: node-level heads on them (opt-in)
+        self.native128_sag = NATIVE128_SAG_DEFAULT                   # hidden_channels 128: the SAGPooling variants on them (opt-in)
         self.output_dim = output_dim = _output_dim(prediction_type, use_z_coord, use_rotations)
         h = hidden_channels
         cat_dec = pooling_layer == "supernode_with_pooling" and prediction_type == "buckling"
@@ -303,8 +311,8 @@ class BuckGNN(nn.Module):
         if self.model_name in ("GraphSAGE_SAG", "EAGNN_SAG"):
             packs["sag_pool"] = engine.pack_sag_pool(self.pool)
         if self.model_name == "EAGNN_SAG":
-            packs["gn1"] = [engine.pack_gnblock(b, prec) for b in self.gnn_layers_1]
-            packs["gn2"] = [engine.pack_gnblock(b, prec) for b in self.gnn_layers_2]
+            packs["gn1"] = [engine.pack_gnblock(b, prec, width=width) for b in self.gnn_layers_1]
+            packs["gn2"] = [engine.pack_gnblock(b, prec, width=width) for b in self.gnn_layers_2]
         self._packs, self._pack_sig = packs, sig
         return packs
 
@@ -363,6 +371,18 @@ class BuckGNN(nn.Module):
             return True
         return self.model_name in _NATIVE128_MODELS and (training or not self.fuse_aggregate)
 
+    def _runs_native128_sag(self, training: Optional[bool] = None) -> bool:
+        """With `native128_sag` on, GraphSAGE_SAG / EAGNN_SAG at hidden_channels == 128 run on the 128-wide kernels: eval
+        forwards with every head the 512-wide path has (graph-level heads with the six poolings, node-level heads), and
+        train-mode forwards with the eigenvalue head (the only one the SAGPooling variants train with).  The other four
+        flags leave them on the twin.  `training` overrides the module's mode."""
+        training = self.training if training is None else training
+        if self.hidden_channels != 128 or not self.native128_sag or self.model_name not in _SAG_MODELS:
+            return False
+        graph_level = self.prediction_type == "buckling" and self.pooling_layer in _POOLINGS
+        node_level = "static" in self.prediction_type or "mode_shape" in self.prediction_type
+        return graph_level or (node_level and not training)
+
     def forward(self, x, edge_index, edge_attr, batch=None, mask=None):
         self._check_supported(x)
         self._ran_native128 = False
@@ -395,6 +415,15 @@ class BuckGNN(nn.Module):
             pred = train.forward_train(self, x, edge_index, batch, edge_attr=edge_attr)
             self._pack_sig = None                # BatchNorm statistics changed: the next native eval forward repacks
             return pred.squeeze(), batch
+        if self._runs_native128_sag():
+            if self.training:
+                from . import train
+                pred = train.forward_train(self, x, edge_index, batch, edge_attr=edge_attr)
+                self._pack_sig = None            # BatchNorm statistics changed: the next native eval forward repacks
+                return pred.squeeze(), self.last_pool.batch         # `batch` was reassigned by self.pool (:365, :502)
+            out = self._eval_sag(x, edge_index, edge_attr, batch, width=128)
+            self._ran_native128 = True
+            return out
         if self.hidden_channels != 512:
             if self.training and getattr(self, "_grad_sync", None) is not None:
                 # the twin's parameters are not the module's own: the installed GradSync would never see a gradient
@@ -434,15 +463,9 @@ class BuckGNN(nn.Module):
                     return pred[is_real_node], (batch[is_real_node] if batch is not None else None)
                 return pred, batch
             return pred.squeeze(), batch
+        if self.model_name in _SAG_MODELS:
+            return self._eval_sag(x, edge_index, edge_attr, batch)
         with torch.no_grad():
-            if self.model_name in ("GraphSAGE_SAG", "EAGNN_SAG"):
-                if node_level and "super" in self.pooling_layer:
-                    # the reference indexes the POOLED x with the un-pooled is_real_node mask here (:518-521)
-                    raise IndexError("The shape of the mask (is_real_node over all nodes) does not match the pooled node "
-                                     "tensor (same failure as the reference, Models/BuckGNN.py:521 after SAGPooling)")
-                fwd = self._forward_cuda_sag if self.model_name == "GraphSAGE_SAG" else self._forward_cuda_eagnn_sag
-                pred, pooled_batch = fwd(x, edge_index, edge_attr, batch, node_level)
-                return (pred if node_level else pred.squeeze()), pooled_batch      # `batch` was reassigned by self.pool (:365, :502)
             if self.model_name in ("EA_GNN", "EA_GNN_Shared"):
                 pred = self._forward_cuda_eagnn(x, edge_index, edge_attr, batch, node_level)
             else:
@@ -465,12 +488,13 @@ class BuckGNN(nn.Module):
         parameters over `group`, bucketed per layer and overlapped with the backward pass (dist.GradSync).  Call once
         after `.to(device)`, on every rank; `loss.backward()` then leaves the REDUCED gradients in `.grad`."""
         native128 = (self.native128_train or (self.native128_eagnn_train and self.model_name in _NATIVE128_EAGNN_MODELS)
-                     or self._runs_native128_node_head(training=True))
+                     or self._runs_native128_node_head(training=True)
+                     or self._runs_native128_sag(training=True))
         if self.hidden_channels != 512 and not (self.hidden_channels == 128 and native128):
             raise NotImplementedError("buckgnn_b200: overlapped gradient sync is built for hidden_channels=512, and for "
                                       "128 with native128_train (EA_GNN / EA_GNN_Shared: native128_eagnn_train; "
-                                      "node-level heads: native128_node_head) on; use "
-                                      "dist.allreduce_gradients(model.parameters()) after backward() instead")
+                                      "node-level heads: native128_node_head; GraphSAGE_SAG / EAGNN_SAG: native128_sag) "
+                                      "on; use dist.allreduce_gradients(model.parameters()) after backward() instead")
         from . import train
         from .dist import GradSync
         self._grad_sync = GradSync(train.trainable_parameters(self), next(self.parameters()).device, group)
@@ -594,17 +618,37 @@ class BuckGNN(nn.Module):
         return pred
 
     # ------------------------------------------------------------------ SAGPooling variants (SURVEY.md section 8 row f4)
-    def _tail(self, cur, idx, packs, node_level, cg):
+    def _eval_sag(self, x, edge_index, edge_attr, batch, width=512):
+        """Eval forward of GraphSAGE_SAG / EAGNN_SAG at `width` (512, or 128: a hidden_channels = 128 model on the
+        128-wide kernels): `(pred, pooled batch)`."""
+        node_level = "static" in self.prediction_type or "mode_shape" in self.prediction_type
+        if node_level and "super" in self.pooling_layer:
+            # the reference indexes the POOLED x with the un-pooled is_real_node mask here (:518-521)
+            raise IndexError("The shape of the mask (is_real_node over all nodes) does not match the pooled node "
+                             "tensor (same failure as the reference, Models/BuckGNN.py:521 after SAGPooling)")
+        fwd = self._forward_cuda_sag if self.model_name == "GraphSAGE_SAG" else self._forward_cuda_eagnn_sag
+        with torch.no_grad():
+            pred, pooled_batch = fwd(x, edge_index, edge_attr, batch, node_level, width=width)
+        return (pred if node_level else pred.squeeze()), pooled_batch      # `batch` was reassigned by self.pool (:365, :502)
+
+    def _tail(self, cur, idx, packs, node_level, cg, nonfinite=None):
         if node_level:
             return engine.node_head(cur, idx.n_nodes, packs["node_head"], self.output_dim, cg)
         pre = packs["pool_mlp"] if self.pooling_layer in ("mlp", "mlp_no_super") else None
-        pred, _ = engine.pool_head(cur, idx, packs["dec"], self.output_dim, pooling=self.pooling_layer, pre=pre)
+        pred, _ = engine.pool_head(cur, idx, packs["dec"], self.output_dim, pooling=self.pooling_layer, pre=pre,
+                                   nonfinite=nonfinite)
         return pred
 
-    def _forward_cuda_sag(self, x, edge_index, edge_attr, batch, node_level=False):
+    def _sag_nonfinite_flag(self, device, width):
+        """The 128-wide path keeps a fresh nonfinite flag for `check_finite()`, as the other 128-wide forwards do; the
+        512-wide path (and with it the twin) runs without one, as it always has."""
+        return self._new_nonfinite_flag(device) if width == 128 else None
+
+    def _forward_cuda_sag(self, x, edge_index, edge_attr, batch, node_level=False, width=512):
         """`GraphSAGE_SAG` (reference :190-217, :493-511): num_layers // 2 SAGE('add') layers, SAGPooling(0.5),
-        the remaining layers on the pooled graph, every layer after the first with a skip."""
-        packs = self._packed()
+        the remaining layers on the pooled graph, every layer after the first with a skip.  `width` 128: a
+        hidden_channels = 128 model on the 128-wide kernels."""
+        packs = self._packed(width)
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         n = x.shape[0]
@@ -612,15 +656,16 @@ class BuckGNN(nn.Module):
         layers = packs["layers"]
         n_before = len(self.sage_layers_1)
         folded = packs["layer0_folded"] if n_before > 0 else None
-        cur = Activation(n, 512, prec, x.device)
+        flag = self._sag_nonfinite_flag(x.device, width)
+        cur = Activation(n, width, prec, x.device)
         if folded is not None:
-            h = engine.encoder_hidden(x, packs["enc"], prec)
+            h = engine.encoder_hidden(x, packs["enc"], prec, nonfinite=flag)
         else:
-            engine.encoder_forward(x, packs["enc"], packs["enc_w3"], prec, cur, cg)
+            engine.encoder_forward(x, packs["enc"], packs["enc_w3"], prec, cur, cg, nonfinite=flag)
         idx = pending.finish()
         if n_before > 0:
-            nxt = Activation(n, 512, prec, x.device)
-            agg = Activation(n, 512, prec, x.device)
+            nxt = Activation(n, width, prec, x.device)
+            agg = Activation(n, width, prec, x.device)
             for i in range(n_before):
                 if i == 0 and folded is not None:
                     engine.sage_layer0_folded(h, nxt, idx, folded, aggr="add", normalize=True, relu=True, cta_group=cg)
@@ -634,18 +679,18 @@ class BuckGNN(nn.Module):
         idx2 = engine.build_graph_index(pooled.edge_index, pooled.batch, pooled.n_nodes)
         cur = pooled.x
         n2 = pooled.n_nodes
-        nxt = Activation(n2, 512, prec, x.device)
-        agg = Activation(n2, 512, prec, x.device)
+        nxt = Activation(n2, width, prec, x.device)
+        agg = Activation(n2, width, prec, x.device)
         for layer in layers[n_before:]:
             engine.sage_layer(cur, agg, nxt, idx2, layer, aggr="add", normalize=True, relu=True, residual=True,
                               cta_group=cg)
             cur, nxt = nxt, cur
-        return self._tail(cur, idx2, packs, node_level, cg), pooled.batch
+        return self._tail(cur, idx2, packs, node_level, cg, flag), pooled.batch
 
-    def _forward_cuda_eagnn_sag(self, x, edge_index, edge_attr, batch, node_level=False):
+    def _forward_cuda_eagnn_sag(self, x, edge_index, edge_attr, batch, node_level=False, width=512):
         """`EAGNN_SAG` (reference :219-244, :354-373): GraphNetBlocks around a SAGPooling; the pooled edge features are
-        the rows of the kept edges."""
-        packs = self._packed()
+        the rows of the kept edges.  `width` 128: a hidden_channels = 128 model on the 128-wide kernels."""
+        packs = self._packed(width)
         prec, cg = self.precision, self.cta_group
         x = x.detach().to(torch.float32).contiguous()
         if not edge_attr.is_cuda:
@@ -654,18 +699,19 @@ class BuckGNN(nn.Module):
         n = x.shape[0]
         pending = engine.begin_graph_index(edge_index, batch, n, key_row=0)       # GraphNetBlock direction (:553, :561)
         pending_t = engine.begin_graph_index(edge_index, None, n, key_row=1)      # SAGEConv direction of the score GNN
-        cur = Activation(n, 512, prec, x.device)
-        engine.encoder_forward(x, packs["enc"], packs["enc_w3"], prec, cur, cg)
+        flag = self._sag_nonfinite_flag(x.device, width)
+        cur = Activation(n, width, prec, x.device)
+        engine.encoder_forward(x, packs["enc"], packs["enc_w3"], prec, cur, cg, nonfinite=flag)
         idx = pending.finish()
         idx_t = pending_t.finish()
         ne = idx.n_edges
-        e = Activation(max(ne, 1), 512, prec, x.device)
+        e = Activation(max(ne, 1), width, prec, x.device)
         if ne > 0:
             engine.encoder_forward(edge_attr, packs["edge_enc"], packs["edge_enc_w3"], prec, e, cg,
-                                   row_gather=idx.perm[:ne])
+                                   row_gather=idx.perm[:ne], nonfinite=flag)
         if packs["gn1"]:
             ex = engine.edge_extras(idx, prec)
-            buf = engine.GNBlockBuffers(n, ne, prec, x.device)
+            buf = engine.GNBlockBuffers(n, ne, prec, x.device, width)
             for i, w in enumerate(packs["gn1"]):
                 cur, e_next = engine.gnblock_layer(cur, e, buf, idx, ex, w, skip=(i > 0), need_edges_out=True, cta_group=cg)
                 e = e_next
@@ -677,10 +723,10 @@ class BuckGNN(nn.Module):
         cur = pooled.x
         n2, ne2 = pooled.n_nodes, idx2.n_edges
         ex2 = engine.edge_extras(idx2, prec)
-        buf2 = engine.GNBlockBuffers(n2, ne2, prec, x.device)
+        buf2 = engine.GNBlockBuffers(n2, ne2, prec, x.device, width)
         last = len(packs["gn2"]) - 1
         for i, w in enumerate(packs["gn2"]):
             cur, e_next = engine.gnblock_layer(cur, e, buf2, idx2, ex2, w, skip=True, need_edges_out=(i < last), cta_group=cg)
             if e_next is not None:
                 e = e_next
-        return self._tail(cur, idx2, packs, node_level, cg), pooled.batch
+        return self._tail(cur, idx2, packs, node_level, cg, flag), pooled.batch

@@ -5,9 +5,10 @@ The reference's shipped configurations use `hidden_channels=128` (`TRAIN_FINAL.p
 model with a graph-level head runs on its own 128-wide kernels (`BuckGNN._forward_cuda(width=128)`, bg_gemm128), and so
 does that of EA_GNN / EA_GNN_Shared when `native128_eagnn` is on (`BuckGNN._forward_cuda_eagnn(width=128)`,
 bg_gemm128_gathered).  Node-level heads of those models run 128 wide, in eval and training, when `native128_node_head`
-is on (bg_node_head128 in eval).  What has no narrow kernels -- EA-GNN by default, the SAGPooling variants, node-level
-heads without that flag and widths 64 / 256 -- and training without `native128_train` (EA_GNN / EA_GNN_Shared:
-`native128_eagnn_train`) runs as the model's zero-padded 512-wide twin:
+is on (bg_node_head128 in eval), and so do GraphSAGE_SAG / EAGNN_SAG when `native128_sag` is on (eval with every head,
+training with the eigenvalue head; bg_sag_select128).  What has no narrow kernels -- EA-GNN by default, the SAGPooling
+variants and node-level heads without their flags, widths 64 / 256 -- and training without `native128_train`
+(EA_GNN / EA_GNN_Shared: `native128_eagnn_train`) runs as the model's zero-padded 512-wide twin:
 
 * every `[h, h]` weight sits in the top-left corner of a `[512, 512]` one, biases / BatchNorm affine terms are padded
   with zeros (running_var with ones): padded activation columns are exactly 0 through Linear, L2-normalize (the norm

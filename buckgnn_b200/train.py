@@ -21,6 +21,7 @@ Width: the step runs at the model's hidden_channels, 512 or 128 (`BuckGNN.native
 model trains on its own 128-wide kernels -- bg_gemm128, bg_wgrad128 and the `*128` row kernels -- instead of the
 zero-padded 512-wide twin of narrow.py).  At 128 the encoder and decoder are the reference's 2-layer MLPs
 (Models/BuckGNN.py:41-65), all on bg_sgemm.  Node-level heads train at 128 when `BuckGNN.native128_node_head` is on.
+GraphSAGE_SAG (`SagTrainFunction`) runs at the model's width too: at 128 when `BuckGNN.native128_sag` is on.
 
 Precision: `train_precision` in {"tf32" (default; fp32 storage), "bf16", "fp16"}: activations, saved tensors and
 gradients of activations are stored in that format, weight gradients and all reductions are fp32.
@@ -546,27 +547,28 @@ class SageTrainFunction(torch.autograd.Function):
 def _sag_layer_forward(conv, bn, cur: Activation, idx, prec: str, bias_host, residual: bool, p_drop: float, seed_i: int,
                        ws, ws_bytes, ones, zeros):
     """One layer of the GraphSAGE_SAG loops (Models/BuckGNN.py:494-511): x = dropout(relu(bn(conv(x)))), then
-    `x + identity` -- the skip is added AFTER the dropout here, unlike the plain variants."""
-    dev, n = cur.data.device, cur.data.shape[0]
+    `x + identity` -- the skip is added AFTER the dropout here, unlike the plain variants.  Runs at the width of `cur`."""
+    dev, (n, W) = cur.data.device, cur.data.shape
     code = cur.code
     s = _stream()
     wl, wr = engine.pack_linear(conv.lin_l.weight, prec), engine.pack_linear(conv.lin_r.weight, prec)
-    agg = Activation(n, 512, prec, dev)
+    agg = Activation(n, W, prec, dev)
     engine.aggregate(cur, agg, idx, "add")
-    u = Activation(n, 512, prec, dev)
+    u = Activation(n, W, prec, dev)
     inv_norm = _f32((n,), dev)
     with engine.TIMERS.span("train_update_gemm"):
-        engine.gemm512(engine._segments(agg, wl) + engine._segments(cur, wr), n, prec, u, bias=bias_host.data_ptr(),
-                       normalize=True, inv_norm_out=inv_norm.data_ptr())
-    vec = _f32((4, 512), dev)
+        engine.gemm(engine._segments(agg, wl) + engine._segments(cur, wr), n, prec, u, bias=bias_host.data_ptr(),
+                    normalize=True, inv_norm_out=inv_norm.data_ptr())
+    vec = _f32((4, W), dev)
     track = bn.track_running_stats and bn.running_mean is not None
     momentum = 0.1 if bn.momentum is None else float(bn.momentum)
     capi.bn_batch_stats(u.data.data_ptr(), code, n, bn.weight.detach().data_ptr(), bn.bias.detach().data_ptr(), float(bn.eps),
                         momentum, bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
                         bn.num_batches_tracked.data_ptr() if track else None, vec[0].data_ptr(), vec[1].data_ptr(),
-                        vec[2].data_ptr(), vec[3].data_ptr(), ws.data_ptr(), ws_bytes, s)
-    y = Activation(n, 512, prec, dev)
-    capi.bn_act_forward(u.data.data_ptr(), None, y.data.data_ptr(), code, n, vec[0].data_ptr(), vec[1].data_ptr(), p_drop, seed_i, s)
+                        vec[2].data_ptr(), vec[3].data_ptr(), ws.data_ptr(), ws_bytes, s, width=W)
+    y = Activation(n, W, prec, dev)
+    capi.bn_act_forward(u.data.data_ptr(), None, y.data.data_ptr(), code, n, vec[0].data_ptr(), vec[1].data_ptr(), p_drop, seed_i, s,
+                        width=W)
     if residual:
         capi.add(y.data.data_ptr(), cur.data.data_ptr(), None, y.data.data_ptr(), code, y.data.numel(), s)
     y.refresh_split()
@@ -576,28 +578,28 @@ def _sag_layer_forward(conv, bn, cur: Activation, idx, prec: str, bias_host, res
 def _sag_layer_backward(saved, gup: Activation, idx, idx_t, prec: str, p_drop: float, grads: GradStore, ws, ws_bytes) -> Activation:
     """Backward of `_sag_layer_forward`: `gup` is d loss / d (layer output); returns d loss / d (layer input)."""
     conv, bn, x_in, agg, u, inv_norm, vec, residual, seed_i = saved
-    dev, n = gup.data.device, gup.data.shape[0]
+    dev, (n, W) = gup.data.device, gup.data.shape
     code = gup.code
     s = _stream()
-    dz = Activation(n, 512, prec, dev)
+    dz = Activation(n, W, prec, dev)
     dgam, acc_g = grads.get(bn.weight); dbet, _ = grads.get(bn.bias)
     capi.sage_backward_rows(u.data.data_ptr(), gup.data.data_ptr(), None, inv_norm.data_ptr(), None, code, n,
                             vec[0].data_ptr(), vec[1].data_ptr(), vec[2].data_ptr(), vec[3].data_ptr(), p_drop, seed_i,
-                            dgam.data_ptr(), dbet.data_ptr(), acc_g, dz.data.data_ptr(), None, None, ws.data_ptr(), ws_bytes, s)
+                            dgam.data_ptr(), dbet.data_ptr(), acc_g, dz.data.data_ptr(), None, None, ws.data_ptr(), ws_bytes, s,
+                            width=W)
     dz.refresh_split()
     dwl, acc_l = grads.get(conv.lin_l.weight)
     dwr, acc_r = grads.get(conv.lin_r.weight)
-    weight_grad_mn(dz.data, agg.data, code, n, dwl, acc_l)
-    weight_grad_mn(dz.data, x_in.data, code, n, dwr, acc_r)
+    sage_weight_grads(dz.data, agg.data, x_in.data, code, n, dwl, acc_l, dwr, acc_r)
     dbl, acc_b = grads.get(conv.lin_l.bias)
-    colsum(dz.data, code, n, 512, 512, dbl, accumulate=acc_b)
+    colsum(dz.data, code, n, W, W, dbl, accumulate=acc_b)
     wlt, wrt = transposed_pack(conv.lin_l.weight, prec), transposed_pack(conv.lin_r.weight, prec)
-    dagg = Activation(n, 512, prec, dev)
-    engine.gemm512(engine._segments(dz, wlt), n, prec, dagg)
-    sbuf = Activation(n, 512, prec, dev)
+    dagg = Activation(n, W, prec, dev)
+    engine.gemm(engine._segments(dz, wlt), n, prec, dagg)
+    sbuf = Activation(n, W, prec, dev)
     engine.aggregate(dagg, sbuf, idx_t, "sum")                      # A^T dagg ('add' aggregation: no degree scaling)
-    dx = Activation(n, 512, prec, dev)
-    engine.gemm512(engine._segments(dz, wrt), n, prec, dx, residual=sbuf.data.data_ptr(), ldr=512)
+    dx = Activation(n, W, prec, dev)
+    engine.gemm(engine._segments(dz, wrt), n, prec, dx, residual=sbuf.data.data_ptr(), ldr=W)
     if residual:                                                    # the skip branch carries the undropped gradient
         capi.add(dx.data.data_ptr(), gup.data.data_ptr(), None, dx.data.data_ptr(), code, dx.data.numel(), s)
         dx.refresh_split()
@@ -607,7 +609,9 @@ def _sag_layer_backward(saved, gup: Activation, idx, idx_t, prec: str, p_drop: f
 class SagTrainFunction(torch.autograd.Function):
     """Training step of `GraphSAGE_SAG` (Models/BuckGNN.py:190-217, 493-511): num_layers // 2 SAGE('add') layers,
     SAGPooling(0.5) -- differentiable through `x[perm] * score[perm]` and the tanh score GNN, the selection itself is
-    piecewise constant -- then the remaining layers on the pooled graph, pooling and the eigenvalue head."""
+    piecewise constant -- then the remaining layers on the pooled graph, pooling and the eigenvalue head.  Runs at
+    W = model.hidden_channels: 512, or 128 (`BuckGNN.native128_sag`: engine.gemm picks bg_gemm128, the weight gradients
+    run on bg_wgrad128, the row kernels on their `*128` entry points and the 2-layer encoder on bg_sgemm)."""
 
     @staticmethod
     def forward(ctx, model, x, edge_index, batch, seed, *params):
@@ -620,16 +624,19 @@ class SagTrainFunction(torch.autograd.Function):
         enc = model.node_encoder
         convs = model._sage_layers()
         n_before = len(model.sage_layers_1)
-        biases = torch.stack([enc[4].bias.detach().float()] + [c.lin_l.bias.detach().float() for c, _ in convs]).cpu()
+        W = model.hidden_channels                          # 512, or 128 (BuckGNN.native128_sag)
+        if W not in (512, 128):
+            raise NotImplementedError(f"buckgnn_b200: the GraphSAGE_SAG training step runs at width 512 or 128, not {W}")
+        biases = torch.stack([enc[-1].bias.detach().float()] + [c.lin_l.bias.detach().float() for c, _ in convs]).cpu()
         sv = _Saved()
         sv.model, sv.prec, sv.n, sv.x, sv.seed, sv.p_drop = model, prec, n, x, seed, p_drop
-        sv.h1, sv.h2, cur = encoder_forward_train(enc, x, prec, biases[0])
+        sv.h1, sv.h2, cur = encoder_forward_train(enc, x, prec, biases[0], width=W)
         idx = pending.finish()
         sv.idx_full, sv.edge_index = idx, pending.edge_index
         ws_bytes = capi.train_workspace_bytes(n)
         ws = _ws(ws_bytes, dev)
-        ones = torch.ones(512, dtype=torch.float32, device=dev)
-        zeros = torch.zeros(512, dtype=torch.float32, device=dev)
+        ones = torch.ones(W, dtype=torch.float32, device=dev)
+        zeros = torch.zeros(W, dtype=torch.float32, device=dev)
         sv.first, sv.second = [], []
         for i in range(n_before):
             conv, bn = convs[i]
@@ -675,21 +682,22 @@ class SagTrainFunction(torch.autograd.Function):
         # ---- SAGPooling backward
         idx_t = engine.build_graph_index(sv.edge_index, None, n, key_row=0)
         xin = sv.pool_in
-        dx = Activation(n, 512, prec, dev)
+        W = xin.data.shape[1]
+        dx = Activation(n, W, prec, dev)
         t, dpre = _f32((n,), dev), _f32((n,), dev)
         pack = sv.pool_pack
+        pool_backward = capi.sag_pool_backward128 if W == 128 else capi.sag_pool_backward
         with engine.TIMERS.span("sag_pool_bwd"):
-            capi.sag_pool_backward(dcur.data.data_ptr(), xin.data.data_ptr(), code, n, n2, pooled.perm.data_ptr(),
-                                   pooled.new_id.data_ptr(), pooled.all_scores.data_ptr(), float(model._sag_sign),
-                                   idx_t.rowptr.data_ptr(), idx_t.col.data_ptr(), idx_t.big_rows.data_ptr(), idx_t.n_big,
-                                   pack["w_l"].data_ptr(), pack["w_r"].data_ptr(), dx.data.data_ptr(), t.data_ptr(),
-                                   dpre.data_ptr(), s)
+            pool_backward(dcur.data.data_ptr(), xin.data.data_ptr(), code, n, n2, pooled.perm.data_ptr(),
+                          pooled.new_id.data_ptr(), pooled.all_scores.data_ptr(), float(model._sag_sign),
+                          idx_t.rowptr.data_ptr(), idx_t.col.data_ptr(), idx_t.big_rows.data_ptr(), idx_t.n_big,
+                          pack["w_l"].data_ptr(), pack["w_r"].data_ptr(), dx.data.data_ptr(), t.data_ptr(), dpre.data_ptr(), s)
             dx.refresh_split()
             gnn = model.pool.gnn
             dwl, _ = grads.get(gnn.lin_l.weight); dwr, _ = grads.get(gnn.lin_r.weight); dbl, _ = grads.get(gnn.lin_l.bias)
-            # dw_l = sum_j t_j x_j, dw_r = sum_j dpre_j x_j: [1, n] x [n, 512]
-            sgemm(t, F32, 0, 1, xin.data, code, 512, 1, 1, 512, n, dwl, F32, 512)
-            sgemm(dpre, F32, 0, 1, xin.data, code, 512, 1, 1, 512, n, dwr, F32, 512)
+            # dw_l = sum_j t_j x_j, dw_r = sum_j dpre_j x_j: [1, n] x [n, W]
+            sgemm(t, F32, 0, 1, xin.data, code, W, 1, 1, W, n, dwl, F32, W)
+            sgemm(dpre, F32, 0, 1, xin.data, code, W, 1, 1, W, n, dwr, F32, W)
             colsum(dpre, F32, n, 1, 1, dbl)
         dcur = dx
         for saved in reversed(sv.first):

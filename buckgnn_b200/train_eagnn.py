@@ -20,7 +20,9 @@ hidden_channels = 128 model trains on its own 128-wide kernels instead of the ze
 At 128 the products run on `bg_gemm128` / `bg_gemm128_gathered` (engine.gemm picks by the output width), the weight
 gradients on `bg_wgrad128_ld` (written in place into the column slices of the concatenated Linears, the pair
 `[x | agg]` of node_mlp_gamma[0] in one launch), the row kernels are the `*128` entry points, and the encoders and the
-decoder are the reference's 2-layer MLPs on bg_sgemm (train.py).  EAGNN_SAG trains at 512 only.
+decoder are the reference's 2-layer MLPs on bg_sgemm (train.py).  EAGNN_SAG (`EAGNNSagTrainFunction`) runs at the
+model's width as well: at 128 when `BuckGNN.native128_sag` is on, with the SAGPooling rows on bg_gather_rows128 /
+bg_sag_pool_backward128.
 """
 from __future__ import annotations
 
@@ -341,7 +343,8 @@ class EAGNNTrainFunction(torch.autograd.Function):
 class EAGNNSagTrainFunction(torch.autograd.Function):
     """Training step of `EAGNN_SAG` (Models/BuckGNN.py:219-244, 354-373): GraphNetBlocks, SAGPooling (node rows scaled by
     the tanh score, edge rows of the kept edges carried over), GraphNetBlocks on the pooled graph, pooling + head.  The
-    skip is added after the Dropout in both loops (`i > 0` in the first, always in the second)."""
+    skip is added after the Dropout in both loops (`i > 0` in the first, always in the second).  Runs at
+    W = model.hidden_channels: 512, or 128 (`BuckGNN.native128_sag`)."""
 
     @staticmethod
     def forward(ctx, model, x, edge_index, edge_attr, batch, seed, *params):
@@ -357,11 +360,14 @@ class EAGNNSagTrainFunction(torch.autograd.Function):
         pending = engine.begin_graph_index(edge_index, batch, n, key_row=0)       # GraphNetBlock direction (source-keyed)
         pending_t = engine.begin_graph_index(edge_index, None, n, key_row=1)      # SAGEConv direction of the score GNN
         first, second = list(model.gnn_layers_1), list(model.gnn_layers_2)
-        W = 512                                            # EAGNN_SAG trains at 512 (the twin at other widths)
+        W = model.hidden_channels                          # 512, or 128 (BuckGNN.native128_sag)
+        if W not in (512, 128):
+            raise NotImplementedError(f"buckgnn_b200: the EAGNN_SAG training step runs at width 512 or 128, not {W}")
+        gather = capi.gather_rows128 if W == 128 else capi.gather_rows
         biases, bias_of, weights = _block_tables(model, first + second, prec, W)
         sv = _Saved()
         sv.model, sv.prec, sv.n, sv.x, sv.seed, sv.p_drop = model, prec, n, x, seed, p_drop
-        sv.h1, sv.h2, cur = encoder_forward_train(model.node_encoder, x, prec, biases[0])
+        sv.h1, sv.h2, cur = encoder_forward_train(model.node_encoder, x, prec, biases[0], width=W)
         idx = pending.finish()
         idx_t = pending_t.finish()
         ne = idx.n_edges
@@ -370,7 +376,7 @@ class EAGNNSagTrainFunction(torch.autograd.Function):
         st1 = _Stage(idx, prec, dev, W)
         ea = edge_attr.detach().to(torch.float32).index_select(0, idx.perm[:ne].long()).contiguous()
         sv.ea = ea
-        sv.eh1, sv.eh2, e = encoder_forward_train(model.edge_encoder, ea, prec, biases[1])
+        sv.eh1, sv.eh2, e = encoder_forward_train(model.edge_encoder, ea, prec, biases[1], width=W)
         sv.first, sv.second = [], []
         for i, blk in enumerate(first):
             cur, e, saved = _block_forward(st1, blk, weights[id(blk)], bias_of[id(blk)], cur, e, i > 0, p_drop, seed, i, True)
@@ -384,7 +390,7 @@ class EAGNNSagTrainFunction(torch.autograd.Function):
             raise NotImplementedError("buckgnn_b200: EAGNN_SAG training needs at least one edge after the pooling")
         slot_map = engine.edge_slot_map(idx, idx2, pooled.kept_edge)             # new slot -> old slot
         e2 = Activation(idx2.n_edges, W, prec, dev)
-        capi.gather_rows(e.data.data_ptr(), code, W, slot_map.data_ptr(), None, idx2.n_edges, e2.data.data_ptr(), W, s)
+        gather(e.data.data_ptr(), code, W, slot_map.data_ptr(), None, idx2.n_edges, e2.data.data_ptr(), W, s)
         e2.refresh_split()
         sv.pool_in, sv.pooled, sv.pool_pack, sv.slot_map = cur, pooled, pack, slot_map
         st2 = _Stage(idx2, prec, dev, W)
@@ -426,12 +432,13 @@ class EAGNNSagTrainFunction(torch.autograd.Function):
         dx = Activation(n, W, prec, dev)
         t, dpre = _f32((n,), dev), _f32((n,), dev)
         pack = sv.pool_pack
+        pool_backward, gather = ((capi.sag_pool_backward128, capi.gather_rows128) if W == 128 else
+                                 (capi.sag_pool_backward, capi.gather_rows))
         with engine.TIMERS.span("sag_pool_bwd"):
-            capi.sag_pool_backward(dxn.data.data_ptr(), xin.data.data_ptr(), code, n, n2, pooled.perm.data_ptr(),
-                                   pooled.new_id.data_ptr(), pooled.all_scores.data_ptr(), float(model._sag_sign),
-                                   idx.rowptr.data_ptr(), idx.col.data_ptr(), idx.big_rows.data_ptr(), idx.n_big,
-                                   pack["w_l"].data_ptr(), pack["w_r"].data_ptr(), dx.data.data_ptr(), t.data_ptr(),
-                                   dpre.data_ptr(), s)
+            pool_backward(dxn.data.data_ptr(), xin.data.data_ptr(), code, n, n2, pooled.perm.data_ptr(),
+                          pooled.new_id.data_ptr(), pooled.all_scores.data_ptr(), float(model._sag_sign),
+                          idx.rowptr.data_ptr(), idx.col.data_ptr(), idx.big_rows.data_ptr(), idx.n_big,
+                          pack["w_l"].data_ptr(), pack["w_r"].data_ptr(), dx.data.data_ptr(), t.data_ptr(), dpre.data_ptr(), s)
             dx.refresh_split()
             gnn = model.pool.gnn
             dwl, _ = grads.get(gnn.lin_l.weight); dwr, _ = grads.get(gnn.lin_r.weight); dbl, _ = grads.get(gnn.lin_l.bias)
@@ -445,7 +452,7 @@ class EAGNNSagTrainFunction(torch.autograd.Function):
                 inv = torch.full((ne,), -1, dtype=torch.int32, device=dev)     # old slot -> new slot, -1 for a dropped edge
                 capi.index_invert(sv.slot_map.data_ptr(), ne2, inv.data_ptr(), s)
                 de = Activation(ne, W, prec, dev)
-                capi.gather_rows(den.data.data_ptr(), code, W, inv.data_ptr(), None, ne, de.data.data_ptr(), W, s)
+                gather(den.data.data_ptr(), code, W, inv.data_ptr(), None, ne, de.data.data_ptr(), W, s)
                 de.refresh_split()
         dxn, den = dx, de
         for i in range(len(sv.first) - 1, -1, -1):

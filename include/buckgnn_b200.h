@@ -385,6 +385,28 @@ int bg_gather_rows(const void* x, int dtype, int64_t ldx, const int32_t* row_ind
                    int64_t n_rows_out, void* out, int64_t ldo, void* stream);
 int bg_index_invert(const int32_t* perm, int64_t n, int32_t* out, void* stream);
 int bg_index_gather(const int32_t* table, const int32_t* idx, int64_t n, int32_t* out, void* stream);
+/* SAGPooling of a hidden_channels = 128 model (BuckGNN.native128_sag), on [*, 128] rows: every argument and rule is the
+ * one of the 512-wide call above, with 128 for 512 --
+ *   bg_sag_select128: x [N,128], w_l / w_r [128].  Only the pass computing w_l . x and w_r . x reads rows; the score,
+ *     the top-k, the new offsets and the edge count are the 512-wide call's, and bg_sag_connect /
+ *     bg_sag_workspace_bytes serve both widths.
+ *   bg_gather_rows128: out[r, 0:128] = x[row_index[r], 0:128] * (row_scale ? row_scale[row_index[r]] : 1), ldx / ldo
+ *     >= 128; a negative row_index[r] gives a zero row.
+ *   bg_sag_pool_backward128: dx_pooled [N',128], x / dx [N,128], w_l / w_r [128]; t and dpre stay [N].
+ * Every argument is checked before the first CUDA call.  fp32 accumulation in a fixed order, no floating-point atomics:
+ * repeated calls are bit-identical. */
+int bg_sag_select128(const void* x, int dtype, int64_t n_nodes, const int32_t* rowptr, const int32_t* col,
+                     const int32_t* big_rows, int32_t n_big, const float* w_l, const float* w_r, float bias, float sign,
+                     const int32_t* graph_ptr, int64_t n_graphs, float ratio, const int64_t* edge_index, int64_t n_edges,
+                     float* score, int32_t* new_id, int32_t* perm, int64_t* batch_out, float* score_out,
+                     int32_t* new_graph_ptr, int32_t* info, void* workspace, size_t workspace_bytes, void* stream);
+int bg_gather_rows128(const void* x, int dtype, int64_t ldx, const int32_t* row_index, const float* row_scale,
+                      int64_t n_rows_out, void* out, int64_t ldo, void* stream);
+int bg_sag_pool_backward128(const void* dx_pooled, const void* x, int dtype, int64_t n_nodes, int64_t n_nodes_out,
+                            const int32_t* perm, const int32_t* new_id, const float* score, float sign,
+                            const int32_t* rowptr_src, const int32_t* col_src, const int32_t* big_rows_src,
+                            int32_t n_big_src, const float* w_l, const float* w_r, void* dx, float* t, float* dpre,
+                            void* stream);
 
 /* ------------------------------------------------------------------ training step
  * What `loss.backward()` and train-mode BatchNorm1d / Dropout need around the forward kernels
